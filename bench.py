@@ -4,6 +4,8 @@
   python bench.py --gpus N --steps K --warmup W            our arm (one process per GPU under torchrun)
   python bench.py --impl reference --gpus N ...            the reference arm: the CPU oracle ("port" of
                                                            the CasADi evaluation) on the host cores
+  python bench.py ... --dump-outputs DIR                   also write the outputs of the last timed step
+                                                           (see dump_outputs) as DIR/<name>.npy
 
 A *step* is one evaluation of f, grad_f, g, jac_g and hess_l (what IPOPT requests at an iteration with
 an exact Hessian) for every instance of the batch.  Workload at every N: BASELINE config 3,
@@ -32,6 +34,7 @@ UNIT = "knot-evals/s (f+grad_f+g+jac_g+hess_l)"
 WORKLOAD = "humanoid_kinodynamic single step flat ground (BASELINE config 3), horizon 30, 1024 instances per GPU"
 PLANS_PER_GPU = 512  # BASELINE config 4: 4096 instances sharded over 8 GPUs
 REFERENCE_BUDGET_S = 150.0  # wall-clock budget of the reference arm's timed + warm-up steps
+DUMP_INSTANCES = 64  # instances whose full outputs --dump-outputs writes: 64 x 0.8 MB, under 64 MB in all
 
 
 def parse():
@@ -42,7 +45,37 @@ def parse():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--cpu-sample", type=int, default=256, help="instances in the CPU baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float64): f of every instance of "
+                         f"rank 0's shard, grad_f, g, jac and hess of {DUMP_INSTANCES} of them (dump_rows)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path; the reference arm keeps none")
+    return args
+
+
+def dump_rows(batch: int):
+    """The instances whose grad_f, g, jac and hess --dump-outputs writes: a fixed, seeded, sorted sample of the batch."""
+    import numpy as np
+
+    rows = np.random.default_rng(0).choice(batch, min(DUMP_INSTANCES, batch), replace=False)
+    return np.sort(rows)
+
+
+def dump_outputs(out: dict, directory: str) -> None:
+    """Write one evaluation's outputs (``KinoEvaluator.eval``'s dict of (B, ...) float64 device tensors) as
+    directory/<name>.npy: ``f`` whole, the wider arrays only at the rows of ``dump_rows(B)``."""
+    import numpy as np
+    import torch
+
+    os.makedirs(directory, exist_ok=True)
+    f = out["f"]
+    rows = torch.as_tensor(dump_rows(f.shape[0]), device=f.device)
+    for name, t in out.items():
+        a = t if name == "f" else t.index_select(0, rows)
+        np.save(os.path.join(directory, f"{name}.npy"), a.cpu().numpy())
 
 
 class ClockSampler:
@@ -363,7 +396,7 @@ def main():
     t0 = time.perf_counter()
     e0.record()
     for i in range(args.steps):
-        step(i)
+        last = step(i)
     e1.record()
     fence()
     t1 = time.perf_counter()
@@ -371,6 +404,9 @@ def main():
     launches_per_step = ev.last_launch_count()  # kernels one hb_eval of the timed region enqueued
     kernel_ms, n_evals = ev.profile_read()
     ev.profile(False)
+    if args.dump_outputs and rank == 0:
+        # now, while `last` still holds the timed step's values: ev.eval reuses its output buffers
+        dump_outputs(last, args.dump_outputs)
     clocks = sampler.stop(t0, t1) if rank == 0 else None
     t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
     if world > 1:

@@ -1,11 +1,12 @@
 """bench.py's contract that can be checked without a GPU: the reference arm (the CPU oracle on the host cores,
-`--impl reference`) prints one JSON line with the agreed keys, only rank 0 works under torchrun, and the product arm
-refuses to run without a CUDA device instead of falling back to anything."""
+`--impl reference`) prints one JSON line with the agreed keys, only rank 0 works under torchrun, the product arm
+refuses to run without a CUDA device instead of falling back to anything, and arguments it cannot honour are refused."""
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 import torch
 
@@ -41,6 +42,21 @@ def test_reference_arm_honours_steps_and_warmup():
     assert r.returncode == 0, r.stderr[-2000:]
     d = json.loads([ln for ln in r.stdout.splitlines() if ln.strip()][0])
     assert d["steps"] == 4 and d["warmup"] == 2 and "(4 timed steps, 2 warm-up)" in d["cpu_baseline"]["sample"]
+
+
+@pytest.mark.parametrize("args,message", [(["--steps", "0"], "--steps must be at least 1"),
+                                          (["--impl", "reference", "--dump-outputs", "out"], "the reference arm keeps none")])
+def test_arguments_that_are_refused(args, message):
+    r = run(args)
+    assert r.returncode == 2 and message in r.stderr and r.stdout == ""
+
+
+def test_dump_rows_are_a_fixed_sample():
+    import bench
+
+    rows = bench.dump_rows(1024)
+    assert len(rows) == bench.DUMP_INSTANCES and np.all(np.diff(rows) > 0) and rows[-1] < 1024
+    assert np.array_equal(rows, bench.dump_rows(1024)) and np.array_equal(bench.dump_rows(5), np.arange(5))
 
 
 def test_reference_arm_other_ranks_exit_quietly():
