@@ -9,6 +9,14 @@
 
 namespace hb {
 
+// D (8 x 8) = A (8 x 4, row) B (4 x 8, col) + C on the fp64 tensor cores.  Fragments (PTX ISA, mma.m8n8k4 .f64):
+// a: row lane / 4, column lane % 4;  b: row lane % 4, column lane / 4;  c, d: row lane / 4, columns 2 (lane % 4) + {0, 1}.
+__device__ __forceinline__ void dmma_m8n8k4(double& c0, double& c1, double a, double b) {
+  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};"
+               : "+d"(c0), "+d"(c1)
+               : "d"(a), "d"(b));
+}
+
 struct Dual {
   double v, d;
 };

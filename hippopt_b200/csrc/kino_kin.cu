@@ -648,27 +648,32 @@ __device__ __forceinline__ void kin_tangent_sweep_packed(const KinTopo& T, const
   }
 }
 
-// quaternion maps: g_a (rotation tangent of R(q/|q|) along q_a), u_a = d omega_0 / d q_a,
+// quaternion maps of component a: g_a (rotation tangent of R(q/|q|) along q_a), u_a = d omega_0 / d q_a,
 // w_a = d omega_0 / d q_dot_a.
 template <class T>
-__device__ __forceinline__ void quat_maps(const T* q, const double* qd, V3<T>* g, V3<T>* u, V3<T>* w) {
+__device__ __forceinline__ void quat_map(const T* q, const double* qd, int a, V3<T>& g, V3<T>& u, V3<T>& w) {
   const T r2 = q[0] * q[0] + q[1] * q[1] + q[2] * q[2] + q[3] * q[3];
   const T r = dsqrt(r2);
   const T ir = 1.0 / r;
-  T qh[4];
+  T qh[4], t[4];
 #pragma unroll
   for (int i = 0; i < 4; ++i) qh[i] = q[i] * ir;
+  T qha = qh[0];  // qh[a] by selects: a may be lane-dependent, and an indexed qh[a] would go to local memory
 #pragma unroll
-  for (int a = 0; a < 4; ++a) {
-    T t[4];
+  for (int i = 1; i < 4; ++i)
+    if (i == a) qha = qh[i];
 #pragma unroll
-    for (int i = 0; i < 4; ++i) t[i] = ((i == a ? 1.0 : 0.0) - qh[i] * qh[a]) * ir;
-    g[a] = omega_map(qh, t);
-    u[a] = omega_map(t, qd);
-    double e[4] = {0.0, 0.0, 0.0, 0.0};
-    e[a] = 1.0;
-    w[a] = omega_map(qh, e);
-  }
+  for (int i = 0; i < 4; ++i) t[i] = ((i == a ? 1.0 : 0.0) - qh[i] * qha) * ir;
+  g = omega_map(qh, t);
+  u = omega_map(t, qd);
+  double e[4] = {0.0, 0.0, 0.0, 0.0};
+#pragma unroll
+  for (int i = 0; i < 4; ++i) e[i] = i == a ? 1.0 : 0.0;
+  w = omega_map(qh, e);
+}
+__device__ __forceinline__ void quat_maps(const double* q, const double* qd, D3* g, D3* u, D3* w) {
+#pragma unroll
+  for (int a = 0; a < 4; ++a) quat_map(q, qd, a, g[a], u[a], w[a]);
 }
 
 struct JacEmit {
@@ -1197,7 +1202,7 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
     // base chain rule
     D3 gq[4], uq[4], wq[4];
     const double qraw[4] = {q0, q1, q2, q3};
-    quat_maps<double>(qraw, qdv, gq, uq, wq);
+    quat_maps(qraw, qdv, gq, uq, wq);
     double dq[4], dqd[4];
 #pragma unroll
     for (int a = 0; a < 4; ++a) {
@@ -1264,23 +1269,26 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
     Dir dir;
     dir.mask = 0u;
     dir.alpha = dir.pi = dir.wpi = dir.vpi = dir.u = v3<double>(0.0, 0.0, 0.0);
-    // only the primal maps are needed for the directions; the dual maps are rebuilt after the sweep
-    // so that they are not live (144 registers) across it
-    D3 wq_lane = v3<double>(0.0, 0.0, 0.0);  // d omega_0 / d qd_a for the velocity-direction lanes 3..6
-    {
-      D3 gq0[4], uq0[4], wq0[4];
-      const double qraw[4] = {q0, q1, q2, q3};
-      quat_maps<double>(qraw, qdv, gq0, uq0, wq0);
-#pragma unroll
-      for (int a = 0; a < 4; ++a) {
-        if (a == lane) {
-          dir.alpha = gq0[a];
-          dir.u = uq0[a];
-        }
-        if (a + 3 == lane) wq_lane = wq0[a];
-      }
-    }
+    // quaternion maps, once per warp: lane a < 4 builds g_a, u_a, w_a into the point block of z, which the
+    // kinematics no longer reads (the g rows are done).  The packed sweep and the root chain rule read them there.
+    double* qdat = zs;       // [4][6]: g_a, u_a
+    double* qw = zs + 48;    // [4][3]: w_a  (zs + 24: the body masses of the sweep)
+    double* qK = zs + 60;    // [4][4]: K[a][b], then [4][4]: Kd[a][b] (root chain rule)
+    static_assert(48 + 12 + 32 <= Z_VB && HB_N_JOINTS + 1 <= 24, "quaternion tables overlap z or the masses");
     if (lane < 4) {
+      D3 g, u, w;
+      const double qraw[4] = {q0, q1, q2, q3};
+      quat_map<double>(qraw, qdv, lane, g, u, w);
+      st3(qdat + 6 * lane, g);
+      st3(qdat + 6 * lane + 3, u);
+      st3(qw + 3 * lane, w);
+    }
+    __syncwarp();
+    D3 wq_lane = v3<double>(0.0, 0.0, 0.0);  // d omega_0 / d qd_a for the velocity-direction lanes 3..6
+    if (lane >= 3 && lane < 7) wq_lane = ld3(qw + 3 * (lane - 3));
+    if (lane < 4) {
+      dir.alpha = ld3(qdat + 6 * lane);
+      dir.u = ld3(qdat + 6 * lane + 3);
       dir.mask = 0xffffffffu;
       dir.wpi = ld3(sb + SB_W);
       dir.vpi = ld3(sb + SB_V);
@@ -1320,22 +1328,37 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
     }
     __syncwarp();
     {
-      // lane = body: sum the rows of its sub-tree (every lane reads the same row: broadcast loads, no
-      // barriers; the leaf-to-root read-modify-write version of this pass took 12 % of the kernel)
-      double acc[16];
+      // sub-tree sums D[body][i] = sum_l S[body][l] CM[l][i] with the 0/1 mask S[body][l] = (sub_mask[body] >> l) & 1,
+      // on the fp64 tensor cores: 24 bodies x 16 components x 24 bodies is exactly 3 x 2 row/column tiles of
+      // 6 m8n8k4 steps, no padding.  (The FMA version broadcast-loaded all 384 moments on every lane; the
+      // leaf-to-root read-modify-write version before it took 12 % of the kernel.)
+      constexpr int NBODY = HB_N_JOINTS + 1;
+      static_assert(NBODY % 8 == 0, "the composite-moment product tiles the bodies by 8");
+      double acc[NBODY / 8][2][2];
 #pragma unroll
-      for (int i = 0; i < 16; ++i) acc[i] = 0.0;
-      for (int l = 0; l < nb; ++l) {
-        const double in = ((my_submask >> l) & 1u) ? 1.0 : 0.0;
-        const double* cl = comp + l * CM_STRIDE;
+      for (int mt = 0; mt < NBODY / 8; ++mt) {
+        // fragment rows: body 8 mt + lane / 4 (a: mask row; c, d: output row)
+        const unsigned rmask = __shfl_sync(0xffffffffu, my_submask, 8 * mt + (lane >> 2));
 #pragma unroll
-        for (int i = 0; i < 16; ++i) acc[i] = fma(in, cl[i], acc[i]);
+        for (int nt = 0; nt < 2; ++nt) acc[mt][nt][0] = acc[mt][nt][1] = 0.0;
+#pragma unroll
+        for (int kt = 0; kt < NBODY / 4; ++kt) {
+          const int l = 4 * kt + (lane & 3);
+          const double a = ((rmask >> l) & 1u) ? 1.0 : 0.0;
+#pragma unroll
+          for (int nt = 0; nt < 2; ++nt)
+            dmma_m8n8k4(acc[mt][nt][0], acc[mt][nt][1], a, comp[l * CM_STRIDE + 8 * nt + (lane >> 2)]);
+        }
       }
-      __syncwarp();
-      if (lane < nb) {
-        double* cm = comp + lane * CM_STRIDE;
+      __syncwarp();  // every tile has read the moments before they are overwritten
 #pragma unroll
-        for (int i = 0; i < 16; ++i) cm[i] = acc[i];
+      for (int mt = 0; mt < NBODY / 8; ++mt) {
+        double* cm = comp + (8 * mt + (lane >> 2)) * CM_STRIDE + 2 * (lane & 3);
+#pragma unroll
+        for (int nt = 0; nt < 2; ++nt) {
+          cm[8 * nt] = acc[mt][nt][0];
+          cm[8 * nt + 1] = acc[mt][nt][1];
+        }
       }
       __syncwarp();
     }
@@ -1579,23 +1602,17 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
         // initialises the stage; rows: vb3 qd4 sd23 (velocity lane = row) q4 s23 (direction lane = row - 30)
         double* stg = sm + L.stage;
         double* pslot = sm + L.gbuf;  // gbuf + lamk + slot: 474 contiguous doubles, all dead by now
-        // tangents of P (rows q, s) and of Pdot (all rows) parked in the slot area for the cross terms;
-        // quaternion direction data and the masses in the part of z the kinematics no longer reads
-        double* xt = pslot;           // [57][6]: dP_r (zero for velocity rows), dPdot_r
-        double* qdat = zs;            // [4][6]: g_a, u_a
+        // tangents of P (rows q, s) and of Pdot (all rows) parked in the slot area for the cross terms (odd row
+        // stride: the (q, s) block below reads a different row on every lane); the masses next to the quaternion
+        // maps in the part of z the kinematics no longer reads
+        constexpr int XT = 7;
+        double* xt = pslot;           // [57][XT]: dP_r (velocity rows: not stored, zero), dPdot_r
         double* massv = zs + 24;      // [nb]
         if (lane < 27) {
-          st3(xt + (30 + lane) * 6, tP);
-          st3(xt + (30 + lane) * 6 + 3, tPd);
+          st3(xt + (30 + lane) * XT, tP);
+          st3(xt + (30 + lane) * XT + 3, tPd);
         }
-        if (lane < 30) {
-          st3(xt + lane * 6, v3<double>(0.0, 0.0, 0.0));
-          st3(xt + lane * 6 + 3, vel_pv);
-        }
-        if (lane < 4) {
-          st3(qdat + 6 * lane, dir.alpha);
-          st3(qdat + 6 * lane + 3, dir.u);
-        }
+        if (lane < 30) st3(xt + lane * XT + 3, vel_pv);
         if (lane < nb) massv[lane] = my_mass;
         __syncwarp();
         if (lane < 27) {
@@ -1605,9 +1622,18 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
           const double sM = -1.0 / M;
           // velocity rows (vb, qd, sd: 0..29) have dP_r = 0: half the loads and products
 #pragma unroll 5
-          for (int r = 0; r < 30; ++r) col[r] = sM * dot(ld3(xt + 6 * r + 3), a2);
-#pragma unroll 3
-          for (int r = 30; r < 57; ++r) col[r] = sM * (dot(ld3(xt + 6 * r), a1) + dot(ld3(xt + 6 * r + 3), a2));
+          for (int r = 0; r < 30; ++r) col[r] = sM * dot(ld3(xt + XT * r + 3), a2);
+          // (q, s) x (q, s) block: hb.(dP_r x dPdot_d + dP_d x dPdot_r) is symmetric in (r, d).  Lane d takes the
+          // pairs {d, d + j mod 27}, j = 0..13 -- every unordered pair exactly once, 14 per lane -- and stores the
+          // value in both columns, so the stage holds every entry whichever of a mirrored pair the scatter reads.
+#pragma unroll 2
+          for (int j = 0; j < 14; ++j) {
+            const int e = lane + j < 27 ? lane + j : lane + j - 27;
+            const double* xe = xt + XT * (30 + e);
+            const double v = sM * (dot(ld3(xe), a1) + dot(ld3(xe + 3), a2));
+            col[30 + e] = v;
+            stg[e * 57 + 30 + lane] = v;
+          }
           if (lane >= 4) {  // joint regularisation on (sd_j, s_j), (s_j, s_j)
             col[7 + lane - 4] += em.add_sd;
             col[34 + lane - 4] += em.add_s;
@@ -1631,34 +1657,46 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
       v0 = lift<Dual>(ld3(sb + SB_ACC + 9), tv0);
     }
 #endif
+    // Root chain rule dq_a = n0.g_a + w0.u_a, dqd_a = w0.w_a along direction d: the tangents of the root totals
+    // against the maps, plus (quaternion directions d < 4 only) the curvature of the maps against the primal
+    // totals, K[a][d] = n0.dg_a/dq_d + w0.du_a/dq_d and Kd[a][d] = w0.dw_a/dq_d.  K and Kd are the same on
+    // every lane: lane 4 a + b builds entry (a, b) in dual arithmetic, the other lanes need none.
+    if (lane < 16) {
+      const int a = lane >> 2, bq = lane & 3;
+      Dual qD[4];
+      double qdv2[4];
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        qD[i] = mkdual(zs[Z_Q + i], i == bq ? 1.0 : 0.0);
+        qdv2[i] = zs[Z_QD + i];
+      }
+      V3<Dual> g, u, w;
+      quat_map<Dual>(qD, qdv2, a, g, u, w);
+      const D3 pn0 = primal_of(n0), pw0 = primal_of(w0);
+      qK[lane] = dot(pn0, tangent_of(g)) + dot(pw0, tangent_of(u));
+      qK[16 + lane] = dot(pw0, tangent_of(w));
+    }
+    __syncwarp();
     if (dirj >= 0) {
+      const D3 tn0 = tangent_of(n0), tw0 = tangent_of(w0);
       em.put(0, v0.x.d);
       em.put(1, v0.y.d);
       em.put(2, v0.z.d);
       const double lu = lu_pre;
-      // dual quaternion maps, rebuilt from shared memory after the sweep (see above)
-      Dual qD[4];
-      double qdv2[4];
-#pragma unroll
-      for (int a = 0; a < 4; ++a) {
-        qD[a] = mkdual(zs[Z_Q + a], a == lane ? 1.0 : 0.0);
-        qdv2[a] = zs[Z_QD + a];
-      }
-      V3<Dual> gq[4], uq[4], wq[4];
-      quat_maps<Dual>(qD, qdv2, gq, uq, wq);
       // Hessian of w_bq |qd^-1 (x) q - 1|^2 is 2 w_bq A^T A = 2 w_bq |qd|^2 I (left-multiplication matrix)
       const double nqd = rbq[0] * rbq[0] + rbq[1] * rbq[1] + rbq[2] * rbq[2] +
                          rbq[3] * rbq[3];  // re-read (L1/L2 hit by now) rather than kept live across the sweep
 #pragma unroll
       for (int a = 0; a < 4; ++a) {
-        const Dual dq = dot(n0, gq[a]) + dot(w0, uq[a]);
-        const Dual dqd = dot(w0, wq[a]);
+        const bool qdir = lane < 4;
+        const double dq = dot(tn0, ld3(qdat + 6 * a)) + dot(tw0, ld3(qdat + 6 * a + 3)) + (qdir ? qK[4 * a + lane] : 0.0);
+        const double dqd = dot(tw0, ld3(qw + 3 * a)) + (qdir ? qK[16 + 4 * a + lane] : 0.0);
         const double extra = (a == lane && k1) ? 2.0 * sg * T.w_bq * nqd + 2.0 * lu : 0.0;
-        em.put(3 + a, dqd.d);
-        em.put(30 + a, dq.d + extra);
+        em.put(3 + a, dqd);
+        em.put(30 + a, dq + extra);
       }
     }
-    HB_PHASE(0, 12);  // root chain rule (dual quaternion maps)
+    HB_PHASE(0, 12);  // root chain rule
     __syncwarp();
     if (em.stage) {
       // scatter the staged columns (27 directions x 57 rows) with coalesced map reads

@@ -20,6 +20,8 @@
 // panel by panel in the same order; piv[j] is the row (>= j) exchanged with row j.
 #include <cstdint>
 
+#include "hb_math.cuh"  // dmma_m8n8k4
+
 namespace hb {
 
 constexpr int LU_NB = 16;
@@ -39,14 +41,6 @@ constexpr int LU_NB = 16;
 #endif
 constexpr int LU_THREADS = HB_LU_THREADS;
 constexpr int LU_MAXN = 768;
-
-// D (8 x 8) = A (8 x 4, row) B (4 x 8, col) + C on the fp64 tensor cores.  Fragments (PTX ISA, mma.m8n8k4 .f64):
-// a: row lane / 4, column lane % 4;  b: row lane % 4, column lane / 4;  c, d: row lane / 4, columns 2 (lane % 4) + {0, 1}.
-__device__ __forceinline__ void dmma_m8n8k4(double& c0, double& c1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};"
-               : "+d"(c0), "+d"(c1)
-               : "d"(a), "d"(b));
-}
 
 __host__ __device__ inline int lu_ldp(int n) { return (n + 3) & ~3; }
 // dynamic shared memory of the factor kernel: panel + U strip (+ slack: the last vector loads of a tile may
