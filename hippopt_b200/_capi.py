@@ -106,6 +106,9 @@ def lib() -> ctypes.CDLL:
     L.hb_debug_sweep_schedule.restype = ctypes.c_int
     L.hb_debug_sweep_schedule.argtypes = [ctypes.c_int32, i32p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
                                           ctypes.c_int32, i32p, i32p]
+    L.hb_debug_sweep_schedule_n_base.restype = ctypes.c_int
+    L.hb_debug_sweep_schedule_n_base.argtypes = [ctypes.c_int32, i32p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
+                                                 ctypes.c_int32, ctypes.c_int32, i32p, i32p]
     L.hb_host_set_parameters.restype = ctypes.c_int
     L.hb_host_set_parameters.argtypes = [vp, vp, ctypes.c_int64, ctypes.c_int64]
     L.hb_eval_host.restype = ctypes.c_int
@@ -144,7 +147,8 @@ EXPORTED_SYMBOLS = [
     "hb_last_launch_count", "hb_last_error", "hb_probe_fp64_tflops", "hb_profile_enable", "hb_profile_read",
     "hb_host_set_parameters", "hb_eval_host", "hb_host_last_traffic", "hb_host_alloc", "hb_host_free",
     "hb_lu_factor_batched", "hb_lu_solve_batched", "hb_set_option", "hb_interpolate_humanoid_states",
-    "hb_eval_cost_terms", "hb_debug_sweep_schedule", "hb_kino_attach_tables", "hb_bounds", "hb_save", "hb_load",
+    "hb_eval_cost_terms", "hb_debug_sweep_schedule", "hb_debug_sweep_schedule_n_base", "hb_kino_attach_tables",
+    "hb_bounds", "hb_save", "hb_load",
     "hb_ccs_group_mul", "hb_external_bind", "hb_external_stats", "hb_kkt_assemble_stage",
 ] + ['hb_nlp_f', 'hb_nlp_f_n_in', 'hb_nlp_f_n_out', 'hb_nlp_f_sparsity_in', 'hb_nlp_f_sparsity_out', 'hb_nlp_f_work', 'hb_nlp_f_name_in', 'hb_nlp_f_name_out', 'hb_nlp_f_incref', 'hb_nlp_f_decref', 'hb_nlp_f_alloc_mem', 'hb_nlp_f_init_mem', 'hb_nlp_f_free_mem', 'hb_nlp_f_checkout', 'hb_nlp_f_release', 'hb_nlp_g', 'hb_nlp_g_n_in', 'hb_nlp_g_n_out', 'hb_nlp_g_sparsity_in', 'hb_nlp_g_sparsity_out', 'hb_nlp_g_work', 'hb_nlp_g_name_in', 'hb_nlp_g_name_out', 'hb_nlp_g_incref', 'hb_nlp_g_decref', 'hb_nlp_g_alloc_mem', 'hb_nlp_g_init_mem', 'hb_nlp_g_free_mem', 'hb_nlp_g_checkout', 'hb_nlp_g_release', 'hb_nlp_grad_f', 'hb_nlp_grad_f_n_in', 'hb_nlp_grad_f_n_out', 'hb_nlp_grad_f_sparsity_in', 'hb_nlp_grad_f_sparsity_out', 'hb_nlp_grad_f_work', 'hb_nlp_grad_f_name_in', 'hb_nlp_grad_f_name_out', 'hb_nlp_grad_f_incref', 'hb_nlp_grad_f_decref', 'hb_nlp_grad_f_alloc_mem', 'hb_nlp_grad_f_init_mem', 'hb_nlp_grad_f_free_mem', 'hb_nlp_grad_f_checkout', 'hb_nlp_grad_f_release', 'hb_nlp_jac_g', 'hb_nlp_jac_g_n_in', 'hb_nlp_jac_g_n_out', 'hb_nlp_jac_g_sparsity_in', 'hb_nlp_jac_g_sparsity_out', 'hb_nlp_jac_g_work', 'hb_nlp_jac_g_name_in', 'hb_nlp_jac_g_name_out', 'hb_nlp_jac_g_incref', 'hb_nlp_jac_g_decref', 'hb_nlp_jac_g_alloc_mem', 'hb_nlp_jac_g_init_mem', 'hb_nlp_jac_g_free_mem', 'hb_nlp_jac_g_checkout', 'hb_nlp_jac_g_release', 'hb_nlp_hess_l', 'hb_nlp_hess_l_n_in', 'hb_nlp_hess_l_n_out', 'hb_nlp_hess_l_sparsity_in', 'hb_nlp_hess_l_sparsity_out', 'hb_nlp_hess_l_work', 'hb_nlp_hess_l_name_in', 'hb_nlp_hess_l_name_out', 'hb_nlp_hess_l_incref', 'hb_nlp_hess_l_decref', 'hb_nlp_hess_l_alloc_mem', 'hb_nlp_hess_l_init_mem', 'hb_nlp_hess_l_free_mem', 'hb_nlp_hess_l_checkout', 'hb_nlp_hess_l_release']
 

@@ -158,14 +158,18 @@ static hb::SweepTopo sweep_topo_of(const hb::KinoConst& C) {
   T.foot_body[0] = C.foot_body[0];
   T.foot_body[1] = C.foot_body[1];
   T.chest_body = C.chest_body;
+  T.n_base = 0;  // the kernel fills the four quaternion columns in closed form (kino_kin.cu)
   return T;
 }
 
-extern "C" int hb_debug_sweep_schedule(int32_t nb, const int32_t* parent, int32_t foot_l, int32_t foot_r, int32_t chest,
-                                       int32_t typed, int32_t* tasks, int32_t* info) {
-  if (!parent || !tasks || !info || nb < 2 || nb > 28) return fail(HB_ERR_INVALID, "hb_debug_sweep_schedule: bad argument");
+extern "C" int hb_debug_sweep_schedule_n_base(int32_t nb, const int32_t* parent, int32_t foot_l, int32_t foot_r,
+                                              int32_t chest, int32_t typed, int32_t n_base, int32_t* tasks,
+                                              int32_t* info) {
+  if (!parent || !tasks || !info || nb < 2 || nb > 28 || n_base < 0 || n_base > 4)
+    return fail(HB_ERR_INVALID, "hb_debug_sweep_schedule: bad argument");
   hb::SweepTopo T;
   T.nb = nb;
+  T.n_base = n_base;
   for (int l = 0; l < 32; ++l) {
     T.parent[l] = l < nb ? parent[l] : -1;
     T.sub_mask[l] = 0u;
@@ -186,6 +190,11 @@ extern "C" int hb_debug_sweep_schedule(int32_t nb, const int32_t* parent, int32_
   info[5] = (int32_t)s.seed_mask;
   for (int d = 0; d < 27 && d < 4 + nb - 1; ++d) info[6 + d] = s.root_slot[d];
   return HB_OK;
+}
+
+extern "C" int hb_debug_sweep_schedule(int32_t nb, const int32_t* parent, int32_t foot_l, int32_t foot_r, int32_t chest,
+                                       int32_t typed, int32_t* tasks, int32_t* info) {
+  return hb_debug_sweep_schedule_n_base(nb, parent, foot_l, foot_r, chest, typed, 4, tasks, info);
 }
 
 template <class T>

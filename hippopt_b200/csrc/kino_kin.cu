@@ -489,6 +489,8 @@ __device__ __forceinline__ void kin_tangent_sweep(const KinTopo& C, const double
 // pure propagation through the ancestors of the joint.  Here those (direction, body) steps are TASKS,
 // list-scheduled by the host (api.cu::build_sweep_schedule) on the 32 lanes in ~12 rounds instead of
 // 23: in every round a lane executes the task sched[round][lane] -- whatever direction it belongs to.
+// The four quaternion directions are left out of the schedule (their columns are closed-form, see the
+// quaternion columns in kino_kin_kernel): 256 tasks, 92 of them in a sub-tree, in 13 rounds.
 //   * direction data (alpha, pivot, ...) and seed tangents stay in the registers of the OWNER lane d and
 //     are fetched with warp shuffles by the lane that executes a task of direction d;
 //   * a lane keeps the running adjoint of its chain in registers; where a chain ends it is added to a
@@ -498,7 +500,7 @@ __device__ __forceinline__ void kin_tangent_sweep(const KinTopo& C, const double
 //     step non-zero; its Hessian is the rank-structured term -(1/M) hb.(dP_i x dPdot_j + dP_j x dPdot_i),
 //     written into the stage beforehand (cross_terms), and the sweep runs with d xc = d xdot_c = 0.
 struct DirData {
-  D3 alpha, pi, wpi, vpi, u;
+  D3 alpha, pi, wpi, vpi;
 };
 __device__ __forceinline__ D3 shfl3(const D3& v, int src) {
   return v3<double>(__shfl_sync(0xffffffffu, v.x, src), __shfl_sync(0xffffffffu, v.y, src),
@@ -506,8 +508,8 @@ __device__ __forceinline__ D3 shfl3(const D3& v, int src) {
 }
 
 __device__ __forceinline__ void kin_tangent_sweep_packed(const KinTopo& T, const double* sb, const double* zs,
-                                                         const double* qdat, const double* massv, const SeedsT& ownS,
-                                                         D3 hb, double* pslot, double* stage) {
+                                                         const double* massv, const SeedsT& ownS, D3 hb, double* pslot,
+                                                         double* stage) {
   const int lane = threadIdx.x & 31;
   const D3 zero = v3<double>(0.0, 0.0, 0.0);
   for (int i = lane; i < T.n_pslots * 12; i += 32) pslot[i] = 0.0;
@@ -537,34 +539,27 @@ __device__ __forceinline__ void kin_tangent_sweep_packed(const KinTopo& T, const
       D3 tax = zero, trho = zero, twpar = zero;
       const D3 rho = ld3(bl + SB_RHO), wpar = ld3(sb + p * SB_STRIDE + SB_W);
       if (heavy) {
-        // direction data: a joint direction is the axis / origin / twist of its body (already in shared
-        // memory); the four quaternion directions rotate everything about the base origin (qdat: g_a, u_a)
+        // direction data: the axis / origin / twist of the joint's body, already in shared memory.  The schedule
+        // holds joint directions only (SweepTopo::n_base = 0): the quaternion columns are closed-form
         DirData dir;
         {
-          const double* bd = sb + (d < 4 ? 0 : d - 3) * SB_STRIDE;
+          const double* bd = sb + (d - 3) * SB_STRIDE;
           dir.wpi = ld3(bd + SB_W);
           dir.vpi = ld3(bd + SB_V);
-          if (d < 4) {
-            dir.alpha = ld3(qdat + 6 * d);
-            dir.u = ld3(qdat + 6 * d + 3);
-            dir.pi = zero;
-          } else {
-            dir.alpha = ld3(bd + SB_AX);
-            dir.u = zero;
-            dir.pi = ld3(bd + SB_O);
-          }
+          dir.alpha = ld3(bd + SB_AX);
+          dir.pi = ld3(bd + SB_O);
         }
         const double m = massv[l];
         // with typed rounds every task of a heavy round lies in the sub-tree of its direction (KT_IN_L set); the
         // untyped fallback schedule mixes both kinds, hence the select
         const bool in = (t & KT_IN_L) != 0;
-        const D3 a = in ? dir.alpha : zero, uu = in ? dir.u : zero;
+        const D3 a = in ? dir.alpha : zero;
         const D3 d_ = ld3(bl + SB_D), w = ld3(bl + SB_W);
         const D3 rr = ld3(bl + SB_O) - dir.pi;
         const D3 to = cross(a, rr);
         const D3 td = cross(a, d_);
-        const D3 tw = cadd(uu, a, w - dir.wpi);
-        const D3 tv = cadd(cadd(cross(dir.wpi, to), a, (ld3(bl + SB_V) - dir.vpi) - cross(dir.wpi, rr)), uu, rr);
+        const D3 tw = cross(a, w - dir.wpi);
+        const D3 tv = cadd(cross(dir.wpi, to), a, (ld3(bl + SB_V) - dir.vpi) - cross(dir.wpi, rr));
         tax = cross(a, ax);
         if (in) {  // local adjoints of body l move with the sub-tree of the direction
           const double* I = bl + SB_I;
@@ -585,7 +580,7 @@ __device__ __forceinline__ void kin_tangent_sweep_packed(const KinTopo& T, const
         }
         if (t & KT_IN_P) {  // the parent moves with the direction as well
           trho = cross(dir.alpha, rho);
-          twpar = cadd(dir.u, dir.alpha, wpar - dir.wpi);
+          twpar = cross(dir.alpha, wpar - dir.wpi);
         }
       }
       // seed tangents (zero where they do not apply).  The feet-distance row couples the two feet: a
@@ -1270,11 +1265,12 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
     dir.mask = 0u;
     dir.alpha = dir.pi = dir.wpi = dir.vpi = dir.u = v3<double>(0.0, 0.0, 0.0);
     // quaternion maps, once per warp: lane a < 4 builds g_a, u_a, w_a into the point block of z, which the
-    // kinematics no longer reads (the g rows are done).  The packed sweep and the root chain rule read them there.
+    // kinematics no longer reads (the g rows are done).  The root chain rule reads them there.
     double* qdat = zs;       // [4][6]: g_a, u_a
     double* qw = zs + 48;    // [4][3]: w_a  (zs + 24: the body masses of the sweep)
     double* qK = zs + 60;    // [4][4]: K[a][b], then [4][4]: Kd[a][b] (root chain rule)
-    static_assert(48 + 12 + 32 <= Z_VB && HB_N_JOINTS + 1 <= 24, "quaternion tables overlap z or the masses");
+    double* qt = zs + 92;    // [4][6]: tangents of the root totals n0, w0 along q_a (closed form, below)
+    static_assert(92 + 24 <= Z_VB && HB_N_JOINTS + 1 <= 24, "quaternion tables overlap z or the masses");
     if (lane < 4) {
       D3 g, u, w;
       const double qraw[4] = {q0, q1, q2, q3};
@@ -1397,6 +1393,45 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
       const D3 hv = symmul(cm + CM_J, A) - cross(P, cross(A, piv)) + cross(P, B);
       vel_dh = scale(-1.0 / mass_p, hv - scale(1.0 / M, cross(Pm, pv)));
       vel_pv = pv;
+    }
+    // ---- quaternion columns of the Hessian in closed form: the packed sweep walks the joint directions only.
+    // q_a turns the whole tree about the base origin (alpha = g_a) and adds u_a to omega_0.  Every kinematic row is
+    // either rotation invariant (feet distance) or a world-fixed multiplier mu dotted with a vector X that turns with
+    // the tree (contact points, CoM, angular momentum about the CoM), so the root totals are
+    //   w0 = I_c hb,  n0 = sum_X X x mu - omega_0 x w0 + kappa m(G)      (I_c: locked inertia about the CoM)
+    // and their tangents along q_a follow from root quantities (T = sum_X X mu^T over the points and the CoM):
+    //   tw0 = alpha x w0 - I_c (alpha x hb)
+    //   tn0 = (T - tr(T)) alpha + dhang x hb - u_a x w0 - omega_0 x tw0 + kappa' m(G) (alpha.m(G)) + kappa (G - phi) alpha
+    // (dhang: tangent of the angular momentum about the CoM, kappa' = 2 sigma w_frame).  Parked in z for the root
+    // chain rule, which turns them into rows vb, qd, q of the q columns; tests/test_quat_hessian_closed_form_cpu.py
+    // checks these forms against the oracle's Hessian.
+    if (with_l) {
+      double* Tm = qK;  // [3][3], dead before the curvature tables are built
+      if (lane < 9) {
+        const int i = lane / 3, j = lane % 3;
+        double t = -(i == 0 ? xc.x : (i == 1 ? xc.y : xc.z)) * lamk[24 + j];
+#pragma unroll
+        for (int pt = 0; pt < 8; ++pt)
+          t -= (sb[T.foot_body[pt >> 2] * SB_STRIDE + SB_O + i] + sm[L.arms + 3 * pt + i]) * lamk[3 * pt + j];
+        Tm[lane] = t;
+      }
+      __syncwarp();
+      if (lane < 4) {
+        const D3 a = dir.alpha, om = ld3(sb + SB_W), hbv = scale(-1.0 / mass_p, ld3(lamk + 27));
+        const double* J0 = comp + CM_J;  // composite moments of the root: the whole tree
+        const D3 ah = cross(a, hbv);
+        const D3 w0 = symmul(J0, hbv) - scale(1.0 / M, cross(Pm, cross(hbv, Pm)));  // I_c x = J0 x - P x (x x P) / M
+        const D3 tw0 = cross(a, w0) - (symmul(J0, ah) - scale(1.0 / M, cross(Pm, cross(ah, Pm))));
+        const D3 dhang = th - scale(1.0 / M, cross(tP, Pd) + cross(Pm, tPd));
+        const double trT = Tm[0] + Tm[4] + Tm[8];
+        const double cf = k1 ? 2.0 * sg * T.w_frame : 0.0, kap = cf * (phi - 3.0);
+        D3 tn0 = v3<double>(Tm[0] * a.x + Tm[1] * a.y + Tm[2] * a.z, Tm[3] * a.x + Tm[4] * a.y + Tm[5] * a.z,
+                            Tm[6] * a.x + Tm[7] * a.y + Tm[8] * a.z) - scale(trT, a);
+        tn0 = tn0 + cross(dhang, hbv) - cross(dir.u, w0) - cross(om, tw0);
+        tn0 = tn0 + scale(cf * dot(a, mG), mG) + scale(kap, matvec(G, a) - scale(phi, a));
+        st3(qt + 6 * lane, tn0);
+        st3(qt + 6 * lane + 3, tw0);
+      }
     }
     __syncwarp();  // the stage is reused for the Jacobian columns below
     const V3<Dual> xcD = lift<Dual>(xc, scale(1.0 / M, tP));
@@ -1573,6 +1608,7 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
     }
     V3<Dual> n0, w0, v0;
     const double lu_pre = lamk[31];  // read now: the slots of the packed sweep alias gbuf + lamk + slot
+    const D3 lam_al = cross(ld3(lamk + 27), dir.alpha);  // quaternion lanes: velocity rows of their column (below)
 #ifdef HB_DUAL_SWEEP
     // reference implementation: the whole adjoint sweep in dual arithmetic on every lane
     kin_backward<Dual>(T, sb, zs, dir, S, xcD, xdD, slot, em, n0, w0, v0);
@@ -1606,13 +1642,16 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
         // stride: the (q, s) block below reads a different row on every lane); the masses next to the quaternion
         // maps in the part of z the kinematics no longer reads
         constexpr int XT = 7;
-        double* xt = pslot;           // [57][XT]: dP_r (velocity rows: not stored, zero), dPdot_r
+        double* xt = pslot;           // [57][XT]: dP_r (velocity rows: zero, the place holds vel_dh), dPdot_r
         double* massv = zs + 24;      // [nb]
         if (lane < 27) {
           st3(xt + (30 + lane) * XT, tP);
           st3(xt + (30 + lane) * XT + 3, tPd);
         }
-        if (lane < 30) st3(xt + lane * XT + 3, vel_pv);
+        if (lane < 30) {
+          st3(xt + lane * XT, vel_dh);
+          st3(xt + lane * XT + 3, vel_pv);
+        }
         if (lane < nb) massv[lane] = my_mass;
         __syncwarp();
         if (lane < 27) {
@@ -1620,9 +1659,16 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
           const D3 a1 = cross(tPd, hbv), a2 = cross(hbv, tP);  // hb.(dP_r x dPdot_d) = dP_r.a1, hb.(dP_d x dPdot_r) = dPdot_r.a2
           double* col = stg + lane * 57;
           const double sM = -1.0 / M;
-          // velocity rows (vb, qd, sd: 0..29) have dP_r = 0: half the loads and products
+          // velocity rows (vb, qd, sd: 0..29) have dP_r = 0: half the loads and products.  A quaternion column takes
+          // the whole entry there instead: the momentum row is linear in the velocities with a coefficient that turns
+          // with the tree, so d/dq_a (lam_m . vel_dh_r) = vel_dh_r . (lam_m x g_a) (rows qd get the curvature of the
+          // maps on top: they are replaced in the root chain rule)
+          const bool qc = lane < 4;
+          const D3 cr = qc ? lam_al : a2;
+          const double sc = qc ? 1.0 : sM;
+          const double* xr0 = xt + (qc ? 0 : 3);
 #pragma unroll 5
-          for (int r = 0; r < 30; ++r) col[r] = sM * dot(ld3(xt + XT * r + 3), a2);
+          for (int r = 0; r < 30; ++r) col[r] = sc * dot(ld3(xr0 + XT * r), cr);
           // (q, s) x (q, s) block: hb.(dP_r x dPdot_d + dP_d x dPdot_r) is symmetric in (r, d).  Lane d takes the
           // pairs {d, d + j mod 27}, j = 0..13 -- every unordered pair exactly once, 14 per lane -- and stores the
           // value in both columns, so the stage holds every entry whichever of a mirrored pair the scatter reads.
@@ -1642,12 +1688,20 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
         __syncwarp();
         HB_PHASE(0, 10);  // cross terms
         em.acc = true;
-        kin_tangent_sweep_packed(T, sb, zs, qdat, massv, ST, S.hb, pslot, stg);
+        kin_tangent_sweep_packed(T, sb, zs, massv, ST, S.hb, pslot, stg);
         HB_PHASE(0, 11);  // packed tangent sweep
-        const double* rs = pslot + (lane < 27 ? T.root_slot[lane] : 0) * 12;
-        tn0 = ld3(rs);
-        tw0 = ld3(rs + 6);
-        tv0 = ld3(rs + 9);
+        if (lane < 4) {  // closed form; v0 = 0 because hang does not depend on the base linear velocity
+          tn0 = ld3(qt + 6 * lane);
+          tw0 = ld3(qt + 6 * lane + 3);
+          tv0 = v3<double>(0.0, 0.0, 0.0);
+        } else {
+          const double* rs = pslot + (lane < 27 ? T.root_slot[lane] : 0) * 12;
+          tn0 = ld3(rs);
+          tw0 = ld3(rs + 6);
+          tv0 = ld3(rs + 9);
+        }
+        // the quaternion columns' rows vb, qd, q are complete (cross term included): stored, not added
+        em.acc = lane >= 4;
       }
 #else
       kin_tangent_sweep(T, sb, zs, dir, S.hb, ST, tangent_of(xcD), tangent_of(xdD), slot, em, tn0, tw0, tv0);
@@ -1694,6 +1748,10 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
         const double extra = (a == lane && k1) ? 2.0 * sg * T.w_bq * nqd + 2.0 * lu : 0.0;
         em.put(3 + a, dqd);
         em.put(30 + a, dq + extra);
+#if HB_SWEEP_PACKED && !defined(HB_DUAL_SWEEP)
+        // row s_j of column q_a by symmetry, on top of the cross term already staged there
+        if (lane >= 4) em.stage[a * 57 + 34 + lane - 4] += dq;
+#endif
       }
     }
     HB_PHASE(0, 12);  // root chain rule

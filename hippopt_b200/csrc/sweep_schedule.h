@@ -1,7 +1,8 @@
 // sweep_schedule.h -- host-side list scheduler of the packed tangent sweep (kino_kin.cu).  Plain C++ (no CUDA):
 // included by api.cu and compiled on its own by the CPU tests (hb_debug_sweep_schedule).
 //
-// Direction d (0..3 base quaternion, 4 + j joint j) only needs the bodies of its sub-tree (non-zero state
+// Direction d (0..3 base quaternion, 4 + j joint j; SweepTopo::n_base says how many of the four quaternion
+// directions take part) only needs the bodies of its sub-tree (non-zero state
 // tangents: "in") and the ancestors of its joint (pure propagation of the adjoint tangent).  Those bodies are cut
 // into chains that walk from a leaf towards the root; a chain ends where it meets a body that another chain of the
 // same direction continues through, and flushes its running adjoint into that body's slot.  Chains are
@@ -34,6 +35,8 @@ struct SweepTopo {
   int foot_body[2];
   int chest_body = 0;
   unsigned sub_mask[32];  // bit l: body l is in the sub-tree rooted at this body
+  int n_base = 4;         // base quaternion directions 0 .. n_base - 1 in the sweep (the kernel's schedule: none,
+                          // it fills the quaternion columns in closed form)
 };
 
 struct SweepSchedule {
@@ -58,6 +61,7 @@ inline SweepSchedule build_sweep_schedule(const SweepTopo& C, bool typed_rounds 
   std::vector<std::vector<char>> in_full(n_dir, std::vector<char>(nb, 0));
   int n_slots = 0;
   for (int d = 0; d < n_dir; ++d) {
+    if (d < 4 && d >= C.n_base) continue;  // a direction left out keeps no task and no slot (root_slot -1)
     const int ld = d < 4 ? 0 : d - 3;
     std::vector<char> rel(nb, 0);
     for (int l = 0; l < nb; ++l)
@@ -243,7 +247,7 @@ inline SweepSchedule build_sweep_schedule(const SweepTopo& C, bool typed_rounds 
   out.n_rounds = n_rounds;
   out.n_slots = n_slots;
   out.heavy_mask = typed_rounds ? heavy_mask : 0xffffffffu;
-  for (int d = 0; d < n_dir && d < 32; ++d) out.root_slot[d] = slot_of[d][0];
+  for (int d = 0; d < n_dir && d < 32; ++d) out.root_slot[d] = slot_of[d][0];  // -1: direction left out
   return out;
 }
 

@@ -461,6 +461,10 @@ void hb_nlp_hess_l_release(int mem);
  *   info[40]      n_rounds, n_slots, n_tasks, n_heavy_tasks, heavy_mask, seed_mask, root_slot[27] */
 int hb_debug_sweep_schedule(int32_t nb, const int32_t* parent, int32_t foot_l, int32_t foot_r, int32_t chest,
                             int32_t typed, int32_t* tasks, int32_t* info);
+/* The same with n_base (0..4) of the four base quaternion directions in the sweep; hb_debug_sweep_schedule keeps all
+ * four.  The kinematics kernel runs the schedule with none (its quaternion columns are closed-form). */
+int hb_debug_sweep_schedule_n_base(int32_t nb, const int32_t* parent, int32_t foot_l, int32_t foot_r, int32_t chest,
+                                   int32_t typed, int32_t n_base, int32_t* tasks, int32_t* info);
 
 const char* hb_last_error(void);
 
