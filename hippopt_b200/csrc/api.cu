@@ -1025,6 +1025,54 @@ extern "C" int hb_host_free(void* ptr) {
 
 // ---------------------------------------------------------------------------------------------
 // batched LU of the KKT stage blocks (lu.cu)
+
+// The kernel variant both launch paths use for (n, batch, nrhs) on a device with `sms` SMs:
+//   rpt, mb   lu_factor_kernel<RPT, MB>: panel rows per thread (n <= RPT * LU_THREADS) and CTAs per SM the register
+//             allocation is tuned for -- the 128-register MB = 2 build when the batch exceeds one CTA per SM and two
+//             CTAs fit an SM's shared memory
+//   ct        lu_solve_staged_kernel<CT> (8-column tiles of right-hand sides per CTA), 0 = the unstaged lu_solve_kernel
+//   chunks    column chunks (CTAs) per matrix of the solve
+struct LuPlan {
+  int rpt, mb, ct, chunks;
+};
+static LuPlan lu_plan(int64_t n, int64_t batch, int64_t nrhs, int sms, bool unstaged) {
+  LuPlan p{};
+  const size_t smem = hb::lu_factor_smem((int)n);
+  const bool two = batch > sms && 2 * (smem + 2048) <= 227 * 1024;
+  p.rpt = n <= hb::LU_THREADS ? 1 : n <= 2 * hb::LU_THREADS ? 2 : 3;
+  p.mb = two && p.rpt < 3 ? 2 : 1;
+  // staged substitution (lu.cu): 32 or 24 right-hand sides per CTA while two CTAs fit an SM, else 32 / 24 / 16 / 8 on
+  // one CTA per SM
+  const size_t two_per_sm = (233472 / 2) - 1024 - 2560, one_per_sm = 232448 - 1024 - 2560;  // minus the static arrays
+  p.ct = 0;  // 8-column tiles per CTA
+  if (!unstaged) {
+    if (hb::lu_staged_smem((int)n, 4) <= two_per_sm) p.ct = 4;
+    else if (hb::lu_staged_smem((int)n, 3) <= two_per_sm) p.ct = 3;
+    else if (hb::lu_staged_smem((int)n, 4) <= one_per_sm) p.ct = 4;
+    else if (hb::lu_staged_smem((int)n, 3) <= one_per_sm) p.ct = 3;
+    else if (hb::lu_staged_smem((int)n, 2) <= one_per_sm) p.ct = 2;
+    else if (hb::lu_staged_smem((int)n, 1) <= one_per_sm) p.ct = 1;
+  }
+  const int64_t rc = p.ct > 0 ? 8 * p.ct : hb::LU_RC;
+  p.chunks = (int)((nrhs + rc - 1) / rc);
+  return p;
+}
+static bool lu_solve_unstaged() {
+  static const bool unstaged = getenv("HB_LU_SOLVE_UNSTAGED") != nullptr;  // A/B timing against the round-1 kernel
+  return unstaged;
+}
+
+extern "C" int hb_debug_lu_plan(int64_t n, int64_t batch, int64_t nrhs, int32_t sms, int32_t* out) {
+  if (!out || n <= 0 || n > 768 || batch <= 0 || nrhs <= 0 || sms <= 0)
+    return fail(HB_ERR_INVALID, "hb_debug_lu_plan: need 0 < n <= 768, batch > 0, nrhs > 0, sms > 0, out");
+  const LuPlan p = lu_plan(n, batch, nrhs, sms, lu_solve_unstaged());
+  out[0] = p.rpt;
+  out[1] = p.mb;
+  out[2] = p.ct;
+  out[3] = p.chunks;
+  return HB_OK;
+}
+
 extern "C" int hb_lu_factor_batched(double* A, int32_t* piv, int32_t* info, int64_t n, int64_t batch, void* stream) {
   if (!A || !piv || !info) return fail(HB_ERR_INVALID, "hb_lu_factor_batched: null argument");
   if (n <= 0 || n > 768 || batch <= 0) return fail(HB_ERR_INVALID, "hb_lu_factor_batched: need 0 < n <= 768, batch > 0");
@@ -1032,20 +1080,14 @@ extern "C" int hb_lu_factor_batched(double* A, int32_t* piv, int32_t* info, int6
   int dev = 0;
   CUDA_TRY(cudaGetDevice(&dev));
   CUDA_TRY(ensure_kernel_attributes(dev));
-  const int sms = device_sms[dev];
+  const LuPlan p = lu_plan(n, batch, 1, device_sms[dev], lu_solve_unstaged());  // (the solve fields are not used here)
   cudaStream_t st = (cudaStream_t)stream;
   const unsigned grid = (unsigned)batch;
-  // more than one block per SM and two of them fit (shared memory): the 128-register variant
-  const bool two = batch > sms && 2 * (smem + 2048) <= 227 * 1024;
-  if (n <= hb::LU_THREADS) {
-    if (two) hb::lu_factor_kernel<1, 2><<<grid, hb::LU_THREADS, smem, st>>>(A, piv, info, (int)n);
-    else hb::lu_factor_kernel<1, 1><<<grid, hb::LU_THREADS, smem, st>>>(A, piv, info, (int)n);
-  } else if (n <= 2 * hb::LU_THREADS) {
-    if (two) hb::lu_factor_kernel<2, 2><<<grid, hb::LU_THREADS, smem, st>>>(A, piv, info, (int)n);
-    else hb::lu_factor_kernel<2, 1><<<grid, hb::LU_THREADS, smem, st>>>(A, piv, info, (int)n);
-  } else {
-    hb::lu_factor_kernel<3, 1><<<grid, hb::LU_THREADS, smem, st>>>(A, piv, info, (int)n);
-  }
+  if (p.rpt == 1 && p.mb == 2) hb::lu_factor_kernel<1, 2><<<grid, hb::LU_THREADS, smem, st>>>(A, piv, info, (int)n);
+  else if (p.rpt == 1) hb::lu_factor_kernel<1, 1><<<grid, hb::LU_THREADS, smem, st>>>(A, piv, info, (int)n);
+  else if (p.rpt == 2 && p.mb == 2) hb::lu_factor_kernel<2, 2><<<grid, hb::LU_THREADS, smem, st>>>(A, piv, info, (int)n);
+  else if (p.rpt == 2) hb::lu_factor_kernel<2, 1><<<grid, hb::LU_THREADS, smem, st>>>(A, piv, info, (int)n);
+  else hb::lu_factor_kernel<3, 1><<<grid, hb::LU_THREADS, smem, st>>>(A, piv, info, (int)n);
   CUDA_TRY(cudaGetLastError());
   return HB_OK;
 }
@@ -1055,36 +1097,23 @@ extern "C" int hb_lu_solve_batched(const double* LU, const int32_t* piv, double*
   if (!LU || !piv || !Bm) return fail(HB_ERR_INVALID, "hb_lu_solve_batched: null argument");
   if (n <= 0 || n > 768 || batch <= 0 || nrhs <= 0)
     return fail(HB_ERR_INVALID, "hb_lu_solve_batched: need 0 < n <= 768, batch > 0, nrhs > 0");
-  {
-    int dev = 0;
-    CUDA_TRY(cudaGetDevice(&dev));
-    CUDA_TRY(ensure_kernel_attributes(dev));
-  }
-  static const bool unstaged = getenv("HB_LU_SOLVE_UNSTAGED") != nullptr;  // A/B timing against the round-1 kernel
-  // staged substitution (lu.cu): 24 right-hand sides per CTA while two CTAs fit an SM, else 16 / 8 on one CTA per SM
-  const size_t two_per_sm = (233472 / 2) - 1024 - 2560, one_per_sm = 232448 - 1024 - 2560;  // minus the static arrays
-  int ct = 0;  // 8-column tiles per CTA
-  if (!unstaged) {
-    if (hb::lu_staged_smem((int)n, 4) <= two_per_sm) ct = 4;
-    else if (hb::lu_staged_smem((int)n, 3) <= two_per_sm) ct = 3;
-    else if (hb::lu_staged_smem((int)n, 4) <= one_per_sm) ct = 4;
-    else if (hb::lu_staged_smem((int)n, 3) <= one_per_sm) ct = 3;
-    else if (hb::lu_staged_smem((int)n, 2) <= one_per_sm) ct = 2;
-    else if (hb::lu_staged_smem((int)n, 1) <= one_per_sm) ct = 1;
-  }
-  if (ct > 0) {
-    const size_t smem = hb::lu_staged_smem((int)n, ct);
-    const int n_chunks = (int)((nrhs + 8 * ct - 1) / (8 * ct));
+  int dev = 0;
+  CUDA_TRY(cudaGetDevice(&dev));
+  CUDA_TRY(ensure_kernel_attributes(dev));
+  const LuPlan p = lu_plan(n, batch, nrhs, device_sms[dev], lu_solve_unstaged());
+  if (p.ct > 0) {
+    const size_t smem = hb::lu_staged_smem((int)n, p.ct);
+    const int n_chunks = p.chunks;
     const unsigned grid = (unsigned)(batch * n_chunks);
-    if (ct == 4) hb::lu_solve_staged_kernel<4><<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs, n_chunks);
-    else if (ct == 3) hb::lu_solve_staged_kernel<3><<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs, n_chunks);
-    else if (ct == 2) hb::lu_solve_staged_kernel<2><<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs, n_chunks);
+    if (p.ct == 4) hb::lu_solve_staged_kernel<4><<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs, n_chunks);
+    else if (p.ct == 3) hb::lu_solve_staged_kernel<3><<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs, n_chunks);
+    else if (p.ct == 2) hb::lu_solve_staged_kernel<2><<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs, n_chunks);
     else hb::lu_solve_staged_kernel<1><<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs, n_chunks);
     CUDA_TRY(cudaGetLastError());
     return HB_OK;
   }
   const size_t smem = (size_t)n * (hb::LU_RC + 1) * sizeof(double);
-  const dim3 grid((unsigned)batch, (unsigned)((nrhs + hb::LU_RC - 1) / hb::LU_RC));
+  const dim3 grid((unsigned)batch, (unsigned)p.chunks);
   hb::lu_solve_kernel<<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs);
   CUDA_TRY(cudaGetLastError());
   return HB_OK;

@@ -311,6 +311,11 @@ int hb_profile_read(hb_handle h, double* ms3, int64_t* n_evals);
 int hb_lu_factor_batched(double* A, int32_t* piv, int32_t* info, int64_t n, int64_t batch, void* stream);
 int hb_lu_solve_batched(const double* LU, const int32_t* piv, double* Bm, int64_t n, int64_t nrhs, int64_t batch,
                         void* stream);
+/* Host-only: the kernel variants hb_lu_factor_batched / hb_lu_solve_batched launch for (n, batch, nrhs) on a device
+ * with `sms` SMs (the same function picks them), for tests that must know which variant a case runs.
+ *   out[4]  RPT (panel rows per thread), MB (CTAs per SM of the factor kernel's register budget), ct (8-column tiles of
+ *           right-hand sides per CTA of the staged solve; 0 = the unstaged kernel), column chunks per matrix */
+int hb_debug_lu_plan(int64_t n, int64_t batch, int64_t nrhs, int32_t sms, int32_t* out);
 
 /* One stage of the block-tridiagonal KKT sweep (hippopt_b200/kkt.py::StageKKT) assembled in one launch from the CCS
  * value arrays: the dense symmetric stage block D (batch x nb x nb) = hess_l block + J_I^T Sigma J_I + shifts, with the

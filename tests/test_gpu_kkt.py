@@ -104,3 +104,54 @@ def test_stage_sweep_on_evaluated_values(model, built_library, periodic):
     # and the sweep is reproducible bit for bit
     dx2, dl2 = kkt.solve(hv, jv, sig, delta, 1e-9, RXm, REm)
     assert torch.equal(dx2, dxm) and torch.equal(dl2, dlm)
+
+
+@pytest.mark.parametrize("periodic", [False, True])
+def test_stage_sweep_at_the_production_chunk(model, built_library, periodic):
+    """The default chunk of StageKKT.solve (2 x SM count instances) on 2 sms + 3 instances: one full chunk, whose
+    stage blocks the MB = 2 factor kernel takes, then a ragged chunk of 3 on the MB = 1 kernel.  Every instance's
+    residual against the dense matrix, and a dense solve on both sides of the chunk boundary and at the ends."""
+    import ctypes
+
+    from hippopt_b200.evaluator import ALL, KinoEvaluator
+    from hippopt_b200.kino_layout import KinoSettings
+    from hippopt_b200.kkt import StageKKT
+    from hippopt_b200.workloads import kino_batch
+
+    d = dev()
+    sms = torch.cuda.get_device_properties(d).multi_processor_count
+    chunk = 2 * sms
+    N, B = 4, chunk + 3
+    ev = KinoEvaluator(model, KinoSettings(horizon=N, final_state_constraint=True, periodicity_constraint=periodic))
+    x, p, lam, sigma = kino_batch(ev.layout, model, B, seed=4, noise=0.05)
+    lb, ub = ev.bounds(p)
+    out = ev.eval(ALL, *(torch.tensor(a, device=d) for a in (x, p, lam, np.ones(B))))
+    hv, jv = out["hess"].clone(), out["jac"].clone()
+    kkt, eq, ine = StageKKT.for_evaluator(ev, lb[0], ub[0], device=d, linalg="hb")
+    assert kkt.fused
+    plan = (ctypes.c_int32 * 4)()
+    for batch, mb in ((chunk, 2), (3, 1)):
+        assert built_library.hb_debug_lu_plan(kkt.nb, batch, 1, sms, plan) == 0 and plan[1] == mb, (kkt.nb, batch)
+    g = torch.Generator().manual_seed(2)
+    sig = (torch.rand((B, len(ine)), generator=g, dtype=torch.float64) * 10.0).to(d)
+    delta = torch.full((B,), 1e-2, dtype=torch.float64, device=d)
+    rx = torch.randn((B, ev.n_x), generator=g, dtype=torch.float64).to(d)
+    rE = torch.randn((B, len(eq)), generator=g, dtype=torch.float64).to(d)
+    rE[:, torch.as_tensor(kkt.dead_eq, device=d)] = 0.0
+    u = torch.cat(kkt.solve(hv, jv, sig, delta, 1e-9, rx, rE), dim=1)  # default chunk
+    rhs = torch.cat([rx, rE], dim=1)
+    jc, jr = ev.jac_sparsity()
+    hc, hr = ev.hess_sparsity()
+    dense_check = {0, chunk - 1, chunk, B - 1}
+    for s in range(0, B, 32):
+        sl = slice(s, min(s + 32, B))
+        K = kkt.dense_matrix(hv[sl], jv[sl], sig[sl], delta[sl], 1e-9, eq, ine, jc, jr, hc, hr)
+        scale = u[sl].abs().amax(dim=1, keepdim=True)
+        res = torch.einsum("bij,bj->bi", K, u[sl]) - rhs[sl]
+        worst = (res.abs() / scale).amax(dim=1)
+        assert worst.max().item() < 1e-12, (s + int(worst.argmax()), worst.max().item())
+        for i in sorted(dense_check & set(range(sl.start, sl.stop))):
+            ref = torch.linalg.solve(K[i - s], rhs[i])
+            err = ((u[i] - ref).abs().max() / ref.abs().max()).item()
+            assert err < 1e-6, (i, err)  # cond(K) ~ 1e11: the residual is the sharp check
+        del K
