@@ -1073,6 +1073,35 @@ extern "C" int hb_debug_lu_plan(int64_t n, int64_t batch, int64_t nrhs, int32_t 
   return HB_OK;
 }
 
+namespace hb {
+// one thread per point: the production surface and frame jets, unchanged, written out for the tests
+__global__ void debug_smooth_terrain_kernel(const double* __restrict__ tp, const double* __restrict__ pts, long n,
+                                            double* __restrict__ out) {
+  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const double* t = tp + 10 * i;
+  const double x = pts[3 * i], y = pts[3 * i + 1], z = pts[3 * i + 2];
+  double* o = out + HB_SMOOTH_TERRAIN_OUT * i;
+  const BJ<4> T = smooth_steps_surface(t, x, y);
+  for (int k = 0; k < BJ<4>::SIZE; ++k) o[k] = T.c[k];
+  TFrame F;
+  smooth_terrain_frame(t, x, y, z, F);
+  const TJ* f[18] = {&F.h, &F.gx, &F.gy, &F.n[0], &F.n[1], &F.n[2], &F.xh[0], &F.xh[1], &F.xh[2],
+                     &F.yh[0], &F.yh[1], &F.yh[2], &F.Dn[0][0], &F.Dn[0][1], &F.Dn[1][0], &F.Dn[1][1],
+                     &F.Dn[2][0], &F.Dn[2][1]};
+  for (int a = 0; a < 18; ++a)
+    for (int k = 0; k < 10; ++k) o[BJ<4>::SIZE + 10 * a + k] = f[a]->c[k];
+}
+static_assert(BJ<4>::SIZE + 18 * 10 == HB_SMOOTH_TERRAIN_OUT, "hb_debug_smooth_terrain output layout");
+}  // namespace hb
+
+extern "C" int hb_debug_smooth_terrain(const double* tp, const double* pts, int64_t n, double* out, void* stream) {
+  if (!tp || !pts || !out || n <= 0) return fail(HB_ERR_INVALID, "hb_debug_smooth_terrain: null argument or n <= 0");
+  hb::debug_smooth_terrain_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(tp, pts, (long)n, out);
+  CUDA_TRY(cudaGetLastError());
+  return HB_OK;
+}
+
 extern "C" int hb_lu_factor_batched(double* A, int32_t* piv, int32_t* info, int64_t n, int64_t batch, void* stream) {
   if (!A || !piv || !info) return fail(HB_ERR_INVALID, "hb_lu_factor_batched: null argument");
   if (n <= 0 || n > 768 || batch <= 0) return fail(HB_ERR_INVALID, "hb_lu_factor_batched: need 0 < n <= 768, batch > 0");

@@ -471,6 +471,15 @@ int hb_debug_sweep_schedule(int32_t nb, const int32_t* parent, int32_t foot_l, i
 int hb_debug_sweep_schedule_n_base(int32_t nb, const int32_t* parent, int32_t foot_l, int32_t foot_r, int32_t chest,
                                    int32_t typed, int32_t n_base, int32_t* tasks, int32_t* info);
 
+/* The smooth-step terrain jets of the contact kernel (hippopt_b200/csrc/kino_smooth.cuh), evaluated by the production
+ * smooth_steps_surface and smooth_terrain_frame at n points, for tests that compare them with a symbolic reference.
+ *   tp   device [n][10]   terrain parameters of each point, (l, w, height, ox, oy) x 2
+ *   pts  device [n][3]    (x, y, z)
+ *   out  device [n][HB_SMOOTH_TERRAIN_OUT]  the 15 normalised coefficients of the order-4 surface jet T(x, y), then the
+ *        TFrame fields in declaration order, 10 trivariate coefficients each: h, gx, gy, n[3], xh[3], yh[3], Dn[3][2] */
+#define HB_SMOOTH_TERRAIN_OUT 195
+int hb_debug_smooth_terrain(const double* tp, const double* pts, int64_t n, double* out, void* stream);
+
 const char* hb_last_error(void);
 
 /* fp64 FMA throughput probe (TFLOP/s) used as roofline denominator when none is published */

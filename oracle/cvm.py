@@ -133,11 +133,15 @@ def _program(tape: sx.Tape, seed_idx):
 _numpy_eval, _numpy_eval_fwd = sx.Tape.eval, sx.Tape.eval_fwd
 
 
-def _c_eval(self, X):
+def _c_eval(self, X, dtype=np.float64):
+    if np.dtype(dtype) != np.float64:  # the C VM computes in double only
+        return _numpy_eval(self, X, dtype)
     return _program(self, ()).run(X)[0]
 
 
-def _c_eval_fwd(self, X, seed_idx):
+def _c_eval_fwd(self, X, seed_idx, dtype=np.float64):
+    if np.dtype(dtype) != np.float64:
+        return _numpy_eval_fwd(self, X, seed_idx, dtype)
     vals, tang = _program(self, seed_idx).run(X)
     return vals, tang
 

@@ -108,9 +108,9 @@ class NLP:
             groups.setdefault(id(app[0]), []).append(app)
         return list(groups.values())
 
-    def _w(self, X, P):
-        X = np.atleast_2d(np.asarray(X, dtype=np.float64))
-        P = np.atleast_2d(np.asarray(P, dtype=np.float64))
+    def _w(self, X, P, dtype=np.float64):
+        X = np.atleast_2d(np.asarray(X, dtype=dtype))
+        P = np.atleast_2d(np.asarray(P, dtype=dtype))
         assert X.shape[1] == self.n_x and P.shape[1] == self.n_p
         if P.shape[0] == 1 and X.shape[0] > 1:
             P = np.repeat(P, X.shape[0], axis=0)
@@ -124,65 +124,67 @@ class NLP:
         return U.reshape(-1, idx.shape[1]), idx
 
     # -- values ---------------------------------------------------------------------
-    def eval_g(self, X, P):
-        W = self._w(X, P)
+    # Every eval_* takes ``dtype``, the floating type of the whole evaluation (Tape.eval): np.longdouble gives an
+    # extended-precision reference, finite where the float64 tapes form 0 * inf far from a smooth step.
+    def eval_g(self, X, P, dtype=np.float64):
+        W = self._w(X, P, dtype)
         B = W.shape[0]
-        out = np.zeros((B, self.m))
+        out = np.zeros((B, self.m), dtype=dtype)
         for apps in self._group(self.row_apps):
             t = apps[0][0]
             U, idx = self._gather(W, apps)
-            vals = t.tape.eval(U).reshape(B, len(apps), -1)
+            vals = t.tape.eval(U, dtype).reshape(B, len(apps), -1)
             for a, (_, _, off) in enumerate(apps):
                 out[:, off:off + vals.shape[2]] = vals[:, a, :]
         return out
 
-    def eval_bounds(self, P):
-        P = np.atleast_2d(np.asarray(P, dtype=np.float64))
-        W = np.concatenate([np.zeros((P.shape[0], self.n_x)), P], axis=1)
+    def eval_bounds(self, P, dtype=np.float64):
+        P = np.atleast_2d(np.asarray(P, dtype=dtype))
+        W = np.concatenate([np.zeros((P.shape[0], self.n_x), dtype=dtype), P], axis=1)
         B = W.shape[0]
-        lb = np.zeros((B, self.m))
-        ub = np.zeros((B, self.m))
+        lb = np.zeros((B, self.m), dtype=dtype)
+        ub = np.zeros((B, self.m), dtype=dtype)
         for apps in self._group(self.row_apps):
             t = apps[0][0]
             n = len(t.rows)
             U, idx = self._gather(W, apps)
-            vals = t.bound_tape.eval(U).reshape(B, len(apps), -1)
+            vals = t.bound_tape.eval(U, dtype).reshape(B, len(apps), -1)
             for a, (_, _, off) in enumerate(apps):
                 lb[:, off:off + n] = vals[:, a, :n]
                 ub[:, off:off + n] = vals[:, a, n:]
         return lb, ub
 
-    def eval_f(self, X, P):
-        W = self._w(X, P)
+    def eval_f(self, X, P, dtype=np.float64):
+        W = self._w(X, P, dtype)
         B = W.shape[0]
-        f = np.zeros(B)
+        f = np.zeros(B, dtype=dtype)
         # accumulate in recording order, like ``self._cost += input_cost`` (opti_solver.py:556-559)
         cache = {}
         for apps in self._group(self.cost_apps):
             U, _ = self._gather(W, apps)
-            vals = apps[0][0].tape.eval(U).reshape(B, len(apps))
+            vals = apps[0][0].tape.eval(U, dtype).reshape(B, len(apps))
             for a, app in enumerate(apps):
                 cache[id(app)] = vals[:, a]
         for app in self.cost_apps:
             f = f + app[2] * cache[id(app)]
         return f
 
-    def eval_cost_terms(self, X, P):
-        W = self._w(X, P)
+    def eval_cost_terms(self, X, P, dtype=np.float64):
+        W = self._w(X, P, dtype)
         B = W.shape[0]
-        out = np.zeros((B, len(self.cost_apps)))
+        out = np.zeros((B, len(self.cost_apps)), dtype=dtype)
         pos = {id(app): i for i, app in enumerate(self.cost_apps)}
         for apps in self._group(self.cost_apps):
             U, _ = self._gather(W, apps)
-            vals = apps[0][0].tape.eval(U).reshape(B, len(apps))
+            vals = apps[0][0].tape.eval(U, dtype).reshape(B, len(apps))
             for a, app in enumerate(apps):
                 out[:, pos[id(app)]] = app[2] * vals[:, a]
         return out
 
-    def eval_grad_f(self, X, P):
-        W = self._w(X, P)
+    def eval_grad_f(self, X, P, dtype=np.float64):
+        W = self._w(X, P, dtype)
         B = W.shape[0]
-        grad = np.zeros((B, self.n_x))
+        grad = np.zeros((B, self.n_x), dtype=dtype)
         for apps in self._group(self.cost_apps):
             t = apps[0][0]
             U, idx = self._gather(W, apps)
@@ -191,7 +193,7 @@ class NLP:
             xin = [i for i in xin if i in pat]
             if not xin:
                 continue
-            _, tang = t.tape.eval_fwd(U, xin)
+            _, tang = t.tape.eval_fwd(U, xin, dtype)
             tang = tang.reshape(B, len(apps), len(xin))
             for a, (_, binding, scale) in enumerate(apps):
                 np.add.at(grad, (slice(None), binding[xin]), scale * tang[:, a, :])
@@ -222,18 +224,18 @@ class NLP:
         self._jac = (colind, rows[order], cols[order], uniq)
         return self._jac
 
-    def eval_jac(self, X, P):
+    def eval_jac(self, X, P, dtype=np.float64):
         colind, row, col, keys = self.jac_structure()
-        W = self._w(X, P)
+        W = self._w(X, P, dtype)
         B = W.shape[0]
-        vals = np.zeros((B, len(row)))
+        vals = np.zeros((B, len(row)), dtype=dtype)
         for apps in self._group(self.row_apps):
             t = apps[0][0]
             U, idx = self._gather(W, apps)
             xin = sorted({i for deps in t.pattern for i in deps if np.all(idx[:, i] < self.n_x)})
             if not xin:
                 continue
-            _, tang = t.tape.eval_fwd(U, xin)
+            _, tang = t.tape.eval_fwd(U, xin, dtype)
             tang = tang.reshape(B, len(apps), len(t.rows), len(xin))
             plan = self._plans.get(("jac", id(t)))
             if plan is None:  # scatter plan (application, row, direction) -> CCS slot, built once
@@ -280,13 +282,13 @@ class NLP:
         self._hess = (colind, row, col, keys)
         return self._hess
 
-    def eval_hess(self, X, P, lam, sigma=1.0):
+    def eval_hess(self, X, P, lam, sigma=1.0, dtype=np.float64):
         colind, row, col, keys = self.hess_structure()
-        W = self._w(X, P)
+        W = self._w(X, P, dtype)
         B = W.shape[0]
-        lam = np.atleast_2d(np.asarray(lam, dtype=np.float64))
-        sigma = np.broadcast_to(np.asarray(sigma, dtype=np.float64), (B,))
-        vals = np.zeros((B, len(keys)))
+        lam = np.atleast_2d(np.asarray(lam, dtype=dtype))
+        sigma = np.broadcast_to(np.asarray(sigma, dtype=dtype), (B,))
+        vals = np.zeros((B, len(keys)), dtype=dtype)
 
         def run(apps, lam_of_app):
             t = apps[0][0]
@@ -296,7 +298,7 @@ class NLP:
             if not xin:
                 return
             L = np.stack([lam_of_app(app) for app in apps], axis=1).reshape(B * len(apps), -1)
-            _, tang = tape.eval_fwd(np.concatenate([U, L], axis=1), xin)
+            _, tang = tape.eval_fwd(np.concatenate([U, L], axis=1), xin, dtype)
             tang = tang.reshape(B, len(apps), len(t.inputs), len(xin))
             plan = self._plans.get(("hess", id(t)))
             if plan is None:
@@ -332,17 +334,17 @@ class NLP:
         return vals
 
     # -- dense helpers for tests -----------------------------------------------------------
-    def dense_jac(self, X, P):
+    def dense_jac(self, X, P, dtype=np.float64):
         colind, row, col, _ = self.jac_structure()
-        v = self.eval_jac(X, P)
-        out = np.zeros((v.shape[0], self.m, self.n_x))
+        v = self.eval_jac(X, P, dtype)
+        out = np.zeros((v.shape[0], self.m, self.n_x), dtype=dtype)
         out[:, row, col] = v
         return out
 
-    def dense_hess(self, X, P, lam, sigma=1.0):
+    def dense_hess(self, X, P, lam, sigma=1.0, dtype=np.float64):
         colind, row, col, _ = self.hess_structure()
-        v = self.eval_hess(X, P, lam, sigma)
-        out = np.zeros((v.shape[0], self.n_x, self.n_x))
+        v = self.eval_hess(X, P, lam, sigma, dtype)
+        out = np.zeros((v.shape[0], self.n_x, self.n_x), dtype=dtype)
         out[:, row, col] = v
         out[:, col, row] = v
         return out

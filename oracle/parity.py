@@ -123,7 +123,7 @@ def check_all(got: dict, ref: dict, jac_pattern, hess_pattern, x, rtol=RTOL, key
     return worst
 
 
-def reference_outputs(nlp, x, p, lam, sigma):
-    """The five nlpsol oracle functions evaluated by the CPU oracle (oracle/nlp.py)."""
-    return {"f": nlp.eval_f(x, p), "grad_f": nlp.eval_grad_f(x, p), "g": nlp.eval_g(x, p),
-            "jac": nlp.eval_jac(x, p), "hess": nlp.eval_hess(x, p, lam, sigma)}
+def reference_outputs(nlp, x, p, lam, sigma, dtype=np.float64):
+    """The five nlpsol oracle functions evaluated by the CPU oracle (oracle/nlp.py) in floating type ``dtype``."""
+    return {"f": nlp.eval_f(x, p, dtype), "grad_f": nlp.eval_grad_f(x, p, dtype), "g": nlp.eval_g(x, p, dtype),
+            "jac": nlp.eval_jac(x, p, dtype), "hess": nlp.eval_hess(x, p, lam, sigma, dtype)}

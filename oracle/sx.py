@@ -449,22 +449,25 @@ class Tape:
         self.n_ops = sum(1 for n in self.order if n.op not in (OP_CONST, OP_SYM))
 
     # values only ------------------------------------------------------------------
-    def eval(self, X: np.ndarray) -> np.ndarray:
-        X = np.atleast_2d(np.asarray(X, dtype=np.float64))
+    # ``dtype`` is the floating type of the whole evaluation (inputs, every intermediate, tangents and outputs);
+    # np.longdouble runs the same tape with a 64-bit mantissa where the platform has one.  The tape's constants
+    # stay the float64 numbers the graph was built with.
+    def eval(self, X: np.ndarray, dtype=np.float64) -> np.ndarray:
+        X = np.atleast_2d(np.asarray(X, dtype=dtype))
         B = X.shape[0]
         w: dict[int, np.ndarray | float] = {}
         for k, n in enumerate(self.order):
             w[n.id] = _apply(n, w, X, self.in_index)
             for nid in self.free_after[k]:
                 w.pop(nid, None)
-        out = np.empty((B, len(self.outputs)))
+        out = np.empty((B, len(self.outputs)), dtype=dtype)
         for j, o in enumerate(self.outputs):
             out[:, j] = w[o.id]
         return out
 
     # values + forward-mode tangents along the unit directions of inputs[seed_idx] ---
-    def eval_fwd(self, X: np.ndarray, seed_idx: Sequence[int]):
-        X = np.atleast_2d(np.asarray(X, dtype=np.float64))
+    def eval_fwd(self, X: np.ndarray, seed_idx: Sequence[int], dtype=np.float64):
+        X = np.atleast_2d(np.asarray(X, dtype=dtype))
         B = X.shape[0]
         D = len(seed_idx)
         seed_pos = {int(i): d for d, i in enumerate(seed_idx)}
@@ -481,7 +484,7 @@ class Tape:
                 if d is None:
                     t[n.id] = None
                 else:
-                    tt = np.zeros((B, D))
+                    tt = np.zeros((B, D), dtype=dtype)
                     tt[:, d] = 1.0
                     t[n.id] = tt
             else:
@@ -491,8 +494,8 @@ class Tape:
             for nid in self.free_after[k]:
                 w.pop(nid, None)
                 t.pop(nid, None)
-        vals = np.empty((B, len(self.outputs)))
-        tang = np.zeros((B, len(self.outputs), D))
+        vals = np.empty((B, len(self.outputs)), dtype=dtype)
+        tang = np.zeros((B, len(self.outputs), D), dtype=dtype)
         for j, o in enumerate(self.outputs):
             vals[:, j] = w[o.id]
             if t[o.id] is not None:
