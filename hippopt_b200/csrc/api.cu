@@ -511,7 +511,8 @@ extern "C" int hb_kino_create(const int32_t* icfg, const double* dcfg, const int
   if (e == cudaSuccess) {
     // per-point Hessian terms of the planar contact kernel, in the order kino_contact.cu lists them: 11 complementarity /
     // friction / swing terms, 6 control regularisations, 12 momentum cross terms -> 29 local entries per point, padded to 32
-    std::vector<int16_t> pt(8 * 32, -1);
+    // followed by the 7 local entries per lane of the least-squares cost rows, padded to 8, in the kernel's slot order
+    std::vector<int16_t> pt(8 * 32 + 32 * 8, -1);
     enum { V = 0, FD = 3, P = 6, F = 9, U = 12, COM = 120, NV = 129 };
     for (int i = 0; i < 8; ++i) {
       const int o = 15 * i;
@@ -539,6 +540,27 @@ extern "C" int hb_kino_create(const int32_t* icfg, const double* dcfg, const int
           term(COM + a, o + F + bb);
         }
     }
+    int16_t* ls = pt.data() + 8 * 32;
+    for (int lane = 0; lane < 32; ++lane) {
+      auto entry = [&](int pi, int ci, int pj, int cj) { return hc_index[(15 * pi + ci) * NV + 15 * pj + cj]; };
+      for (int u = 0; u < 4; ++u) {  // p_c of points (a, (a + d) mod 8), t = 36 c + 8 d + a
+        const int t = lane + 32 * u, c = t / 36, q = t % 36, a = q & 7;
+        if (t < 108) ls[8 * lane + u] = entry(a, P + c, (a + (q >> 3)) & 7, P + c);
+      }
+      {  // (p_x, p_y) of points (4 foot + i, 4 foot + j), lane = 16 foot + 4 i + j, where one yaw row holds both points
+        const int foot = lane >> 4, i = (lane >> 2) & 3, j = lane & 3;
+        bool on_row = false;
+        for (int s = 0; s < 2; ++s) {
+          const bool hi = i == C.yaw[s] || i == C.yaw[s + 1], hj = j == C.yaw[s] || j == C.yaw[s + 1];
+          on_row = on_row || (hi && hj);
+        }
+        if (on_row) ls[8 * lane + 4] = entry(4 * foot + i, P, 4 * foot + j, P + 1);
+      }
+      for (int u = 5; u < 7; ++u) {  // f_c of points (a, (a + d) mod 4) of one foot, t = 10 (3 foot + c) + 4 d + a
+        const int t = lane + 32 * (u - 5), foot = t / 30, c = (t / 10) % 3, q = t % 10, a = q & 3;
+        if (t < 60) ls[8 * lane + u] = entry(4 * foot + a, F + c, 4 * foot + ((a + (q >> 2)) & 3), F + c);
+      }
+    }
     e = upload(&h->d_hc_pt, pt.data(), pt.size());
   }
   C.jc_map = h->d_jc;
@@ -558,6 +580,7 @@ extern "C" int hb_kino_create(const int32_t* icfg, const double* dcfg, const int
   h->topo.jc_map = h->d_jc;
   h->topo.hc_index = h->d_hci;
   h->topo.hc_pt = h->d_hc_pt;
+  h->topo.hc_ls = h->d_hc_pt ? h->d_hc_pt + 8 * 32 : nullptr;
   h->topo.hc_map = h->d_hc;
   {
     // 4 warps per CTA; the kinematics kernels keep one branch accumulator per body whose children do not
@@ -762,12 +785,13 @@ extern "C" int hb_eval(hb_handle h, uint32_t mask, const double* x, const double
     st_contact = h->aux;
   }
   {
-    const size_t smem = (size_t)hb::contact_smem_layout(C.n_hc).total * sizeof(double) * warps_per_block;
     {
       int dev = 0;
       CUDA_TRY(cudaGetDevice(&dev));
       CUDA_TRY(ensure_kernel_attributes(dev));
     }
+    const size_t smem = (size_t)(C.kind == 1 ? hb::pose_contact_smem_layout(C.n_hc) : hb::kino_contact_smem_layout(C.n_hc)).total *
+                        sizeof(double) * warps_per_block;
     if (C.kind == 1) {
       hb::pose_contact_kernel<<<grid, 32 * warps_per_block, smem, st>>>(h->dev, mask, x, p, (long)p_stride, lam_g, sigma,
                                                                        d_fpart, grad_f, g, jac_vals, hess_vals,
@@ -1439,7 +1463,7 @@ extern "C" int hb_eval_cost_terms(hb_handle h, const double* x, const double* p,
   int dev = 0;
   CUDA_TRY(cudaGetDevice(&dev));
   CUDA_TRY(ensure_kernel_attributes(dev));
-  const size_t smem_c = (size_t)hb::contact_smem_layout(C.n_hc).total * sizeof(double) * wpb;
+  const size_t smem_c = (size_t)hb::kino_contact_smem_layout(C.n_hc).total * sizeof(double) * wpb;
   if (C.terrain == 0)
     hb::kino_contact_kernel<0><<<grid, 32 * wpb, smem_c, st>>>(h->topo, h->dev, mask, x, p, (long)p_stride, nullptr, nullptr,
                                                               terms, nullptr, nullptr, nullptr, nullptr, (long)batch);

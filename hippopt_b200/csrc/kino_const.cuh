@@ -123,6 +123,8 @@ struct KinTopo {
   const unsigned* hc_list;
   // planar terrain: local Hessian entry of the 29 per-point terms of contact point i (kino_contact.cu), 32 shorts per point
   const short* hc_pt;
+  // local Hessian entries of the least-squares cost rows (kino_contact.cu), 8 shorts per lane; same allocation as hc_pt
+  const short* hc_ls;
   // packed tangent sweep (kino_kin.cu): sched[round * 32 + lane] = task descriptor (see KT_* below)
   const int* sched;
   signed char root_slot[32];  // slot that holds the root totals of direction d after the sweep

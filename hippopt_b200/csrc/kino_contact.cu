@@ -28,11 +28,18 @@
 namespace hb {
 
 enum { NCV = 129, CV_COM = 120, CV_H = 123, LS_ROWS = 31, LS_MAXV = 8 };
+// Hessian-phase inputs of contact point i, parked at park[8 q + i] of the kinodynamic kernel's shared block as soon
+// as they are known: multipliers of the planar (x, y), DCC and friction rows, of the angular momentum dynamics (3),
+// and d tau / d p_z, d2 tau / d p_z2
+enum { PK_L0, PK_L1, PK_LD, PK_LF, PK_LA, PK_DTAU = PK_LA + 3, PK_DDTAU, PK_COUNT };
 
+// Per-warp shared block.  The least-squares row tables (ls_*) are used by the pose-finder kernel only; the
+// kinodynamic kernel sums its least-squares rows in closed form and has the parked Hessian inputs instead
+// (968 doubles per warp at config 3: 7 CTAs of 4 warps fit an SM's shared memory).
 struct ContactSmem {
-  int z, zp, hbuf, gbuf, ls_coef, ls_w, ls_r, ls_var, ls_n, total;
+  int z, zp, hbuf, gbuf, ls_coef, ls_w, ls_r, ls_var, ls_n, park, total;
 };
-__host__ __device__ inline ContactSmem contact_smem_layout(int n_hc) {
+__host__ __device__ inline ContactSmem contact_smem_layout_(int n_hc, bool ls_tables) {
   ContactSmem s;
   int o = 0;
   s.z = o;
@@ -43,19 +50,28 @@ __host__ __device__ inline ContactSmem contact_smem_layout(int n_hc) {
   o += (n_hc + 1) & ~1;
   s.gbuf = o;
   o += NCV + 1;
-  s.ls_coef = o;
-  o += LS_ROWS * LS_MAXV;
-  s.ls_w = o;
-  o += LS_ROWS + 1;
-  s.ls_r = o;
-  o += LS_ROWS + 1;
-  s.ls_var = o;  // ints, two per double slot
-  o += (LS_ROWS * LS_MAXV) / 2 + 1;
-  s.ls_n = o;
-  o += LS_ROWS / 2 + 1;
+  s.ls_coef = s.ls_w = s.ls_r = s.ls_var = s.ls_n = s.park = -1;
+  if (!ls_tables) {
+    s.park = o;
+    o += 8 * PK_COUNT;
+  } else {
+    s.ls_coef = o;
+    o += LS_ROWS * LS_MAXV;
+    s.ls_w = o;
+    o += LS_ROWS + 1;
+    s.ls_r = o;
+    o += LS_ROWS + 1;
+    s.ls_var = o;  // ints, two per double slot
+    o += (LS_ROWS * LS_MAXV) / 2 + 1;
+    s.ls_n = o;
+    o += LS_ROWS / 2 + 1;
+  }
   s.total = o;
   return s;
 }
+// one layout per kernel, so that a launch cannot size the block of the other kernel
+__host__ __device__ inline ContactSmem kino_contact_smem_layout(int n_hc) { return contact_smem_layout_(n_hc, false); }
+__host__ __device__ inline ContactSmem pose_contact_smem_layout(int n_hc) { return contact_smem_layout_(n_hc, true); }
 
 __device__ __forceinline__ double eps3(int a, int b) { return ((b - a + 3) % 3 == 1) ? 1.0 : -1.0; }
 
@@ -96,10 +112,11 @@ __device__ __forceinline__ void linear_state(int j, int& so, int& ro, int& fam_d
 }
 
 // TERRAIN: 0 = PlanarTerrain, 1 = sum of two smooth steps (kino_smooth.cuh)
-// Measured on B200 (planar terrain, full mask): unconstrained 162 registers / 3 CTAs per SM 0.471 ms,
-// 5 CTAs (96 registers) 0.431 ms, 6 CTAs (80 registers, spills) 0.455 ms.
+// CTAs per SM of the planar kernel, kernel time per bench step (config 3, NVIDIA B200 at 1000 W, 1965 MHz, three
+// alternated runs): 5 (96 registers, no spill) 0.241 ms, 6 (80, 12 B spill) 0.224 ms, 7 (72, 8 B spill) 0.213 ms.
+// Shared memory allows 7: 30 976 B per CTA.
 #ifndef CONTACT_MIN_BLOCKS
-#define CONTACT_MIN_BLOCKS 5
+#define CONTACT_MIN_BLOCKS 7
 #endif
 template <int TERRAIN>
 __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) kino_contact_kernel(const __grid_constant__ KinTopo T,
@@ -122,17 +139,13 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
   if (wid >= batch * N) return;
   const long b = wid / N;
   const int k = (int)(wid % N);
-  const ContactSmem L = contact_smem_layout(C.n_hc);
+  const ContactSmem L = kino_contact_smem_layout(C.n_hc);
   double* sm = smem + (size_t)warp * L.total;
   double* zs = sm + L.z;
   double* zp = sm + L.zp;
   double* hbuf = sm + L.hbuf;
   double* gbuf = sm + L.gbuf;
-  double* ls_coef = sm + L.ls_coef;
-  double* ls_w = sm + L.ls_w;
-  double* ls_r = sm + L.ls_r;
-  int* ls_var = reinterpret_cast<int*>(sm + L.ls_var);
-  int* ls_n = reinterpret_cast<int*>(sm + L.ls_n);
+  double* park = sm + L.park;
   const double* xinst = x + b * C.n_x;
   const double* xb = xinst + (long)k * NZ;
   const double* pp = p + b * p_stride;
@@ -142,7 +155,8 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
   const bool want_jac = mask & HB_EVAL_JAC_G, want_hess = mask & HB_EVAL_HESS_L;
   // solution report (hb_eval_cost_terms): fpart is the [batch][N][HB_COST_TERMS] table of named cost values
   const bool want_terms = mask & HB_EVAL_COST_TERMS_BIT;
-  double* ct = want_terms ? fpart + (b * N + k) * HB_COST_TERMS : nullptr;
+  // (the row address is formed where a value is written: kept from here it is a 64-bit value spilled at 72 registers)
+  auto ct = [&](int i) -> double& { return fpart[(b * N + k) * HB_COST_TERMS + i]; };
   double c_swing = 0.0;  // swing-height cost of this lane's point (terrain-dependent block below)
 
   // every global input is requested before the first shared-memory store: a store waits for its load and,
@@ -164,12 +178,13 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
   double* gb = g + b * C.m;
   const double* lb = lam + b * C.m;
   const double sg = want_hess ? sigma[b] : 0.0;
-  const int4 kmaps = *reinterpret_cast<const int4*>(&C.knot_maps[k].jc_base);  // {jc_base, jc_off, jc_cnt, hc_base}
-  const int* jmap = C.jc_map + kmaps.y;
-  double* jb = jac + b * C.nnz_j + kmaps.x;
+  // {jc_base, jc_off, jc_cnt, hc_base} of the knot class: re-read (L1) by each phase that scatters rather than held
+  // in registers from here
+  auto knot_maps = [&]() { return *reinterpret_cast<const int4*>(&C.knot_maps[k].jc_base); };
   auto jput = [&](int e, double v) {
-    const int slot = jmap[e];
-    if (slot >= 0) jb[slot] = v;
+    const int4 km = knot_maps();
+    const int slot = C.jc_map[km.y + e];
+    if (slot >= 0) jac[b * C.nnz_j + km.x + slot] = v;
   };
   auto hadd = [&](int vi, int vj, double v) {
     const int e = C.hc_index[vi * NCV + vj];
@@ -209,19 +224,22 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
       zp[i] = xp_[u];
     }
   }
+  if (want_hess && lane < 8) {
+    double* pk = park + lane;
+    pk[8 * PK_L0] = lam_pl[0];
+    pk[8 * PK_L1] = lam_pl[1];
+    pk[8 * PK_LD] = lam_dcc;
+    pk[8 * PK_LF] = lam_fr;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) pk[8 * (PK_LA + c)] = La[c];
+  }
   for (int i = lane; i < C.n_hc; i += 32) hbuf[i] = 0.0;
   for (int i = lane; i < NCV; i += 32) gbuf[i] = 0.0;
-  if (lane < LS_ROWS) ls_n[lane] = 0;
   __syncwarp();
   HB_PHASE(1, 0);  // inputs loaded and staged
 
   // ------------------------------------------------------------------ per-point quantities (lanes 0..7)
   const int pi_ = lane & 7;
-  const double* zpt = zs + 15 * pi_;
-  const D3 pv = ld3(zpt + Z_V), pfd = ld3(zpt + Z_FD), ppos = ld3(zpt + Z_P), pf = ld3(zpt + Z_F), pu = ld3(zpt + Z_U);
-  const double tau = tanh(kt * ppos.z);
-  const double dtau = kt * (1.0 - tau * tau);          // d tau / d p_z
-  const double ddtau = -2.0 * kt * tau * dtau;         // d2 tau / d p_z2
   double cost = 0.0;
 
   // ------------------------------------------------------------------ g rows
@@ -281,6 +299,10 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
       zs[Z_F + 1] + zs[16 + Z_F] + zs[31 + Z_F] + zs[46 + Z_F] + zs[61 + Z_F] + zs[76 + Z_F] + zs[91 + Z_F] + zs[106 + Z_F],
       zs[Z_F + 2] + zs[17 + Z_F] + zs[32 + Z_F] + zs[47 + Z_F] + zs[62 + Z_F] + zs[77 + Z_F] + zs[92 + Z_F] + zs[107 + Z_F]);
   const D3 comv = ld3(zs + Z_COM);
+  // the point's variables, read here (after the defect and momentum rows) so that they are not live through them
+  const double* zpt = zs + 15 * pi_;
+  const D3 pv = ld3(zpt + Z_V), pfd = ld3(zpt + Z_FD), ppos = ld3(zpt + Z_P), pf = ld3(zpt + Z_F), pu = ld3(zpt + Z_U);
+  const double tau = tanh(kt * ppos.z);
 
   if constexpr (TERRAIN == 1) {
     // ---------------------------------------------------------------- smooth-step terrain (config 5)
@@ -339,6 +361,9 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
         // the 58 entries of this point are listed first and their scatter slots loaded together: one
         // jput() per entry waited for its own map load (19 % of this kernel's stall samples)
         const int pb0 = 846 + 58 * lane;
+        const int4 kmaps = knot_maps();
+        const int* jmap = C.jc_map + kmaps.y;
+        double* jb = jac + b * C.nnz_j + kmaps.x;
         double jv[58];
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
@@ -513,9 +538,9 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
       cost += c_u;
       cost += c_fd;
       if (want_terms) {
-        ct[HB_CT_SWING0 + lane] = c_swing;
-        ct[HB_CT_UV0 + lane] = c_u;
-        ct[HB_CT_FDOT0 + lane] = c_fd;
+        ct(HB_CT_SWING0 + lane) = c_swing;
+        ct(HB_CT_UV0 + lane) = c_u;
+        ct(HB_CT_FDOT0 + lane) = c_fd;
       }
       gp[Z_U] += 2.0 * C.w_u * pu.x;
       gp[Z_U + 1] += 2.0 * C.w_u * pu.y;
@@ -526,7 +551,7 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
     }
   }
   if (want_terms && !k1)  // expressions with apply_to_first_elements = False do not exist at knot 0
-    for (int i = lane; i < HB_CT_FRAME_QUAT; i += 32) ct[i] = 0.0;
+    for (int i = lane; i < HB_CT_FRAME_QUAT; i += 32) ct(i) = 0.0;
   __syncwarp();
   // CoM velocity cost (all knots): sum_c w_c (h_c - ref_c)^2
   {
@@ -537,7 +562,7 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
     }
     if (want_terms) {
       const double t = warp_sum(c_cv);
-      if (lane == 0) ct[HB_CT_COM_VELOCITY] = t;
+      if (lane == 0) ct(HB_CT_COM_VELOCITY) = t;
     }
   }
   if (lane < 3) {
@@ -600,157 +625,174 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
     }
   }
 
+  // The previous knot's variables are dead after the defect rows (last read before the __syncwarp above): the
+  // Jacobian's derived sources and coefficient table take their place here, so that what the Jacobian phase needs
+  // of this lane's point is in shared memory, not held in registers through the least-squares rows.
+  // The point's values are re-read from zs, k_t and k_bs from the parameters (L1): held from the per-point rows to
+  // here and on to the Hessian terms, they were spilled at 72 registers.
+  const double kt_ = pp[C.po_kt], kbs_ = pp[C.po_kbs];
+  const double dtau = kt_ * (1.0 - tau * tau);  // d tau / d p_z
+  const double ddtau = -2.0 * kt_ * tau * dtau;  // d2 tau / d p_z2
+  if (want_jac) {
+    if (lane < 8) {
+      zs[JX_TAU + lane] = tau;
+      zs[JX_DTAU_U + 2 * lane] = dtau * zpt[Z_U];
+      zs[JX_DTAU_U + 2 * lane + 1] = dtau * zpt[Z_U + 1];
+      zs[JX_KF + lane] = kbs_ * zpt[Z_F + 2] + zpt[Z_FD + 2];
+      zs[JX_KP + lane] = kbs_ * zpt[Z_P + 2] + zpt[Z_V + 2];
+    }
+    if (lane < 24) zs[JX_PC + lane] = zs[15 * (lane / 3) + Z_P + lane % 3] - zs[Z_COM + lane % 3];
+    if (lane >= 24 && lane < 27) zs[JX_FSUM + lane - 24] = lane == 24 ? fsum.x : (lane == 25 ? fsum.y : fsum.z);
+    if (lane == 27) zs[JX_ONE] = 1.0;
+    if (lane < JC_COUNT) {  // coefficient table, order of the JC_* codes
+      const double cv = lane == JC_ONE ? 1.0 : lane == JC_MONE ? -1.0 : lane == JC_HDT ? hdt : lane == JC_MHDT ? -hdt
+                      : lane == JC_MASS ? mass : lane == JC_QUARTER ? 0.25 : lane == JC_MQUARTER ? -0.25
+                      : lane == JC_PERIODIC ? (k == 0 ? 1.0 : -1.0) : lane == JC_MTWO ? -2.0 : 2.0 * mu * mu;
+      zs[JX_COEF + lane] = cv;
+    }
+  }
+  if (want_hess && lane < 8) {
+    park[8 * PK_DTAU + lane] = dtau;
+    park[8 * PK_DDTAU + lane] = ddtau;
+  }
+
   HB_PHASE(1, 1);  // g rows, per-point terms
   // ------------------------------------------------------------------ least-squares cost rows (k >= 1)
+  // 31 linear residuals r = c^T z - ref, each with cost w r^2:
+  //   row 0..2    contacts centroid, component c: coefficient -1/8 on the eight p_c
+  //   row 3..6    foot yaw, 3 + 2 foot + side: (sin, -cos) on (p_x, p_y) of point pa, (-sin, cos) on point pb,
+  //               where (pa, pb) = yaw points (yaw[side], yaw[side + 1]) of the foot
+  //   row 7..30   force ratio, 7 + 12 foot + 3 i + c: delta_ij - alpha_i on the four f_c of the foot
+  // Lane `row` evaluates one residual.  The gradient 2 w r c and the Hessian 2 sigma w c c^T are summed in closed
+  // form: lane v < 24 owns the variables p_c and f_c of point v / 3, c = v % 3, and the Hessian entries of lane l
+  // are C.hc_ls[8 l .. 8 l + 6] (hb_kino_create builds them in the order of the slots below).  Every gradient
+  // element and every entry is written by one lane, once: no row tables, no rounds, a fixed summation order.
   if (k1 && (want_f || want_grad || want_hess || want_terms)) {
-    if (lane < LS_ROWS) {
-      int n = 0;
-      int* var = ls_var + lane * LS_MAXV;
-      double* cf = ls_coef + lane * LS_MAXV;
-      double w = 0.0, r = 0.0;
-      if (lane < 3) {  // contacts centroid cost, component `lane`
-        n = 8;
-        double acc = 0.0;
-        for (int i = 0; i < 8; ++i) {
-          var[i] = 15 * i + Z_P + lane;
-          cf[i] = -0.125;
-          acc += zs[15 * i + Z_P + lane];
-        }
-        r = ref[R_CC + lane] - 0.125 * acc;
-        w = C.w_centroid * ref[R_CW + lane];
-      } else if (lane < 7) {  // foot yaw task
-        const int foot = (lane - 3) >> 1, side = (lane - 3) & 1;
-        const double yaw = ref[foot == 0 ? R_YAW_L : R_YAW_R] + (side ? 1.5707963267948966 : 0.0);
-        double sn, cs;
-        sincos(yaw, &sn, &cs);
-        const int pa = 15 * (4 * foot + C.yaw[side ? 1 : 0]) + Z_P, pb2 = 15 * (4 * foot + C.yaw[side ? 2 : 1]) + Z_P;
-        n = 4;
-        var[0] = pa;
-        var[1] = pa + 1;
-        var[2] = pb2;
-        var[3] = pb2 + 1;
-        cf[0] = sn;
-        cf[1] = -cs;
-        cf[2] = -sn;
-        cf[3] = cs;
-        r = -sn * (zs[pb2] - zs[pa]) + cs * (zs[pb2 + 1] - zs[pa + 1]);
-        w = 0.5 * C.w_yaw;
-      } else {  // force ratio
-        const int t = lane - 7;
-        const int foot = t / 12, i = (t % 12) / 3, c = t % 3;
-        const double alpha = ref[(foot == 0 ? R_RATIO_L : R_RATIO_R) + i];
-        n = 4;
-        double ssum = 0.0;
-        for (int j = 0; j < 4; ++j) {
-          var[j] = 15 * (4 * foot + j) + Z_F + c;
-          cf[j] = (j == i ? 1.0 : 0.0) - alpha;
-          ssum += zs[var[j]];
-        }
-        r = zs[var[i]] - alpha * ssum;
-        w = C.w_ratio;
-      }
-      ls_n[lane] = n;
-      ls_w[lane] = w;
-      ls_r[lane] = r;
-      cost += w * r * r;
+    double w = 0.0, r = 0.0, sn = 0.0, cs = 0.0;
+    if (lane < 3) {
+      double acc = 0.0;
+      for (int i = 0; i < 8; ++i) acc += zs[15 * i + Z_P + lane];
+      r = ref[R_CC + lane] - 0.125 * acc;
+      w = C.w_centroid * ref[R_CW + lane];
+    } else if (lane < 7) {
+      const int foot = (lane - 3) >> 1, side = (lane - 3) & 1;
+      const double yaw = ref[foot == 0 ? R_YAW_L : R_YAW_R] + (side ? 1.5707963267948966 : 0.0);
+      sincos(yaw, &sn, &cs);
+      const int pa = 15 * (4 * foot + C.yaw[side]) + Z_P, pb = 15 * (4 * foot + C.yaw[side + 1]) + Z_P;
+      r = -sn * (zs[pb] - zs[pa]) + cs * (zs[pb + 1] - zs[pa + 1]);
+      w = 0.5 * C.w_yaw;
+    } else if (lane < LS_ROWS) {
+      const int t = lane - 7;
+      const int foot = t / 12, i = (t % 12) / 3, c = t % 3;
+      const double alpha = ref[(foot == 0 ? R_RATIO_L : R_RATIO_R) + i];
+      const double* zf = zs + 60 * foot + Z_F + c;
+      r = zf[15 * i] - alpha * (((zf[0] + zf[15]) + zf[30]) + zf[45]);
+      w = C.w_ratio;
     }
-    __syncwarp();
-    if (want_terms && lane < 11) {  // 1 centroid + 2 yaw + 8 force-ratio expressions
-      // rows of one named expression: centroid 0..2; yaw 3,4 (left) 5,6 (right); force ratio of point
-      // (foot, i): 7 + 12 foot + 3 i + c
-      int r0, n;
-      if (lane == 0) r0 = 0, n = 3;
-      else if (lane < 3) r0 = 3 + 2 * (lane - 1), n = 2;
-      else r0 = 7 + 3 * (lane - 3), n = 3;
+    const double cr = w * r * r;
+    cost += cr;
+    if (want_terms) {  // lane 0: centroid (rows 0..2); 1, 2: yaw left / right; 3 + 4 foot + i: force ratio of (foot, i)
+      const int r0 = lane == 0 ? 0 : (lane < 3 ? 3 + 2 * (lane - 1) : 7 + 3 * (lane - 3));
+      const int n = lane == 0 ? 3 : (lane < 3 ? 2 : 3);
       double t = 0.0;
-      for (int i = 0; i < n; ++i) t += ls_w[r0 + i] * ls_r[r0 + i] * ls_r[r0 + i];
-      ct[lane == 0 ? HB_CT_CENTROID : (lane == 1 ? HB_CT_YAW_LEFT : (lane == 2 ? HB_CT_YAW_RIGHT : HB_CT_FRATIO0 + lane - 3))] = t;
+#pragma unroll
+      for (int i = 0; i < 3; ++i) {
+        const double v = __shfl_sync(0xffffffffu, cr, (r0 + i) & 31);
+        if (i < n) t += v;
+      }
+      if (lane < 11)
+        ct(lane == 0 ? HB_CT_CENTROID : (lane == 1 ? HB_CT_YAW_LEFT : (lane == 2 ? HB_CT_YAW_RIGHT : HB_CT_FRATIO0 + lane - 3))) = t;
     }
-    // Rows are grouped in phases whose rows touch disjoint variables, so a phase is one parallel
-    // read-modify-write and the order of the additions into every entry is fixed (deterministic):
-    //   A   centroid rows 0..2 (one per component)            8 variables each
-    //   B/C yaw rows of side 0 / side 1 (one per foot)        4 variables each
-    //   D_i force-ratio rows of point i (one per foot, comp.) 4 variables each, i = 0..3
-    // (ncu, previous version: the 31 rows processed one after the other, each waiting for its own
-    // hc_index load, were 20 % of this kernel's stall samples.)
-    auto ls_row = [](int phase, int grp) {  // phase 0: A, 1: B, 2: C, 3 + i: D_i
-      if (phase == 0) return grp;
-      if (phase < 3) return 3 + 2 * grp + (phase - 1);
-      return 7 + (grp / 3) * 12 + (phase - 3) * 3 + grp % 3;
+    // sine and cosine of the two yaw rows of `foot`; sign of point pt in yaw row (foot, side): +1 on pa, -1 on pb, else 0
+    double ysn[4], ycs[4];
+#pragma unroll
+    for (int y = 0; y < 4; ++y) {
+      ysn[y] = __shfl_sync(0xffffffffu, sn, 3 + y);
+      ycs[y] = __shfl_sync(0xffffffffu, cs, 3 + y);
+    }
+    auto ysgn = [&](int pt, int side) {
+      const int q = pt & 3;
+      return q == C.yaw[side] ? 1.0 : (q == C.yaw[side + 1] ? -1.0 : 0.0);
     };
+    const double wy = 0.5 * C.w_yaw;
     if (want_grad) {
-#pragma unroll 1
-      for (int phase = 0; phase < 7; ++phase) {
-        const int nv = phase == 0 ? 8 : 4;
-        const int ngrp = phase == 0 ? 3 : (phase < 3 ? 2 : 6);
-        const int grp = lane / nv, j = lane % nv;
-        if (grp < ngrp) {
-          const int row = ls_row(phase, grp);
-          gbuf[ls_var[row * LS_MAXV + j]] += 2.0 * ls_w[row] * ls_r[row] * ls_coef[row * LS_MAXV + j];
+      const int pt = lane / 3, c = lane % 3, foot = (pt >> 2) & 1;
+      const double rc = __shfl_sync(0xffffffffu, r, c), wc = __shfl_sync(0xffffffffu, w, c);
+      double ry[2], rf[4];
+#pragma unroll
+      for (int s = 0; s < 2; ++s) ry[s] = __shfl_sync(0xffffffffu, r, 3 + 2 * foot + s);
+#pragma unroll
+      for (int i = 0; i < 4; ++i) rf[i] = __shfl_sync(0xffffffffu, r, (7 + 12 * foot + 3 * i + c) & 31);
+      if (lane < 24) {
+        double gp = 2.0 * wc * rc * -0.125;
+        if (c < 2) {
+#pragma unroll
+          for (int s = 0; s < 2; ++s) {
+            const double kk = c == 0 ? (foot ? ysn[2 + s] : ysn[s]) : -(foot ? ycs[2 + s] : ycs[s]);
+            gp += 2.0 * wy * ry[s] * (ysgn(pt, s) * kk);
+          }
         }
-        __syncwarp();
+        gbuf[15 * pt + Z_P + c] += gp;
+        const double* al = ref + (foot ? R_RATIO_R : R_RATIO_L);
+        double gf = 0.0;
+#pragma unroll
+        for (int i = 0; i < 4; ++i) gf += 2.0 * C.w_ratio * rf[i] * ((i == (pt & 3) ? 1.0 : 0.0) - al[i]);
+        gbuf[15 * pt + Z_F + c] += gf;
       }
     }
     if (want_hess) {
-      // pair (a, c), a <= c, number q of an n-variable row, row-major upper triangle
-      auto pair_of = [](int q, int n, int& a, int& c) {
-        a = 0;
-        while (q >= n - a) {
-          q -= n - a;
-          ++a;
-        }
-        c = a + q;
-      };
-      // every lane prepares its (at most 8) items, loads their local entries together, then adds by phase
-      int it_idx[8];
-      double it_val[8];
+      const int4 q4 = *reinterpret_cast<const int4*>(C.hc_ls + 8 * lane);
+      const int wv[4] = {q4.x, q4.y, q4.z, q4.w};
+      const double tw = 2.0 * sg;
+      double hv[7];
+      // slots 0..3: p_c of points (i, j), component c = t / 36, pair q = t % 36 = 8 d + a -> {a, (a + d) mod 8}:
+      // centroid row c, then (c = x, y, both points on one foot) the yaw rows of that foot
 #pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        it_idx[u] = -1;
-        it_val[u] = 0.0;
-        int row = -1, q = 0, n = 4;
-        if (u < 4) {  // A: 3 rows x 36 pairs
-          const int t = lane + 32 * u;
-          if (t < 108) {
-            row = t / 36;
-            q = t % 36;
-            n = 8;
-          }
-        } else if (u < 6) {  // B (u = 4), C (u = 5): 2 rows x 10 pairs
-          if (lane < 20) {
-            row = ls_row(u - 3, lane / 10);
-            q = lane % 10;
-          }
-        } else {  // D: 6 (foot, component) groups x 10 pairs, the 4 rows of a group summed here
-          const int t = lane + 32 * (u - 6);
-          if (t < 60) {
-            row = ls_row(3, t / 10);
-            q = t % 10;
+      for (int u = 0; u < 4; ++u) {
+        const int t = lane + 32 * u, c = t / 36, q = t % 36;
+        const int a = q & 7, a2 = (a + (q >> 3)) & 7, i = min(a, a2), j = max(a, a2), foot = i >> 2;
+        double v = tw * __shfl_sync(0xffffffffu, w, c & 3) * -0.125 * -0.125;
+        if (c < 2 && foot == (j >> 2)) {
+#pragma unroll
+          for (int s = 0; s < 2; ++s) {
+            const double kk = c == 0 ? (foot ? ysn[2 + s] : ysn[s]) : -(foot ? ycs[2 + s] : ycs[s]);
+            v += tw * wy * (ysgn(i, s) * kk) * (ysgn(j, s) * kk);
           }
         }
-        if (row >= 0) {
-          int a, c;
-          pair_of(q, n, a, c);
-          const int* var = ls_var + row * LS_MAXV;
-          it_idx[u] = var[a] * NCV + var[c];
-          double v = 0.0;
-          const int reps = u < 6 ? 1 : 4;
-          for (int i = 0; i < reps; ++i) {  // D: rows of points i = 0..3 are 3 rows apart
-            const double* cf = ls_coef + (row + 3 * i) * LS_MAXV;
-            v += 2.0 * sg * ls_w[row + 3 * i] * cf[a] * cf[c];
-          }
-          it_val[u] = v;
-        }
+        hv[u] = v;
       }
-      int it_e[8];
+      {  // slot 4: (p_x of point 4 foot + i, p_y of point 4 foot + j), yaw rows only; lane = 16 foot + 4 i + j
+        const int foot = lane >> 4, i = (lane >> 2) & 3, j = lane & 3;
+        double v = 0.0;
 #pragma unroll
-      for (int u = 0; u < 8; ++u) it_e[u] = it_idx[u] >= 0 ? (int)C.hc_index[it_idx[u]] : -1;
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        if (it_e[u] >= 0) hbuf[it_e[u]] += it_val[u];
-        if (u >= 3 && u < 6) __syncwarp();  // phase boundaries: A | B | C | D
+        for (int s = 0; s < 2; ++s) {
+          const double ks = foot ? ysn[2 + s] : ysn[s], kc = -(foot ? ycs[2 + s] : ycs[s]);
+          v += tw * wy * (ysgn(i, s) * ks) * (ysgn(j, s) * kc);
+        }
+        hv[4] = v;
       }
-      __syncwarp();
+      // slots 5, 6: f_c of points (i, j) of one foot, t = 10 (3 foot + c) + q, q = 4 d + a -> {a, (a + d) mod 4}:
+      // the four force-ratio rows of (foot, c)
+#pragma unroll
+      for (int u = 5; u < 7; ++u) {
+        const int t = lane + 32 * (u - 5), foot = (t / 30) & 1, q = t % 10;
+        const int a = q & 3, a2 = (a + (q >> 2)) & 3, i = min(a, a2), j = max(a, a2);
+        const double* al = ref + (foot ? R_RATIO_R : R_RATIO_L);
+        double v = 0.0;
+#pragma unroll
+        for (int m = 0; m < 4; ++m) v += tw * C.w_ratio * ((m == i ? 1.0 : 0.0) - al[m]) * ((m == j ? 1.0 : 0.0) - al[m]);
+        hv[u] = v;
+      }
+      // the entries of the warp are distinct: old values are read together, then written
+      int te[7];
+      double old[7];
+#pragma unroll
+      for (int u = 0; u < 7; ++u) te[u] = (int)(short)((u & 1) ? (wv[u >> 1] >> 16) : (wv[u >> 1] & 0xffff));
+#pragma unroll
+      for (int u = 0; u < 7; ++u) old[u] = te[u] >= 0 ? hbuf[te[u]] : 0.0;
+#pragma unroll
+      for (int u = 0; u < 7; ++u)
+        if (te[u] >= 0) hbuf[te[u]] = old[u] + hv[u];
     }
   }
 
@@ -772,28 +814,12 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
 
   HB_PHASE(1, 3);  // f, grad_f
   // ------------------------------------------------------------------ Jacobian values
-  // Every entry is coefficient x source (contact_jac_desc.h).  The derived sources and the coefficient table go
-  // where the previous knot's variables were (zp is dead after the defect rows), then the knot class's
-  // destination-sorted list is streamed: {slot, descriptor} pairs, coalesced stores, no per-entry branching.
+  // Every entry is coefficient x source (contact_jac_desc.h): the knot class's destination-sorted list is
+  // streamed, {slot, descriptor} pairs, coalesced stores, no per-entry branching.
   if (want_jac) {
     __syncwarp();
-    if (lane < 8) {
-      zs[JX_TAU + lane] = tau;
-      zs[JX_DTAU_U + 2 * lane] = dtau * pu.x;
-      zs[JX_DTAU_U + 2 * lane + 1] = dtau * pu.y;
-      zs[JX_KF + lane] = kbs * pf.z + pfd.z;
-      zs[JX_KP + lane] = kbs * ppos.z + pv.z;
-    }
-    if (lane < 24) zs[JX_PC + lane] = zs[15 * (lane / 3) + Z_P + lane % 3] - zs[Z_COM + lane % 3];
-    if (lane >= 24 && lane < 27) zs[JX_FSUM + lane - 24] = lane == 24 ? fsum.x : (lane == 25 ? fsum.y : fsum.z);
-    if (lane == 27) zs[JX_ONE] = 1.0;
-    if (lane < JC_COUNT) {  // coefficient table, order of the JC_* codes
-      const double cv = lane == JC_ONE ? 1.0 : lane == JC_MONE ? -1.0 : lane == JC_HDT ? hdt : lane == JC_MHDT ? -hdt
-                      : lane == JC_MASS ? mass : lane == JC_QUARTER ? 0.25 : lane == JC_MQUARTER ? -0.25
-                      : lane == JC_PERIODIC ? (k == 0 ? 1.0 : -1.0) : lane == JC_MTWO ? -2.0 : 2.0 * mu * mu;
-      zs[JX_COEF + lane] = cv;
-    }
-    __syncwarp();
+    const int4 kmaps = knot_maps();
+    double* jb = jac + b * C.nnz_j + kmaps.x;
     const int2* lst = C.jc_list + kmaps.y;
     const int n = kmaps.z;
     for (int eb = lane; eb < n; eb += 256) {
@@ -811,58 +837,41 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
   if (want_hess) {
     if (lane < 8) {
       const int o = 15 * lane;
-      // The contributions of this point are listed first, their local entries loaded together, and only
-      // then accumulated: a hadd() per term serialises "index load -> shared read-modify-write" (the
-      // compiler cannot move the next index load above the previous shared store).
-      constexpr int NT = (TERRAIN == 0 ? 11 : 0) + 6 + 12;
-      int ti[NT];
-      double tv[NT];
-      int n = 0;
-      auto term = [&](int vi, int vj, double v) {
-        ti[n] = vi * NCV + vj;
-        tv[n] = v;
-        ++n;
-      };
+      const double* pk = park + lane;
       const double kk1 = k1 ? 1.0 : 0.0;  // cost terms and the friction row exist from knot 1 on
+      // centroidal momentum dynamics: -(dt/2) (lam_k + lam_{k+1})_ang . ((p - x) x f), pair m = 0..5 of (a, b), a != b
+      auto mom = [&](int m) {
+        const int a = m / 2, bb = a == 0 ? 1 + m % 2 : (a == 1 ? 2 * (m % 2) : m % 2);
+        return -hdt * eps3(a, bb) * pk[8 * (PK_LA + 3 - a - bb)];
+      };
       if constexpr (TERRAIN == 0) {
-        const double l0 = lam_pl[0], l1 = lam_pl[1], ld = lam_dcc, lf = kk1 * lam_fr;
-        term(o + Z_P + 2, o + Z_P + 2, -(l0 * pu.x + l1 * pu.y) * ddtau + kk1 * sg * C.w_swing);
-        term(o + Z_P + 2, o + Z_U, -l0 * dtau);
-        term(o + Z_P + 2, o + Z_U + 1, -l1 * dtau);
-        term(o + Z_P + 2, o + Z_F + 2, -ld * kbs);
-        term(o + Z_V + 2, o + Z_F + 2, -ld);
-        term(o + Z_FD + 2, o + Z_P + 2, -ld);
-        term(o + Z_V, o + Z_V, kk1 * sg * C.w_swing);
-        term(o + Z_V + 1, o + Z_V + 1, kk1 * sg * C.w_swing);
-        term(o + Z_F, o + Z_F, -2.0 * lf);
-        term(o + Z_F + 1, o + Z_F + 1, -2.0 * lf);
-        term(o + Z_F + 2, o + Z_F + 2, 2.0 * mu * mu * lf);
-      }
-#pragma unroll
-      for (int c = 0; c < 3; ++c) {
-        term(o + Z_U + c, o + Z_U + c, kk1 * 2.0 * sg * C.w_u);
-        term(o + Z_FD + c, o + Z_FD + c, kk1 * 2.0 * sg * C.w_fd);
-      }
-      // centroidal momentum dynamics: -(dt/2) (lam_k + lam_{k+1})_ang . ((p - x) x f)
-#pragma unroll
-      for (int a = 0; a < 3; ++a)
-#pragma unroll
-        for (int bb = 0; bb < 3; ++bb) {
-          if (a == bb) continue;
-          const int c = 3 - a - bb;
-          const double v = -hdt * eps3(a, bb) * La[c];
-          term(o + Z_P + a, o + Z_F + bb, v);
-          term(CV_COM + a, o + Z_F + bb, -v);
-        }
-      if constexpr (TERRAIN == 0) {
-        // the local entries of this point's 29 terms come from a per-point table (64 bytes per lane, four 16-byte loads
-        // that every warp shares in L1) instead of 29 lookups in the 33 KB (variable, variable) table; the entries of one
-        // lane are distinct and no other lane touches them, so old values are read, updated and written in batches
+        // The 29 terms of this point, in the order of their local entries in the per-point table C.hc_pt (64 bytes
+        // per lane, four 16-byte loads that every warp shares in L1): 11 complementarity / friction / swing terms,
+        // 6 control regularisations, 12 momentum cross terms.  The entries of one lane are distinct and no other
+        // lane touches them, so old values are read, updated and written in batches of 10, each batch computing its
+        // own values (the 29 values are never live at once).
         const int4* tq = reinterpret_cast<const int4*>(C.hc_pt + 32 * lane);
         const int4 q4[4] = {tq[0], tq[1], tq[2], tq[3]};
         const int wv[16] = {q4[0].x, q4[0].y, q4[0].z, q4[0].w, q4[1].x, q4[1].y, q4[1].z, q4[1].w,
                             q4[2].x, q4[2].y, q4[2].z, q4[2].w, q4[3].x, q4[3].y, q4[3].z, q4[3].w};
-        (void)ti;
+        constexpr int NT = 29;
+        auto tval = [&](int t) -> double {
+          const double ld = pk[8 * PK_LD], lf = kk1 * pk[8 * PK_LF];
+          switch (t) {
+            case 0: return -(pk[8 * PK_L0] * zs[o + Z_U] + pk[8 * PK_L1] * zs[o + Z_U + 1]) * pk[8 * PK_DDTAU] + kk1 * sg * C.w_swing;  // (p_z, p_z)
+            case 1: return -pk[8 * PK_L0] * pk[8 * PK_DTAU];                                         // (p_z, u_x)
+            case 2: return -pk[8 * PK_L1] * pk[8 * PK_DTAU];                                         // (p_z, u_y)
+            case 3: return -ld * pp[C.po_kbs];                                                              // (p_z, f_z)
+            case 4: return -ld;                                                                      // (v_z, f_z)
+            case 5: return -ld;                                                                      // (fdot_z, p_z)
+            case 6: case 7: return kk1 * sg * C.w_swing;                                             // (v_x, v_x), (v_y, v_y)
+            case 8: case 9: return -2.0 * lf;                                                        // (f_x, f_x), (f_y, f_y)
+            case 10: return 2.0 * mu * mu * lf;                                                      // (f_z, f_z)
+            default: break;
+          }
+          if (t < 17) return (t & 1) ? kk1 * 2.0 * sg * C.w_u : kk1 * 2.0 * sg * C.w_fd;          // (u_c, u_c), (fdot_c, fdot_c)
+          return ((t - 17) & 1) ? -mom((t - 17) >> 1) : mom((t - 17) >> 1);                       // (p_a, f_b), (com_a, f_b)
+        };
 #pragma unroll
         for (int c0 = 0; c0 < NT; c0 += 10) {
           int te[10];
@@ -876,9 +885,33 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
           for (int u = 0; u < 10; ++u) old[u] = te[u] >= 0 ? hbuf[te[u]] : 0.0;
 #pragma unroll
           for (int u = 0; u < 10; ++u)
-            if (te[u] >= 0) hbuf[te[u]] = old[u] + tv[c0 + u < NT ? c0 + u : 0];
+            if (c0 + u < NT && te[u] >= 0) hbuf[te[u]] = old[u] + tval(c0 + u);
         }
       } else {
+        // The contributions of this point are listed first, their local entries loaded together, and only
+        // then accumulated: a hadd() per term serialises "index load -> shared read-modify-write" (the
+        // compiler cannot move the next index load above the previous shared store).
+        constexpr int NT = 6 + 12;
+        int ti[NT];
+        double tv[NT];
+        int n = 0;
+        auto term = [&](int vi, int vj, double v) {
+          ti[n] = vi * NCV + vj;
+          tv[n] = v;
+          ++n;
+        };
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+          term(o + Z_U + c, o + Z_U + c, kk1 * 2.0 * sg * C.w_u);
+          term(o + Z_FD + c, o + Z_FD + c, kk1 * 2.0 * sg * C.w_fd);
+        }
+#pragma unroll
+        for (int m = 0; m < 6; ++m) {
+          const int a = m / 2, bb = a == 0 ? 1 + m % 2 : (a == 1 ? 2 * (m % 2) : m % 2);
+          const double v = mom(m);
+          term(o + Z_P + a, o + Z_F + bb, v);
+          term(CV_COM + a, o + Z_F + bb, -v);
+        }
         int te[NT];
 #pragma unroll
         for (int u = 0; u < NT; ++u) te[u] = C.hc_index[ti[u]];
@@ -890,7 +923,7 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
     HB_PHASE(1, 5);  // Hessian terms
     __syncwarp();
     const int2 hcm_ = *reinterpret_cast<const int2*>(&C.knot_maps[k].hc_off);  // {hc_off, hc_cnt}
-    const int2 hcm = make_int2(kmaps.w, hcm_.x);
+    const int2 hcm = make_int2(C.knot_maps[k].hc_base, hcm_.x);
     const unsigned* hlst = C.hc_list + hcm.y;  // destination-sorted: entry << 16 | slot
     double* hb_ = hess + b * C.nnz_h + hcm.x;
     const int n_l = hcm_.y;

@@ -30,7 +30,7 @@ __global__ void __launch_bounds__(128) pose_contact_kernel(const KinoConst* __re
   const int warp = threadIdx.x >> 5;
   const long b = (long)blockIdx.x * (blockDim.x >> 5) + warp;
   if (b >= batch) return;
-  const ContactSmem L = contact_smem_layout(C.n_hc);
+  const ContactSmem L = pose_contact_smem_layout(C.n_hc);
   double* sm = smem + (size_t)warp * L.total;
   double* zs = sm + L.z;
   double* hbuf = sm + L.hbuf;
