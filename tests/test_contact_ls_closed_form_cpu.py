@@ -6,6 +6,8 @@ rows), so the gradient is 2 w r c and the Hessian 2 sigma w c c^T.  The kernel s
 Hessian entry, each lane owning a fixed set of entries taken from a host-built table (hb_kino_create, next to the
 per-point table hc_pt).  This test builds that table from the layout's hc_index the way the host does, evaluates the
 kernel's slot formulas and compares them with the rows assembled one by one."""
+import itertools
+
 import numpy as np
 import pytest
 
@@ -17,9 +19,21 @@ Z_P, Z_F, NZ, NCV = 6, 9, 189, 129
 R_RATIO_L, R_YAW_L, R_RATIO_R, R_YAW_R, R_CW, R_CC, R_COUNT = 0, 4, 5, 9, 11, 14, 55
 
 
+# every ordered triple of distinct points of one foot as (bottom-right, top-right, top-left): the yaw rows, the
+# kernel's sign table and the host's per-lane table all follow the triple, and the layout is built with it
+YAW_TRIPLES = list(itertools.permutations(range(4), 3))
+_layouts = {}
+
+
+def layout_for(yaw):
+    if yaw not in _layouts:
+        _layouts[yaw] = KinoLayout(synthetic_ergocub(), KinoSettings(horizon=4, yaw_points=yaw))
+    return _layouts[yaw]
+
+
 @pytest.fixture(scope="module")
 def layout():
-    return KinoLayout(synthetic_ergocub(), KinoSettings(horizon=4))
+    return layout_for(KinoSettings().yaw_points)
 
 
 def rows(z, ref, yaw, w_centroid, w_yaw, w_ratio):
@@ -143,6 +157,15 @@ def closed_form(z, ref, yaw, w_centroid, w_yaw, w_ratio, sg, tab, n_hc):
 
 
 def test_table_entries_are_distinct_and_cover_the_rows(layout):
+    check_table(layout)
+
+
+@pytest.mark.parametrize("yaw", YAW_TRIPLES)
+def test_table_entries_for_every_yaw_triple(yaw):
+    check_table(layout_for(yaw))
+
+
+def check_table(layout):
     yaw = layout.st.yaw_points
     tab = host_table(layout.hc_index, yaw)
     used = tab[tab >= 0]
@@ -159,6 +182,16 @@ def test_table_entries_are_distinct_and_cover_the_rows(layout):
 
 @pytest.mark.parametrize("seed", range(6))
 def test_closed_form_matches_rows(layout, seed):
+    check_closed_form(layout, seed)
+
+
+@pytest.mark.parametrize("yaw", YAW_TRIPLES)
+def test_closed_form_matches_rows_for_every_yaw_triple(yaw):
+    for seed in (100, 101):
+        check_closed_form(layout_for(yaw), seed)
+
+
+def check_closed_form(layout, seed):
     rng = np.random.default_rng(seed)
     yaw = layout.st.yaw_points
     n_hc = layout.n_hc
