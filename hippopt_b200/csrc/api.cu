@@ -50,7 +50,7 @@ struct hb_problem_s {
   short* d_hc_pt = nullptr;
   hb::KnotMaps* d_knot_maps = nullptr;
   int2* d_jc_list = nullptr;
-  unsigned *d_jk_list = nullptr, *d_hc_list = nullptr, *d_hk_list = nullptr;
+  unsigned *d_jk_list = nullptr, *d_hc_list = nullptr;
   // per-knot cost partial sums, one scratch buffer per stream so that evaluations enqueued on
   // different streams (HostPipeline) do not share scratch
   std::map<cudaStream_t, std::pair<double*, int64_t>> fpart;
@@ -499,7 +499,7 @@ extern "C" int hb_kino_create(const int32_t* icfg, const double* dcfg, const int
     if (e == cudaSuccess) e = relative(jc_map, C.n_jc, &KM::jc_base, &KM::jc_off, &KM::jc_cnt, &h->d_jc, (void**)&h->d_jc_list, C.kind == 0);
     if (e == cudaSuccess) e = relative(jk_map, C.n_jk, &KM::jk_base, &KM::jk_off, &KM::jk_cnt, &h->d_jk, (void**)&h->d_jk_list, false);
     if (e == cudaSuccess) e = relative(hc_map, C.n_hc, &KM::hc_base, &KM::hc_off, &KM::hc_cnt, &h->d_hc, (void**)&h->d_hc_list, false);
-    if (e == cudaSuccess) e = relative(hk_map, 27 * 57, &KM::hk_base, &KM::hk_off, &KM::hk_cnt, &h->d_hk, (void**)&h->d_hk_list, false);
+    if (e == cudaSuccess) e = relative(hk_map, 27 * 57, &KM::hk_base, &KM::hk_off, nullptr, &h->d_hk, nullptr, false);
     if (e == cudaSuccess) e = relative(hk2_map, 27, &KM::hk2_base, &KM::hk2_off, nullptr, &h->d_hk2, nullptr, false);
     if (e == cudaSuccess) e = upload(&h->d_knot_maps, km.data(), km.size());
     if (too_wide) {
@@ -573,7 +573,6 @@ extern "C" int hb_kino_create(const int32_t* icfg, const double* dcfg, const int
   C.jc_list = h->d_jc_list;
   C.jk_list = h->d_jk_list;
   C.hc_list = h->d_hc_list;
-  C.hk_list = h->d_hk_list;
   h->topo.knot_maps = h->d_knot_maps;
   h->topo.jc_list = h->d_jc_list;
   h->topo.hc_list = h->d_hc_list;
@@ -585,7 +584,7 @@ extern "C" int hb_kino_create(const int32_t* icfg, const double* dcfg, const int
   {
     // 4 warps per CTA; the kinematics kernels keep one branch accumulator per body whose children do not
     // directly follow it in the joint list (n_slots): an interleaved joint order does not fit
-    const size_t kin_smem = (size_t)hb::kin_smem_layout(C.nb, C.n_slots, true).total * sizeof(double) * (KIN_H_THREADS / 32);
+    const size_t kin_smem = (size_t)hb::kin_smem_layout(C.nb, C.n_slots, true).total * sizeof(double) * (hb::KIN_H_THREADS / 32);
     if (kin_smem > 200 * 1024) {
       hb_destroy(h);
       return fail(HB_ERR_UNSUPPORTED,
@@ -593,18 +592,11 @@ extern "C" int hb_kino_create(const int32_t* icfg, const double* dcfg, const int
                       " branch accumulators (" + std::to_string(kin_smem / 1024) +
                       " KB of shared memory per CTA > 200 KB): list the joints of a limb consecutively");
     }
-    static const bool untyped_env = getenv("HB_SWEEP_UNTYPED") != nullptr;  // A/B timing of the typed rounds
-    hb::SweepSchedule sch = hb::build_sweep_schedule(sweep_topo_of(C), !untyped_env);
+    hb::SweepSchedule sch = hb::build_sweep_schedule(sweep_topo_of(C), true);
     if (sch.n_rounds <= 0 || sch.n_rounds > 32) sch = hb::build_sweep_schedule(sweep_topo_of(C), false);
     if (sch.n_rounds <= 0 || sch.n_rounds > 32 || sch.n_slots > 62 || sch.n_slots * 12 > 58 + 32 + C.n_slots * 32 * 12) {
       hb_destroy(h);
       return fail(HB_ERR_UNSUPPORTED, "hb_kino_create: no sweep schedule for this tree within the kernel's limits");
-    }
-    if (getenv("HB_DEBUG_SCHED")) {
-      int n_tasks = 0;
-      for (int t : sch.tasks) n_tasks += (t & hb::KT_VALID) ? 1 : 0;
-      fprintf(stderr, "hb_kino_create: packed sweep: %d tasks (%d heavy) in %d rounds, %d slots, seed mask %#x, heavy mask %#x\n",
-              n_tasks, sch.n_heavy_tasks, sch.n_rounds, sch.n_slots, sch.seed_mask, sch.heavy_mask);
     }
     if (e == cudaSuccess) e = upload(&h->d_sched, sch.tasks.data(), sch.tasks.size());
     h->topo.sched = h->d_sched;
@@ -651,7 +643,6 @@ extern "C" int hb_destroy(hb_handle h) {
   cudaFree(h->d_jc_list);
   cudaFree(h->d_jk_list);
   cudaFree(h->d_hc_list);
-  cudaFree(h->d_hk_list);
   cudaFree(h->d_sched);
   cudaFree(h->dev);
   for (auto& kv : h->fpart) cudaFree(kv.second.first);
@@ -751,12 +742,10 @@ extern "C" int hb_eval(hb_handle h, uint32_t mask, const double* x, const double
   const unsigned grid = (unsigned)((total_warps + warps_per_block - 1) / warps_per_block);
   // The "Hessian" variant of the kinematics kernel also serves Jacobian / gradient requests: its forward-mode
   // Jacobian (closed-form tangents, no sweep: 0.42 ms) beats the row-per-lane adjoint sweep of the lean
-  // variant (0.62 ms), which is left with f and g.  hb_set_option(HB_OPT_JAC_ADJOINT) or HB_JAC_ADJOINT=1
-  // select the adjoint sweep: an independent algorithm for the same numbers (tests, A/B timing).
-  static const bool jac_adjoint_env = getenv("HB_JAC_ADJOINT") != nullptr;
-  const bool jac_adjoint = jac_adjoint_env || h->jac_adjoint;
+  // variant (0.62 ms), which is left with f and g.  hb_set_option(HB_OPT_JAC_ADJOINT) selects the adjoint sweep:
+  // an independent algorithm for the same numbers (tests).
   const bool with_hess = (mask & HB_EVAL_HESS_L) != 0 ||
-                         (!jac_adjoint && (mask & (HB_EVAL_JAC_G | HB_EVAL_GRAD_F)) != 0);
+                         (!h->jac_adjoint && (mask & (HB_EVAL_JAC_G | HB_EVAL_GRAD_F)) != 0);
   auto mark = [&]() -> int {
     if (!h->prof) return HB_OK;
     cudaEvent_t e;
@@ -811,7 +800,7 @@ extern "C" int hb_eval(hb_handle h, uint32_t mask, const double* x, const double
   if (mark() != HB_OK) return HB_ERR_CUDA;
   {
     // the Hessian variant has its own CTA shape (KIN_H_THREADS, kino_kin.cu): occupancy tuning
-    const int kin_warps = with_hess ? KIN_H_THREADS / 32 : warps_per_block;
+    const int kin_warps = with_hess ? hb::KIN_H_THREADS / 32 : warps_per_block;
     const unsigned kin_grid = (unsigned)((total_warps + kin_warps - 1) / kin_warps);
     const size_t smem = (size_t)hb::kin_smem_layout(C.nb, C.n_slots, with_hess).total * sizeof(double) * kin_warps;
     if (with_hess)

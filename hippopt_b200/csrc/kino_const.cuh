@@ -48,13 +48,15 @@ struct BodyC {
 // interior warp then reads the SAME few kilobytes (L1-resident) where the per-knot tables were an L2 round trip
 // in front of every batch of scattered stores.  `*_off`: element offset of the knot's table inside the map array;
 // `*_base`: what to add to its entries.
-// Besides the entry-indexed tables (`*_map`: local entry -> slot) every class has a DESTINATION-SORTED list
-// (`*_list`, `*_cnt` valid words at the same offset): word = local entry << 16 | slot for the staged outputs, and
-// {slot, value descriptor} (contact_jac_desc.h) for the contact kernel's Jacobian.  Walking a list in order makes
-// consecutive lanes store to consecutive addresses wherever the pattern has runs (whole point blocks of columns).
+// Besides the entry-indexed tables (`*_map`: local entry -> slot) the Jacobian classes and the contact Hessian have a
+// DESTINATION-SORTED list (`*_list`, `*_cnt` valid words at the same offset): word = local entry << 16 | slot for the
+// staged outputs, and {slot, value descriptor} (contact_jac_desc.h) for the contact kernel's Jacobian.  Walking a list in
+// order makes consecutive lanes store to consecutive addresses wherever the pattern has runs (whole point blocks of
+// columns).  The kinematics Hessian is scattered in entry order and has no list.
 struct alignas(16) KnotMaps {
   int jc_base, jc_off, jc_cnt, hc_base, hc_off, hc_cnt, pad0, pad1;         // contact kernel (two 16-byte loads)
-  int jk_base, jk_off, jk_cnt, hk_base, hk_off, hk_cnt, hk2_base, hk2_off;  // kinematics kernel
+  // kinematics kernel (16- and 8-byte loads); hk_cnt is an unused slot that keeps hk2_base 8-byte aligned
+  int jk_base, jk_off, jk_cnt, hk_base, hk_off, hk_cnt, hk2_base, hk2_off;
 };
 
 struct KinoConst {
@@ -87,7 +89,6 @@ struct KinoConst {
   const int2* jc_list;
   const unsigned* jk_list;
   const unsigned* hc_list;
-  const unsigned* hk_list;
 };
 
 // Warp-uniform part of KinoConst.  It is passed BY VALUE as a __grid_constant__ kernel parameter:

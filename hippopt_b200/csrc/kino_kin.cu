@@ -21,9 +21,9 @@
 //      (primal_adjoint_pass); then only the TANGENT of those adjoints along every direction, as
 //      (direction, body) tasks packed on the lanes by a host-built schedule (kin_tangent_sweep_packed):
 //      column j of the Lagrangian Hessian restricted to (q, s) x (vb, qd, sd, q, s).
-//   The file also keeps the first algorithm for the Jacobian -- a row-per-lane adjoint sweep in fp64
-//   (kin_backward: 32 rows = 24 FK, 3 CoM, 3 momentum, feet distance, frame-orientation trace) -- as an
-//   option (hb_set_option) and cross-check, and the unpacked tangent sweep (HB_SWEEP_PACKED 0).
+//   The lean kernel (f and g) also holds the first algorithm for the Jacobian -- a row-per-lane adjoint sweep in
+//   fp64 (kin_backward: 32 rows = 24 FK, 3 CoM, 3 momentum, feet distance, frame-orientation trace) -- selected by
+//   hb_set_option(HB_OPT_JAC_ADJOINT): an independent cross-check of the forward-mode Jacobian.
 #include "kino_const.cuh"
 
 namespace hb {
@@ -37,27 +37,7 @@ enum {
   SB_CB = SB_R, SB_CDB = SB_R + 3  // alias the rotation: it is dead once the frames have been staged
 };
 enum { HSTAGE = 27 * 57 };  // per-warp staging of the Hessian columns (and, before that, the Jacobian rows)
-#ifndef HB_KIN_STAGE
-#define HB_KIN_STAGE 1   // Hessian kernel: stage + batched scatter (2.47 -> 2.25 ms on B200)
-#endif
-#ifndef HB_KIN_STAGE_F
-#define HB_KIN_STAGE_F 0  // Jacobian-only kernel: staging costs a CTA per SM (see DESIGN.md)
-#endif
-#ifndef HB_FWD_JAC
-#define HB_FWD_JAC 1      // Hessian kernel: Jacobian columns from forward tangents instead of a second sweep
-#endif
-#if HB_FWD_JAC && !HB_KIN_STAGE
-#error "HB_FWD_JAC stages the Jacobian columns: it needs HB_KIN_STAGE"
-#endif
-#ifndef KIN_SCAT
-#define KIN_SCAT 17  // scatter-map loads in flight per lane in the Hessian kernel's two scatters (8: 5.3 k -> see DESIGN.md)
-#endif
-#ifndef HB_SWEEP_PACKED
-#define HB_SWEEP_PACKED 1  // Hessian kernel: (direction, body) tasks packed on the lanes (kin_tangent_sweep_packed)
-#endif
-#if HB_SWEEP_PACKED && !HB_KIN_STAGE
-#error "HB_SWEEP_PACKED accumulates in the staged Hessian columns: it needs HB_KIN_STAGE"
-#endif
+constexpr int KIN_SCAT = 17;  // scatter-map loads in flight per lane in the Hessian kernel's two scatters (8: 5.3 k -> see DESIGN.md)
 
 struct KinSmem {
   int bodies, arms, fdu, fdal, fdar, G, z, gbuf, lamk, slot, stage, total;
@@ -86,11 +66,12 @@ __host__ __device__ inline KinSmem kin_smem_layout(int nb, int n_slots, bool wit
   s.slot = o;
   o += n_slots * 32 * 12;  // fp64 sweep: adjoints; Hessian sweep: their tangents (primal totals are per body)
   s.stage = o;
-  // Values are staged per warp and scattered after the sweep with 8 map loads in flight per lane.
+  // The Hessian kernel stages its values per warp and scatters them after the sweep with batched map loads.
   // Measured on B200 (config 3): direct stores from the sweep 2.47 ms (17 % of the stall samples sat on
   // the store waiting for its own map load); staging with a naive scatter loop 2.54 ms; staging with
-  // the batched scatter 2.25 ms.
-  o += with_hess ? (HB_KIN_STAGE ? HSTAGE : 0) : (HB_KIN_STAGE_F ? 928 : 0);
+  // the batched scatter 2.25 ms.  The lean kernel stores straight through the map: a stage would cost it
+  // a CTA per SM.
+  o += with_hess ? HSTAGE : 0;
   s.total = o;
   return s;
 }
@@ -106,7 +87,7 @@ struct St {
   V3<T> o, d, w, v, ax;
 };
 
-__device__ __forceinline__ St<double> load_state(const double* sb, int l, const Dir&, double) {
+__device__ __forceinline__ St<double> load_state(const double* sb, int l) {
   const double* b = sb + l * SB_STRIDE;
   St<double> s;
   s.o = ld3(b + SB_O);
@@ -135,48 +116,17 @@ __device__ __forceinline__ St<Dual> load_state(const double* sb, int l, const Di
   return s;
 }
 
-// world inertia of body l applied to x
-__device__ __forceinline__ D3 iapply(const double* sb, int l, const Dir&, D3 x) {
-  return symmul(sb + l * SB_STRIDE + SB_I, x);
-}
-__device__ __forceinline__ V3<Dual> iapply(const double* sb, int l, const Dir& dir, V3<Dual> x) {
-  const double* I = sb + l * SB_STRIDE + SB_I;
-  const D3 xv = v3<double>(x.x.v, x.y.v, x.z.v), xd = v3<double>(x.x.d, x.y.d, x.z.d);
-  const double in = ((dir.mask >> l) & 1u) ? 1.0 : 0.0;
-  const D3 a = scale(in, dir.alpha);
-  const D3 Ix = symmul(I, xv);
-  // d(I^w) x = [a]x I x - I [a]x x
-  const D3 t = symmul(I, xd) + cross(a, Ix) - symmul(I, cross(a, xv));
-  return lift<Dual>(Ix, t);
-}
-
-// I^w w_l and I^w hbar with the primal products staged in shared memory (SB_L, SB_IH)
-__device__ __forceinline__ D3 iw_omega(const double* sb, int l, const Dir&, const St<double>&) {
+// I^w w_l with the primal product staged in shared memory (SB_L), and I^w hbar
+__device__ __forceinline__ D3 iw_omega(const double* sb, int l) {
   return ld3(sb + l * SB_STRIDE + SB_L);
 }
-__device__ __forceinline__ V3<Dual> iw_omega(const double* sb, int l, const Dir& dir, const St<Dual>& s) {
-  const double* I = sb + l * SB_STRIDE + SB_I;
-  const D3 Lw = ld3(sb + l * SB_STRIDE + SB_L);
-  const D3 wv = v3<double>(s.w.x.v, s.w.y.v, s.w.z.v), wd = v3<double>(s.w.x.d, s.w.y.d, s.w.z.d);
-  const double in = ((dir.mask >> l) & 1u) ? 1.0 : 0.0;
-  const D3 a = scale(in, dir.alpha);
-  return lift<Dual>(Lw, symmul(I, wd - cross(a, wv)) + cross(a, Lw));
-}
-__device__ __forceinline__ D3 iw_hbar(const double* sb, int l, const Dir&, D3 hb, double) {
+__device__ __forceinline__ D3 iw_hbar(const double* sb, int l, D3 hb) {
   return symmul(sb + l * SB_STRIDE + SB_I, hb);  // seeds differ per lane in the fp64 sweep
 }
 // rho_l = o_l - o_parent and the parent's angular velocity, without rebuilding the parent state
-__device__ __forceinline__ void parent_link(const double* sb, int l, int p, const Dir&, D3& rho, D3& wp) {
+__device__ __forceinline__ void parent_link(const double* sb, int l, int p, D3& rho, D3& wp) {
   rho = ld3(sb + l * SB_STRIDE + SB_RHO);
   wp = ld3(sb + p * SB_STRIDE + SB_W);
-}
-__device__ __forceinline__ void parent_link(const double* sb, int l, int p, const Dir& dir, V3<Dual>& rho,
-                                            V3<Dual>& wp) {
-  const D3 r = ld3(sb + l * SB_STRIDE + SB_RHO), w = ld3(sb + p * SB_STRIDE + SB_W);
-  const double in = ((dir.mask >> p) & 1u) ? 1.0 : 0.0;
-  const D3 a = scale(in, dir.alpha);
-  rho = lift<Dual>(r, cross(a, r));
-  wp = lift<Dual>(w, cross(a, w - dir.wpi) + scale(in, dir.u));
 }
 // branch accumulators in shared memory, component-major and lane-minor
 __device__ __forceinline__ void slot_get(D3& v, const double* sl, int c) {
@@ -184,30 +134,10 @@ __device__ __forceinline__ void slot_get(D3& v, const double* sl, int c) {
   v.y += sl[(c + 1) * 32];
   v.z += sl[(c + 2) * 32];
 }
-__device__ __forceinline__ void slot_get(V3<Dual>& v, const double* sl, int c) {
-  v.x = v.x + mkdual(sl[(2 * c) * 32], sl[(2 * c + 1) * 32]);
-  v.y = v.y + mkdual(sl[(2 * c + 2) * 32], sl[(2 * c + 3) * 32]);
-  v.z = v.z + mkdual(sl[(2 * c + 4) * 32], sl[(2 * c + 5) * 32]);
-}
 __device__ __forceinline__ void slot_add(double* sl, int c, D3 v) {
   sl[(c)*32] += v.x;
   sl[(c + 1) * 32] += v.y;
   sl[(c + 2) * 32] += v.z;
-}
-__device__ __forceinline__ void slot_add(double* sl, int c, V3<Dual> v) {
-  sl[(2 * c) * 32] += v.x.v;
-  sl[(2 * c + 1) * 32] += v.x.d;
-  sl[(2 * c + 2) * 32] += v.y.v;
-  sl[(2 * c + 3) * 32] += v.y.d;
-  sl[(2 * c + 4) * 32] += v.z.v;
-  sl[(2 * c + 5) * 32] += v.z.d;
-}
-__device__ __forceinline__ V3<Dual> iw_hbar(const double* sb, int l, const Dir& dir, D3 hb, Dual) {
-  const double* I = sb + l * SB_STRIDE + SB_I;
-  const D3 Ih = ld3(sb + l * SB_STRIDE + SB_IH);
-  const double in = ((dir.mask >> l) & 1u) ? 1.0 : 0.0;
-  const D3 a = scale(in, dir.alpha);
-  return lift<Dual>(Ih, cross(a, Ih) - symmul(I, cross(a, hb)));
 }
 
 template <class T>
@@ -231,25 +161,71 @@ __device__ __forceinline__ V3<typename Prom<A, B>::type> omega_map(const A* a, c
                2.0 * (a[3] * b[2] - b[3] * a[2] - c.z));
 }
 
+struct JacEmit {
+  const int* map;  // jk_map row of this knot
+  double* jac;     // instance base
+  double* gbuf;    // shared: grad_f accumulation for the kinematic variables
+  int lane;
+  double gscale;   // chest lane: 2 w_frame (phi - 3)
+  bool write;
+  // local bases inside JK (kino_layout.py::_enumerate_jk)
+  __device__ __forceinline__ int base_q() const {
+    if (lane < 24) return 4 + lane * 27;
+    if (lane < 27) return 4 + 648 + (lane - 24) * 27;
+    if (lane < 30) return 4 + 648 + 81 + (lane - 27) * 57 + 7;  // after vb(3), qd(4)
+    return -1;
+  }
+  __device__ __forceinline__ void put(int e, double v) const {
+    const int slot = map[e];
+    if (slot >= 0) jac[slot] = v;
+  }
+  // Scatter slots of the two entries the sweep emits at body l, loaded one step ahead (prefetch(l) is
+  // called at the top of the iteration) so that the stores do not wait for their own map loads.
+  int sbase, sdbase, pre_s, pre_sd;
+  __device__ __forceinline__ void init_bases() {
+    sdbase = -1;
+    if (lane < 27) sbase = base_q() + 4;
+    else if (lane < 30) {
+      const int b = 4 + 648 + 81 + (lane - 27) * 57;
+      sdbase = b + 11;
+      sbase = b + 34;
+    } else sbase = lane == 30 ? 4 + 648 + 81 + 171 : -1;
+    pre_s = pre_sd = -1;
+  }
+  __device__ __forceinline__ void prefetch(int l) {
+    if (!write || l < 1) return;
+    pre_s = sbase >= 0 ? map[sbase + l - 1] : -1;
+    pre_sd = sdbase >= 0 ? map[sdbase + l - 1] : -1;
+  }
+  __device__ __forceinline__ void joint(int l, double sbar, double sdbar) const {
+    const int j = l - 1;
+    if (lane == 31) {
+      gbuf[34 + j] += gscale * sbar;  // gbuf order: vb3 qd4 q4 sd23 s23 -> s at 34
+      return;
+    }
+    if (!write) return;
+    if (pre_s >= 0) jac[pre_s] = sbar;
+    if (pre_sd >= 0) jac[pre_sd] = sdbar;
+  }
+};
+
 // One adjoint sweep over the tree.  `emit.joint(l, sbar, sdbar)` receives d Phi / d s_{l-1} and
 // d Phi / d s_dot_{l-1}; the totals at the root are returned for the base chain rule.
-template <class T, class Emit>
-__device__ __forceinline__ void kin_backward(const KinTopo& C, const double* sb, const double* zs, const Dir& dir,
-                                             const Seeds<T>& S, const V3<T>& xc, const V3<T>& xd, double* slot,
-                                             Emit& emit, V3<T>& n0, V3<T>& w0, V3<T>& v0) {
+__device__ __forceinline__ void kin_backward(const KinTopo& C, const double* sb, const double* zs,
+                                             const Seeds<double>& S, const D3& xc, const D3& xd, double* slot,
+                                             JacEmit& emit, D3& n0, D3& w0, D3& v0) {
   const int nb = C.nb;
   const int lane = threadIdx.x & 31;
-  constexpr int SW = sizeof(T) / sizeof(double);  // doubles per T
-  for (int i = 0; i < C.n_slots * 12 * SW; ++i) slot[i * 32 + lane] = 0.0;
-  V3<T> cn = vzero<T>(), cF = vzero<T>(), cw = vzero<T>(), cv = vzero<T>();
-  V3<T> An = vzero<T>(), AF = vzero<T>(), Aw = vzero<T>(), Av = vzero<T>();
+  for (int i = 0; i < C.n_slots * 12; ++i) slot[i * 32 + lane] = 0.0;
+  D3 cn = vzero<double>(), cF = vzero<double>(), cw = vzero<double>(), cv = vzero<double>();
+  D3 An = vzero<double>(), AF = vzero<double>(), Aw = vzero<double>(), Av = vzero<double>();
   for (int l = nb - 1; l >= 0; --l) {
     emit.prefetch(l);
     if (!C.carry[l]) {
-      cn = vzero<T>();
-      cF = vzero<T>();
-      cw = vzero<T>();
-      cv = vzero<T>();
+      cn = vzero<double>();
+      cF = vzero<double>();
+      cw = vzero<double>();
+      cv = vzero<double>();
     }
     if (l == 0) {
       cn = cn + An;
@@ -257,16 +233,16 @@ __device__ __forceinline__ void kin_backward(const KinTopo& C, const double* sb,
       cw = cw + Aw;
       cv = cv + Av;
     }
-    const St<T> s = load_state(sb, l, dir, T());
+    const St<double> s = load_state(sb, l);
     // ---- local adjoints of body l
     {
       const double m = C.mass[l];
-      const V3<T> c = s.o + s.d;
-      const V3<T> cd = s.v + cross(s.w, s.d);
-      const V3<T> cbar = scale(m, cross(cd - xd, S.hb) + S.wc);
-      const V3<T> cdbar = scale(m, cross(S.hb, c - xc));
-      const V3<T> Iw = iw_omega(sb, l, dir, s);
-      const V3<T> Ih = iw_hbar(sb, l, dir, S.hb, T());
+      const D3 c = s.o + s.d;
+      const D3 cd = s.v + cross(s.w, s.d);
+      const D3 cbar = scale(m, cross(cd - xd, S.hb) + S.wc);
+      const D3 cdbar = scale(m, cross(S.hb, c - xc));
+      const D3 Iw = iw_omega(sb, l);
+      const D3 Ih = iw_hbar(sb, l, S.hb);
       cF = cF + cbar;
       cn = cn + cross(s.d, cbar) + cross(s.d, cross(cdbar, s.w)) + cross(Iw, S.hb) + cross(Ih, s.w);
       cv = cv + cdbar;
@@ -282,7 +258,7 @@ __device__ __forceinline__ void kin_backward(const KinTopo& C, const double* sb,
       if (l == C.chest_body) cn = cn + S.chestN;
     }
     if (C.slot[l] >= 0) {
-      const double* sl = slot + C.slot[l] * 12 * SW * 32 + lane;
+      const double* sl = slot + C.slot[l] * 12 * 32 + lane;
       slot_get(cn, sl, 0);
       slot_get(cF, sl, 3);
       slot_get(cw, sl, 6);
@@ -293,11 +269,11 @@ __device__ __forceinline__ void kin_backward(const KinTopo& C, const double* sb,
     emit.joint(l, dot(s.ax, cn), dot(s.ax, cw));
     // ---- contribution to the parent
     const int p = C.parent[l];
-    V3<T> rho, wpar;
-    parent_link(sb, l, p, dir, rho, wpar);
+    D3 rho, wpar;
+    parent_link(sb, l, p, rho, wpar);
     const double sd = zs[Z_SD + l - 1];
-    const V3<T> pn = cn + cross(rho, cF) + scale(sd, cross(s.ax, cw)) + cross(rho, cross(cv, wpar));
-    const V3<T> pw = cw + cross(rho, cv);
+    const D3 pn = cn + cross(rho, cF) + scale(sd, cross(s.ax, cw)) + cross(rho, cross(cv, wpar));
+    const D3 pw = cw + cross(rho, cv);
     if (p == l - 1) {
       cn = pn;
       cw = pw;  // cF, cv carry unchanged
@@ -307,7 +283,7 @@ __device__ __forceinline__ void kin_backward(const KinTopo& C, const double* sb,
       Aw = Aw + pw;
       Av = Av + cv;
     } else {
-      double* sl = slot + C.slot[p] * 12 * SW * 32 + lane;
+      double* sl = slot + C.slot[p] * 12 * 32 + lane;
       slot_add(sl, 0, pn);
       slot_add(sl, 3, cF);
       slot_add(sl, 6, pw);
@@ -324,9 +300,9 @@ __device__ __forceinline__ void kin_backward(const KinTopo& C, const double* sb,
 //   (1) primal_adjoint_pass: the adjoints of the Lagrangian (true multipliers as seeds) are the same
 //       for every direction; they are computed ONCE per warp, lane = body, accumulated leaf-to-root by
 //       depth level, and left in shared memory (SB_ACC totals, SB_CB / SB_CDB local terms);
-//   (2) kin_tangent_sweep: each lane propagates only the TANGENT of those adjoints along its
-//       direction (product rule with the staged primal values) -- 2/3 of the dual-number arithmetic
-//       and half of its registers.
+//   (2) kin_tangent_sweep_packed: only the TANGENT of those adjoints is propagated along every
+//       direction (product rule with the staged primal values) -- 2/3 of the arithmetic of a sweep in
+//       dual numbers and half of its registers.
 struct SeedsP {
   D3 wc, hb, footF[2], footN[2], chestN;
 };
@@ -391,100 +367,8 @@ __device__ __forceinline__ void primal_adjoint_pass(const KinTopo& T, double* sb
 __device__ __forceinline__ D3 tangent_of(const V3<Dual>& a) { return v3<double>(a.x.d, a.y.d, a.z.d); }
 __device__ __forceinline__ D3 primal_of(const V3<Dual>& a) { return v3<double>(a.x.v, a.y.v, a.z.v); }
 
-template <class Emit>
-__device__ __forceinline__ void kin_tangent_sweep(const KinTopo& C, const double* sb, const double* zs,
-                                                  const Dir& dir, D3 hb, const SeedsT& S, D3 txc, D3 txd, double* slot,
-                                                  Emit& emit, D3& n0, D3& w0, D3& v0) {
-  const int nb = C.nb;
-  const int lane = threadIdx.x & 31;
-  const D3 zero = v3<double>(0.0, 0.0, 0.0);
-  for (int i = 0; i < C.n_slots * 12; ++i) slot[i * 32 + lane] = 0.0;
-  D3 cn = zero, cF = zero, cw = zero, cv = zero;
-  D3 An = zero, AF = zero, Aw = zero, Av = zero;
-  for (int l = nb - 1; l >= 0; --l) {
-    if (!C.carry[l]) cn = cF = cw = cv = zero;
-    if (l == 0) {
-      cn = cn + An;
-      cF = cF + AF;
-      cw = cw + Aw;
-      cv = cv + Av;
-    }
-    const double* bl = sb + l * SB_STRIDE;
-    const St<Dual> s = load_state(sb, l, dir, Dual());
-    const D3 d = primal_of(s.d), w = primal_of(s.w), ax = primal_of(s.ax);
-    const D3 to = tangent_of(s.o), td = tangent_of(s.d), tw = tangent_of(s.w), tv = tangent_of(s.v),
-             tax = tangent_of(s.ax);
-    const double in = ((dir.mask >> l) & 1u) ? 1.0 : 0.0;
-    const D3 a = scale(in, dir.alpha);
-    {
-      const double m = C.mass[l];
-      const double* I = bl + SB_I;
-      const D3 cbar = ld3(bl + SB_CB), cdbar = ld3(bl + SB_CDB), Ih = ld3(bl + SB_IH), Iw = ld3(bl + SB_L);
-      const D3 tc = to + td;
-      const D3 tcd = tv + cross(tw, d) + cross(w, td);
-      const D3 tcbar = scale(m, cross(tcd - txd, hb));
-      const D3 tcdbar = scale(m, cross(hb, tc - txc));
-      const D3 tIw = symmul(I, tw - cross(a, w)) + cross(a, Iw);
-      const D3 tIh = cross(a, Ih) - symmul(I, cross(a, hb));
-      cF = cF + tcbar;
-      cn = cn + cross(td, cbar) + cross(d, tcbar) + cross(td, cross(cdbar, w)) +
-           cross(d, cross(tcdbar, w) + cross(cdbar, tw)) + cross(tIw, hb) + cross(tIh, w) + cross(Ih, tw);
-      cv = cv + tcdbar;
-      cw = cw + cross(td, cdbar) + cross(d, tcdbar) + tIh;
-      if (l == C.foot_body[0]) {
-        cF = cF + S.footF[0];
-        cn = cn + S.footN[0];
-      }
-      if (l == C.foot_body[1]) {
-        cF = cF + S.footF[1];
-        cn = cn + S.footN[1];
-      }
-      if (l == C.chest_body) cn = cn + S.chestN;
-    }
-    if (C.slot[l] >= 0) {
-      const double* sl = slot + C.slot[l] * 12 * 32 + lane;
-      slot_get(cn, sl, 0);
-      slot_get(cF, sl, 3);
-      slot_get(cw, sl, 6);
-      slot_get(cv, sl, 9);
-    }
-    if (l == 0) break;
-    // primal totals of body l (all children included)
-    const D3 np = ld3(bl + SB_ACC), Fp = ld3(bl + SB_ACC + 3), wp = ld3(bl + SB_ACC + 6), vp = ld3(bl + SB_ACC + 9);
-    emit.joint_t(l, dot(tax, np) + dot(ax, cn), dot(tax, wp) + dot(ax, cw));
-    const int p = C.parent[l];
-    const D3 rho = ld3(bl + SB_RHO), wpar = ld3(sb + p * SB_STRIDE + SB_W);
-    const double inp = ((dir.mask >> p) & 1u) ? 1.0 : 0.0;
-    const D3 ap = scale(inp, dir.alpha);
-    const D3 trho = cross(ap, rho);
-    const D3 twpar = cross(ap, wpar - dir.wpi) + scale(inp, dir.u);
-    const double sd = zs[Z_SD + l - 1];
-    const D3 pn = cn + cross(trho, Fp) + cross(rho, cF) + scale(sd, cross(tax, wp) + cross(ax, cw)) +
-                  cross(trho, cross(vp, wpar)) + cross(rho, cross(cv, wpar) + cross(vp, twpar));
-    const D3 pw = cw + cross(trho, vp) + cross(rho, cv);
-    if (p == l - 1) {
-      cn = pn;
-      cw = pw;
-    } else if (p == 0) {
-      An = An + pn;
-      AF = AF + cF;
-      Aw = Aw + pw;
-      Av = Av + cv;
-    } else {
-      double* sl = slot + C.slot[p] * 12 * 32 + lane;
-      slot_add(sl, 0, pn);
-      slot_add(sl, 3, cF);
-      slot_add(sl, 6, pw);
-      slot_add(sl, 9, cv);
-    }
-  }
-  n0 = cn;
-  w0 = cw;
-  v0 = cv;
-}
-
 // ---------------------------------------------------------------------------------------------------
-// Packed tangent sweep.  In kin_tangent_sweep lane d walks all the bodies although direction d only
+// Packed tangent sweep.  In a plain sweep lane d would walk all the bodies although direction d only
 // moves its own sub-tree: of the 27 x 23 body steps 188 carry non-zero state tangents and 92 more are
 // pure propagation through the ancestors of the joint.  Here those (direction, body) steps are TASKS,
 // list-scheduled by the host (api.cu::build_sweep_schedule) on the 32 lanes in ~12 rounds instead of
@@ -671,73 +555,15 @@ __device__ __forceinline__ void quat_maps(const double* q, const double* qd, D3*
   for (int a = 0; a < 4; ++a) quat_map(q, qd, a, g[a], u[a], w[a]);
 }
 
-struct JacEmit {
-  const KinoConst* C;
-  const int* map;  // jk_map row of this knot
-  double* jac;     // instance base
-  double* gbuf;    // shared: grad_f accumulation for the kinematic variables
-  int lane, k;
-  double gscale;   // chest lane: 2 w_frame (phi - 3)
-  bool write;
-  // local bases inside JK (kino_layout.py::_enumerate_jk)
-  __device__ __forceinline__ int base_q() const {
-    if (lane < 24) return 4 + lane * 27;
-    if (lane < 27) return 4 + 648 + (lane - 24) * 27;
-    if (lane < 30) return 4 + 648 + 81 + (lane - 27) * 57 + 7;  // after vb(3), qd(4)
-    return -1;
-  }
-  double* stage;   // non-null: values go to shared memory and are scattered after the sweep
-  __device__ __forceinline__ void put(int e, double v) const {
-    if (stage) {
-      stage[e] = v;
-      return;
-    }
-    const int slot = map[e];
-    if (slot >= 0) jac[slot] = v;
-  }
-  // Scatter slots of the two entries the sweep emits at body l, loaded one step ahead (prefetch(l) is
-  // called at the top of the iteration) so that the stores do not wait for their own map loads.
-  int sbase, sdbase, pre_s, pre_sd;
-  __device__ __forceinline__ void init_bases() {
-    sdbase = -1;
-    if (lane < 27) sbase = base_q() + 4;
-    else if (lane < 30) {
-      const int b = 4 + 648 + 81 + (lane - 27) * 57;
-      sdbase = b + 11;
-      sbase = b + 34;
-    } else sbase = lane == 30 ? 4 + 648 + 81 + 171 : -1;
-    pre_s = pre_sd = -1;
-  }
-  __device__ __forceinline__ void prefetch(int l) {
-    if (stage || !write || l < 1) return;
-    pre_s = sbase >= 0 ? map[sbase + l - 1] : -1;
-    pre_sd = sdbase >= 0 ? map[sdbase + l - 1] : -1;
-  }
-  __device__ __forceinline__ void joint(int l, double sbar, double sdbar) const {
-    const int j = l - 1;
-    if (lane == 31) {
-      gbuf[34 + j] += gscale * sbar;  // gbuf order: vb3 qd4 q4 sd23 s23 -> s at 34
-      return;
-    }
-    if (!write) return;
-    if (stage) {
-      if (sbase >= 0) stage[sbase + j] = sbar;
-      if (sdbase >= 0) stage[sdbase + j] = sdbar;
-      return;
-    }
-    if (pre_s >= 0) jac[pre_s] = sbar;
-    if (pre_sd >= 0) jac[pre_sd] = sdbar;
-  }
-};
-
 struct HessEmit {
   const int* map;  // hk_map row of this knot
   double* hess;    // instance base
   int dirj;        // direction index 0..26, or -1 (idle lane)
   double add_sd, add_s;  // joint-regularisation terms on (sd_j, s_j), (s_j, s_j) for joint lanes
   double* stage;   // per-warp staging (HSTAGE doubles); scattered after the sweep
-  bool acc = false;  // packed sweep: the stage already holds the cross terms, entries are added
-  __device__ __forceinline__ void prefetch(int) {}
+  bool acc = false;  // the stage already holds the cross terms, entries are added
+  // stage is never null.  The direct-store branch and the `if (em.stage)` guard of the scatter stay because
+  // without them ptxas allocates the kernel differently and spills 12 bytes per thread.
   __device__ __forceinline__ void put(int row, double v) const {
     if (stage) {
       if (acc) stage[dirj * 57 + row] += v;
@@ -747,33 +573,12 @@ struct HessEmit {
     const int slot = map[dirj * 57 + row];
     if (slot >= 0) hess[slot] = v;
   }
-  __device__ __forceinline__ void joint_t(int l, double tsbar, double tsdbar) const {
-    if (dirj < 0) return;
-    const int j = l - 1;
-    const bool own = (dirj - 4 == j);
-    put(7 + j, tsdbar + (own ? add_sd : 0.0));   // rows: vb3 qd4 sd23 q4 s23
-    put(34 + j, tsbar + (own ? add_s : 0.0));
-  }
-  __device__ __forceinline__ void joint(int l, Dual sbar, Dual sdbar) const { joint_t(l, sbar.d, sdbar.d); }
 };
 
-// Measured on B200 (tools/time_kino.py): the dual sweep is fastest with the full 255 registers
-// (2 CTAs/SM; 168 registers spill 1 KB/thread and lose 12%), the fp64-only variant with 168
-// registers (3 CTAs/SM, -19%).
+// Launch bounds, measured on B200 (tools/time_kino.py): the Hessian kernel is fastest with the full 255 registers
+// (2 CTAs/SM; 168 registers spill 1 KB/thread and lose 12%), the lean kernel with 168 registers (3 CTAs/SM, -19%).
+constexpr int KIN_H_THREADS = 128, KIN_H_MIN_BLOCKS = 2;
 template <bool WITH_HESS>
-#ifndef KIN_H_MIN_BLOCKS
-#define KIN_H_MIN_BLOCKS 2
-#endif
-#ifndef HB_KIN_JAC_LIST
-#define HB_KIN_JAC_LIST 1  // Jacobian scatter through the destination-sorted list (measured 1.145 ms against 1.162 ms in entry order)
-#endif
-#ifndef HB_KIN_HESS_LIST
-#define HB_KIN_HESS_LIST 0  // 1: Hessian scatter through the destination-sorted list.  Measured: 1.161 ms against 1.145 ms in
-                            // entry order -- the staged columns are read conflict-free in entry order, in destination order not
-#endif
-#ifndef KIN_H_THREADS
-#define KIN_H_THREADS 128
-#endif
 __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? KIN_H_MIN_BLOCKS : 3) kino_kin_kernel(
     const __grid_constant__ KinTopo T,
                                                        const KinoConst* __restrict__ Cp, unsigned mask,
@@ -1146,12 +951,10 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
   HB_PHASE(0, 3);  // g rows, costs
   const bool want_jac = (mask & HB_EVAL_JAC_G) != 0, want_grad = (mask & HB_EVAL_GRAD_F) != 0;
   double* slot = sm + L.slot;
-  Dir nodir;
-  nodir.mask = 0u;
   // ------------------------------------------------------------------ adjoint sweep, fp64: Jacobian rows
   // (Jacobian-only kernel.  The Hessian kernel gets the same values from forward tangents that its
   // direction lanes need anyway -- see "forward-mode Jacobian" below.)
-  if ((want_jac || want_grad) && !(WITH_HESS && HB_FWD_JAC)) {
+  if ((want_jac || want_grad) && !WITH_HESS) {
     Seeds<double> S;
     S.wc = S.hb = S.footF[0] = S.footF[1] = S.footN[0] = S.footN[1] = S.chestN = v3<double>(0.0, 0.0, 0.0);
     if (lane < 24) {
@@ -1181,19 +984,16 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
       S.chestN = mG;
     }
     JacEmit em;
-    em.C = Cp;
     const int2 jkm = *reinterpret_cast<const int2*>(&T.knot_maps[k].jk_base);  // {base, table offset}
     em.map = C.jk_map + jkm.y;
     em.jac = jac + b * T.nnz_j + jkm.x;
     em.gbuf = gbuf;
     em.lane = lane;
-    em.k = k;
     em.gscale = k1 ? 2.0 * T.w_frame * (phi - 3.0) : 0.0;
     em.write = want_jac;
-    em.stage = (WITH_HESS ? HB_KIN_STAGE : HB_KIN_STAGE_F) ? sm + L.stage : nullptr;
     em.init_bases();
     D3 n0, w0, v0;
-    kin_backward<double>(T, sb, zs, nodir, S, xc, xcd, slot, em, n0, w0, v0);
+    kin_backward(T, sb, zs, S, xc, xcd, slot, em, n0, w0, v0);
     // base chain rule
     D3 gq[4], uq[4], wq[4];
     const double qraw[4] = {q0, q1, q2, q3};
@@ -1226,21 +1026,6 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
       if (lane < 4) em.put(lane, 2.0 * qraw[lane]);  // unit quaternion row
     }
     __syncwarp();
-    if (em.stage && want_jac) {
-      // scatter the staged rows: coalesced map reads, no load->store dependency inside the sweep
-      const double* st = sm + L.stage;
-      const unsigned* lst = C.jk_list + jkm.y;  // destination-sorted: entry << 16 | slot
-      const int n = T.knot_maps[k].jk_cnt;
-      for (int eb = lane; eb < n; eb += 256) {  // 8 list loads in flight before the dependent stores
-        unsigned w[8];
-#pragma unroll
-        for (int u = 0; u < 8; ++u) w[u] = (eb + 32 * u) < n ? lst[eb + 32 * u] : 0xffffffffu;
-#pragma unroll
-        for (int u = 0; u < 8; ++u)
-          if (w[u] != 0xffffffffu) em.jac[w[u] & 0xffffu] = st[w[u] >> 16];
-      }
-      __syncwarp();
-    }
     if (want_grad) {
       // gbuf order vb3 qd4 q4 sd23 s23 -> x offsets
       double* gf = grad_f + b * T.n_x + (long)k * T.x_stride;
@@ -1257,7 +1042,7 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
     }
   }
   if (!WITH_HESS) return;
-  if (!with_l && !(HB_FWD_JAC && (want_jac || want_grad))) return;
+  if (!with_l && !(want_jac || want_grad)) return;
   // ------------------------------------------------------------------ adjoint sweep, dual: Hessian columns
   {
     const int dirj = lane < 27 ? lane : -1;
@@ -1434,8 +1219,6 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
       }
     }
     __syncwarp();  // the stage is reused for the Jacobian columns below
-    const V3<Dual> xcD = lift<Dual>(xc, scale(1.0 / M, tP));
-    const V3<Dual> xdD = lift<Dual>(xcd, scale(1.0 / M, tPd));
     const double inL = ((dir.mask >> T.foot_body[0]) & 1u) ? 1.0 : 0.0;
     const double inR = ((dir.mask >> T.foot_body[1]) & 1u) ? 1.0 : 0.0;
     const double inC = ((dir.mask >> T.chest_body) & 1u) ? 1.0 : 0.0;
@@ -1451,7 +1234,6 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
                   cross(ac, v3<double>(G[2], G[5], G[8])).z;
     }
     HB_PHASE(0, 5);  // direction tangents of P, Pdot, h, feet distance, trace
-#if HB_FWD_JAC
     // ---------------------------------------------------------------- forward-mode Jacobian
     // The direction lanes already hold the tangent of every link state along q_a / s_j, so column j of
     // the kinematic rows is a few products here; the velocity columns of the momentum rows (the map is
@@ -1499,8 +1281,8 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
       if (want_jac) {
         const int4 jkm = *reinterpret_cast<const int4*>(&T.knot_maps[k].jk_base);  // {base, offset, count, -}
         double* jb = jac + b * T.nnz_j + jkm.x;
-#if HB_KIN_JAC_LIST
-        const unsigned* lst = C.jk_list + jkm.y;  // destination-sorted: entry << 16 | slot
+        // destination-sorted list: entry << 16 | slot (measured 1.145 ms against 1.162 ms in entry order)
+        const unsigned* lst = C.jk_list + jkm.y;
         const int n = jkm.z;
         // KIN_SCAT list loads in flight before the dependent stores: <= 927 entries in two trips
         for (int eb = lane; eb < n; eb += 32 * KIN_SCAT) {
@@ -1511,18 +1293,6 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
           for (int u = 0; u < KIN_SCAT; ++u)
             if (w[u] != 0xffffffffu) jb[w[u] & 0xffffu] = stg[w[u] >> 16];
         }
-#else
-        const int* jmap = C.jk_map + jkm.y;
-        const int n = T.n_jk;
-        for (int eb = lane; eb < n; eb += 32 * KIN_SCAT) {  // entry order: 927 entries in two trips
-          int sl[KIN_SCAT];
-#pragma unroll
-          for (int u = 0; u < KIN_SCAT; ++u) sl[u] = (eb + 32 * u) < n ? jmap[eb + 32 * u] : -1;
-#pragma unroll
-          for (int u = 0; u < KIN_SCAT; ++u)
-            if (sl[u] >= 0) jb[sl[u]] = stg[eb + 32 * u];
-        }
-#endif
       }
       if (want_grad) {
         // gbuf order vb3 qd4 q4 sd23 s23 -> x offsets
@@ -1540,7 +1310,6 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
       }
       __syncwarp();  // the Hessian columns reuse the stage
     }
-#endif
     HB_PHASE(0, 7);  // Jacobian scatter, grad_f
     if (!with_l) return;  // Jacobian / gradient only: done
     Seeds<Dual> S;
@@ -1549,7 +1318,7 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
       // multipliers from lamk (loaded at the top of the kernel; rows that do not exist hold 0)
       S.wc = scale(-1.0 / M, ld3(lamk + 24));
       S.hb = scale(-1.0 / mass_p, ld3(lamk + 27));
-      // stage I^w hbar (same for every lane of the dual sweep)
+      // stage I^w hbar (same for every direction)
       if (lane < nb) st3(sb + lane * SB_STRIDE + SB_IH, symmul(sb + lane * SB_STRIDE + SB_I, S.hb));
       __syncwarp();
     }
@@ -1598,7 +1367,7 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
     HessEmit em;
     em.map = C.hk_map + T.knot_maps[k].hk_off;
     em.hess = hess + b * T.nnz_h + T.knot_maps[k].hk_base;
-    em.stage = HB_KIN_STAGE ? sm + L.stage : nullptr;
+    em.stage = sm + L.stage;
     em.dirj = dirj;
     em.add_sd = em.add_s = 0.0;
     if (lane >= 4 && lane < 27 && k1) {
@@ -1609,10 +1378,6 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
     V3<Dual> n0, w0, v0;
     const double lu_pre = lamk[31];  // read now: the slots of the packed sweep alias gbuf + lamk + slot
     const D3 lam_al = cross(ld3(lamk + 27), dir.alpha);  // quaternion lanes: velocity rows of their column (below)
-#ifdef HB_DUAL_SWEEP
-    // reference implementation: the whole adjoint sweep in dual arithmetic on every lane
-    kin_backward<Dual>(T, sb, zs, dir, S, xcD, xdD, slot, em, n0, w0, v0);
-#else
     {
       SeedsP SP;
       SeedsT ST;
@@ -1632,7 +1397,6 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
       primal_adjoint_pass(T, sb, zs, SP, xc, xcd, my_depth, my_rank, my_parent, my_mass);
       HB_PHASE(0, 9);  // primal adjoint pass
       D3 tn0, tw0, tv0;
-#if HB_SWEEP_PACKED
       {
         // Hessian of -hb.(P x Pdot)/M (see kin_tangent_sweep_packed) for every (direction, row), which also
         // initialises the stage; rows: vb3 qd4 sd23 (velocity lane = row) q4 s23 (direction lane = row - 30)
@@ -1703,14 +1467,10 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
         // the quaternion columns' rows vb, qd, q are complete (cross term included): stored, not added
         em.acc = lane >= 4;
       }
-#else
-      kin_tangent_sweep(T, sb, zs, dir, S.hb, ST, tangent_of(xcD), tangent_of(xdD), slot, em, tn0, tw0, tv0);
-#endif
       n0 = lift<Dual>(ld3(sb + SB_ACC), tn0);
       w0 = lift<Dual>(ld3(sb + SB_ACC + 6), tw0);
       v0 = lift<Dual>(ld3(sb + SB_ACC + 9), tv0);
     }
-#endif
     // Root chain rule dq_a = n0.g_a + w0.u_a, dqd_a = w0.w_a along direction d: the tangents of the root totals
     // against the maps, plus (quaternion directions d < 4 only) the curvature of the maps against the primal
     // totals, K[a][d] = n0.dg_a/dq_d + w0.du_a/dq_d and Kd[a][d] = w0.dw_a/dq_d.  K and Kd are the same on
@@ -1748,30 +1508,17 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
         const double extra = (a == lane && k1) ? 2.0 * sg * T.w_bq * nqd + 2.0 * lu : 0.0;
         em.put(3 + a, dqd);
         em.put(30 + a, dq + extra);
-#if HB_SWEEP_PACKED && !defined(HB_DUAL_SWEEP)
         // row s_j of column q_a by symmetry, on top of the cross term already staged there
         if (lane >= 4) em.stage[a * 57 + 34 + lane - 4] += dq;
-#endif
       }
     }
     HB_PHASE(0, 12);  // root chain rule
     __syncwarp();
     if (em.stage) {
-      // scatter the staged columns (27 directions x 57 rows) with coalesced map reads
+      // scatter the staged columns (27 directions x 57 rows) with coalesced map reads, in entry order: the staged
+      // columns are read conflict-free in entry order, in destination order not (a destination-sorted list measured
+      // 1.161 ms against 1.145 ms)
       const double* st = sm + L.stage;
-#if HB_KIN_HESS_LIST
-      const int2 hkl = *reinterpret_cast<const int2*>(&T.knot_maps[k].hk_off);  // {offset, count}
-      const unsigned* lst = C.hk_list + hkl.x;  // destination-sorted: entry << 16 | slot; mirrored pairs are absent
-      const int n = hkl.y;
-      for (int eb = lane; eb < n; eb += 32 * KIN_SCAT) {
-        unsigned w[KIN_SCAT];
-#pragma unroll
-        for (int u = 0; u < KIN_SCAT; ++u) w[u] = (eb + 32 * u) < n ? lst[eb + 32 * u] : 0xffffffffu;
-#pragma unroll
-        for (int u = 0; u < KIN_SCAT; ++u)
-          if (w[u] != 0xffffffffu) em.hess[w[u] & 0xffffu] = st[w[u] >> 16];
-      }
-#else
       for (int eb = lane; eb < HSTAGE; eb += 32 * KIN_SCAT) {  // entry order: 1539 entries in three trips
         int sl[KIN_SCAT];
 #pragma unroll
@@ -1780,7 +1527,6 @@ __global__ void __launch_bounds__(WITH_HESS ? KIN_H_THREADS : 128, WITH_HESS ? K
         for (int u = 0; u < KIN_SCAT; ++u)
           if (sl[u] >= 0) em.hess[sl[u]] = st[eb + 32 * u];
       }
-#endif
     }
     // velocity-diagonal entries (HK2): quaternion-velocity cost, joint regularisation
     if (lane < 27) {
