@@ -118,7 +118,8 @@ static cudaError_t ensure_kernel_attributes(int dev) {
   if ((e = cudaFuncSetAttribute(hb::kino_contact_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, big)) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(hb::kino_kin_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big)) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(hb::kino_kin_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, big)) != cudaSuccess) return e;
-  if ((e = cudaFuncSetAttribute(hb::pose_contact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, big)) != cudaSuccess) return e;
+  if ((e = cudaFuncSetAttribute(hb::pose_contact_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, big)) != cudaSuccess) return e;
+  if ((e = cudaFuncSetAttribute(hb::pose_contact_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, big)) != cudaSuccess) return e;
   const int lu_big = 210 * 1024;
   if ((e = cudaFuncSetAttribute(hb::lu_factor_kernel<1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, lu_big)) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(hb::lu_factor_kernel<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, lu_big)) != cudaSuccess) return e;
@@ -269,9 +270,9 @@ extern "C" int hb_kino_create(const int32_t* icfg, const double* dcfg, const int
     delete h;
     return fail(HB_ERR_INVALID, "hb_kino_create: kind must be 0 (kinodynamic) or 1 (pose finder)");
   }
-  if (C.kind == 1 && (C.N != 1 || C.terrain != 0)) {
+  if (C.kind == 1 && C.N != 1) {
     delete h;
-    return fail(HB_ERR_UNSUPPORTED, "hb_kino_create: the pose finder is a single-knot problem on the planar terrain");
+    return fail(HB_ERR_UNSUPPORTED, "hb_kino_create: the pose finder is a single-knot problem");
   }
   if (C.terrain != 0 && C.terrain != 1) {
     delete h;
@@ -781,10 +782,15 @@ extern "C" int hb_eval(hb_handle h, uint32_t mask, const double* x, const double
     }
     const size_t smem = (size_t)(C.kind == 1 ? hb::pose_contact_smem_layout(C.n_hc) : hb::kino_contact_smem_layout(C.n_hc)).total *
                         sizeof(double) * warps_per_block;
-    if (C.kind == 1) {
-      hb::pose_contact_kernel<<<grid, 32 * warps_per_block, smem, st>>>(h->dev, mask, x, p, (long)p_stride, lam_g, sigma,
-                                                                       d_fpart, grad_f, g, jac_vals, hess_vals,
-                                                                       (long)batch);
+    // the shared block holds the kernel's n_hc Hessian accumulators (191 planar, 255 on the smooth steps)
+    if (C.kind == 1 && C.terrain == 0) {
+      hb::pose_contact_kernel<0><<<grid, 32 * warps_per_block, smem, st>>>(h->dev, mask, x, p, (long)p_stride, lam_g, sigma,
+                                                                          d_fpart, grad_f, g, jac_vals, hess_vals,
+                                                                          (long)batch);
+    } else if (C.kind == 1) {
+      hb::pose_contact_kernel<1><<<grid, 32 * warps_per_block, smem, st>>>(h->dev, mask, x, p, (long)p_stride, lam_g, sigma,
+                                                                          d_fpart, grad_f, g, jac_vals, hess_vals,
+                                                                          (long)batch);
     } else if (C.terrain == 0)
       hb::kino_contact_kernel<0><<<grid, 32 * warps_per_block, smem, st_contact>>>(h->topo, h->dev, mask, x, p, (long)p_stride,
                                                                                   lam_g, sigma, d_fpart, grad_f, g, jac_vals,

@@ -105,6 +105,31 @@ __device__ __forceinline__ void smooth_terrain_frame(const double* __restrict__ 
 __device__ __forceinline__ TJ tj_dot(const TJ* a, D3 b) { return b.x * a[0] + b.y * a[1] + b.z * a[2]; }
 __device__ __forceinline__ double comp(D3 a, int i) { return i == 0 ? a.x : (i == 1 ? a.y : a.z); }
 
+// A contact force in the terrain frame at the point, as series in the point position: its normal component
+// N = n.f (contacts.py:24), its tangential components X = x.f, Y = y.f, and the friction-cone margin
+// mu^2 N^2 - X^2 - Y^2 (contacts.py:54-66), as the pose-finder contact kernel uses them.  kino_contact.cu spells the
+// same expressions inline: routed through these helpers its smooth-terrain Hessian changes in the last bits.
+struct FrameForce {
+  TJ N, X, Y, fric;
+};
+__device__ __forceinline__ FrameForce frame_force(const TFrame& F, D3 f, double mu) {
+  FrameForce r;
+  r.N = tj_dot(F.n, f);
+  r.X = tj_dot(F.xh, f);
+  r.Y = tj_dot(F.yh, f);
+  r.fric = (mu * mu) * (r.N * r.N) - r.X * r.X - r.Y * r.Y;
+  return r;
+}
+// d (friction-cone margin) / d f_d, as a series in the point position
+__device__ __forceinline__ TJ frame_force_fric_df(const TFrame& F, const FrameForce& r, double mu, int d) {
+  return (2.0 * mu * mu) * (r.N * F.n[d]) - 2.0 * (r.X * F.xh[d]) - 2.0 * (r.Y * F.yh[d]);
+}
+// d2 (friction-cone margin) / d f_a d f_b at the point
+__device__ __forceinline__ double frame_force_fric_dff(const TFrame& F, double mu, int a, int b) {
+  return 2.0 * mu * mu * F.n[a].c[0] * F.n[b].c[0] - 2.0 * F.xh[a].c[0] * F.xh[b].c[0] -
+         2.0 * F.yh[a].c[0] * F.yh[b].c[0];
+}
+
 // Values and derivatives of every terrain-dependent row / cost of one contact point.
 struct SmoothPoint {
   // rows (Taylor series in the point position, all other variables frozen)

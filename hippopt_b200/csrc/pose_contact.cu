@@ -1,5 +1,5 @@
 // pose_contact.cu -- contact constraints, static balance and regularisation costs of the humanoid
-// pose finder (BASELINE config 2): one warp per instance (single knot); PlanarTerrain.
+// pose finder (BASELINE config 2): one warp per instance (single knot).
 //
 // Rows / costs (reference file:line restated):
 //   relaxed complementarity  eps - h(p) n.(f mass) >= 0   humanoid_pose_finder/planner.py:704-726,
@@ -13,10 +13,74 @@
 //
 // Local Jacobian order: hippopt_b200/pose_layout.py::_enumerate_jp.  Cost weights reuse KinoConst
 // slots: w_centroid = com, w_ratio = average force, w_swing = point position, w_fd = force.
+//
+// TERRAIN: 0 = PlanarTerrain (h = p_z, n = e_z, R_t = I), 1 = the two smooth steps of the stairs (BASELINE config 5,
+// kino_smooth.cuh) with their ten parameters at p + po_terrain.  On the steps h depends on the whole point position and
+// n, R_t on (x, y): lane i < 8 evaluates the terrain frame of point i as order-2 series in its position and forms the
+// four terrain rows, their 25 Jacobian entries and the multiplier-weighted second derivatives from them.
 #include "kino_const.cuh"
+#include "kino_smooth.cuh"
 
 namespace hb {
 
+// Terrain rows of contact point i on the smooth steps: relaxed complementarity eps - h n.(f mass), height h, normal
+// force n.f and friction-cone margin mu^2 (n.f)^2 - (x.f)^2 - (y.f)^2 (g rows, local Jacobian entries 25 i .. 25 i + 18
+// in pose_layout.py::_enumerate_jp order, and the multiplier-weighted (p, p), (p, f), (f, f) second derivatives).
+template <class JPut, class HAdd, class LamRow>
+__device__ __forceinline__ void smooth_point_rows(const KinoConst& C, const double* __restrict__ tp, int i, D3 ppos, D3 pf,
+                                                  double mass, double eps, double mu, bool want_g, bool want_jac,
+                                                  bool want_hess, double* __restrict__ gb, JPut& jput, HAdd& hadd,
+                                                  LamRow& lamrow) {
+  const int fb_ = i * HB_KF_PT_COUNT, o = 15 * i;
+  TFrame F;
+  smooth_terrain_frame(tp, ppos.x, ppos.y, ppos.z, F);
+  const FrameForce ff = frame_force(F, pf, mu);
+  const TJ hN = F.h * ff.N;  // h n.f: the complementarity row is eps - mass h n.f
+  if (want_g) {
+    int r = grow(C, fb_ + HB_KF_PT_DCC, 0, 0);
+    if (r >= 0) gb[r] = eps - mass * hN.c[0];
+    r = grow(C, fb_ + HB_KF_PT_HEIGHT, 0, 0);
+    if (r >= 0) gb[r] = F.h.c[0];
+    r = grow(C, fb_ + HB_KF_PT_NORMAL, 0, 0);
+    if (r >= 0) gb[r] = ff.N.c[0];
+    r = grow(C, fb_ + HB_KF_PT_FRICTION, 0, 0);
+    if (r >= 0) gb[r] = ff.fric.c[0];
+  }
+  if (want_jac) {
+    // complementarity (p, f), height (p), normal (p_xy, f), friction (p_xy, f): n and R_t do not depend on z
+    const int b0 = 25 * i;
+    const double h0 = F.h.c[0];
+    for (int d = 0; d < 3; ++d) {
+      jput(b0 + d, -mass * hN.c[1 + d]);
+      jput(b0 + 3 + d, -mass * h0 * F.n[d].c[0]);
+      jput(b0 + 6 + d, F.h.c[1 + d]);
+      jput(b0 + 11 + d, F.n[d].c[0]);
+      jput(b0 + 16 + d, frame_force_fric_df(F, ff, mu, d).c[0]);
+    }
+    jput(b0 + 9, ff.N.c[1]);
+    jput(b0 + 10, ff.N.c[2]);
+    jput(b0 + 14, ff.fric.c[1]);
+    jput(b0 + 15, ff.fric.c[2]);
+  }
+  if (want_hess) {
+    const double lc = lamrow(fb_ + HB_KF_PT_DCC, 0), lh = lamrow(fb_ + HB_KF_PT_HEIGHT, 0);
+    const double ln = lamrow(fb_ + HB_KF_PT_NORMAL, 0), lf = lamrow(fb_ + HB_KF_PT_FRICTION, 0);
+    const double lcm = -lc * mass;
+    // the four rows weighted by their multipliers, as one series in the point position
+    const TJ Lp = lcm * hN + lh * F.h + ln * ff.N + lf * ff.fric;
+    int e = 0;
+    for (int a = 0; a < 3; ++a)
+      for (int bb = a; bb < 3; ++bb) hadd(o + Z_P + a, o + Z_P + bb, tj_hess(Lp, e++));
+    for (int d = 0; d < 3; ++d) {
+      const TJ Gf = lcm * (F.h * F.n[d]) + ln * F.n[d] + lf * frame_force_fric_df(F, ff, mu, d);  // d Lp / d f_d
+      for (int a = 0; a < 3; ++a) hadd(o + Z_P + a, o + Z_F + d, Gf.c[1 + a]);
+    }
+    for (int a = 0; a < 3; ++a)
+      for (int bb = a; bb < 3; ++bb) hadd(o + Z_F + a, o + Z_F + bb, lf * frame_force_fric_dff(F, mu, a, bb));
+  }
+}
+
+template <int TERRAIN>
 __global__ void __launch_bounds__(128) pose_contact_kernel(const KinoConst* __restrict__ Cp, unsigned mask,
                                                            const double* __restrict__ x, const double* __restrict__ p,
                                                            long p_stride, const double* __restrict__ lam,
@@ -51,6 +115,8 @@ __global__ void __launch_bounds__(128) pose_contact_kernel(const KinoConst* __re
   for (int i = lane; i < NCV; i += 32) gbuf[i] = 0.0;
   __syncwarp();
   const double mass = pp[C.po_mass], eps = pp[C.po_eps], mu = pp[C.po_mu];
+  // local Jacobian entries per contact point (complementarity, height, normal, friction, FK) and of the robot rows
+  constexpr int JC_PT = TERRAIN == 0 ? 13 : 25, JC_ROBOT = 8 * JC_PT;
   const double* refst = pp + C.po_init;  // references.state: per point (p, f, descriptor), pb, q, s, com
   double* gb = g + b * C.m;
   const double* lb = lam + b * C.m;
@@ -88,8 +154,13 @@ __global__ void __launch_bounds__(128) pose_contact_kernel(const KinoConst* __re
                              __shfl_sync(0xffffffffu, lin.z, 0));
   const D3 asum = v3<double>(__shfl_sync(0xffffffffu, ang.x, 0), __shfl_sync(0xffffffffu, ang.y, 0),
                              __shfl_sync(0xffffffffu, ang.z, 0));
+  if constexpr (TERRAIN == 1) {
+    if (lane < 8 && (want_g || want_jac || want_hess))
+      smooth_point_rows(C, pp + C.po_terrain, lane, ppos, pf, mass, eps, mu, want_g, want_jac, want_hess,
+                        gb, jput, hadd, lamrow);
+  }
   if (want_g) {
-    if (lane < 8) {
+    if (TERRAIN == 0 && lane < 8) {
       const int fb_ = lane * HB_KF_PT_COUNT;
       int r = grow(C, fb_ + HB_KF_PT_DCC, 0, 0);
       if (r >= 0) gb[r] = eps - ppos.z * (pf.z * mass);
@@ -177,7 +248,7 @@ __global__ void __launch_bounds__(128) pose_contact_kernel(const KinoConst* __re
   }
   // ---- Jacobian
   if (want_jac) {
-    if (lane < 8) {
+    if (TERRAIN == 0 && lane < 8) {
       const int b0 = 13 * lane;
       jput(b0 + 0, -pf.z * mass);
       jput(b0 + 1, -ppos.z * mass);
@@ -191,7 +262,14 @@ __global__ void __launch_bounds__(128) pose_contact_kernel(const KinoConst* __re
         jput(b0 + 10 + c, -1.0);
       }
     }
-    if (lane < 6) jput(104 + lane, lane < 3 ? 1.0 : -1.0);
+    if (TERRAIN == 1 && lane < 8) {
+      const int b0 = JC_PT * lane + 19;  // the FK entries follow the point's 19 terrain-row entries
+      for (int c = 0; c < 3; ++c) {
+        jput(b0 + c, 1.0);
+        jput(b0 + 3 + c, -1.0);
+      }
+    }
+    if (lane < 6) jput(JC_ROBOT + lane, lane < 3 ? 1.0 : -1.0);
     for (int e = lane; e < 126; e += 32) {
       double v;
       if (e < 24) v = 1.0;
@@ -204,19 +282,22 @@ __global__ void __launch_bounds__(128) pose_contact_kernel(const KinoConst* __re
         else if (e < 120) v = -eps3(a, bcol) * (zs[15 * i + Z_P + c] - zs[Z_COM + c]);
         else v = -eps3(a, bcol) * comp(fsum, c);
       }
-      jput(110 + e, v);
+      jput(JC_ROBOT + 6 + e, v);
     }
-    if (lane < HB_N_JOINTS) jput(236 + lane, 1.0);
+    if (lane < HB_N_JOINTS) jput(JC_ROBOT + 132 + lane, 1.0);
   }
   // ---- Hessian
   if (want_hess) {
     if (lane < 8) {
-      const int fb_ = lane * HB_KF_PT_COUNT, o = 15 * lane;
-      const double lc = lamrow(fb_ + HB_KF_PT_DCC, 0), lf = lamrow(fb_ + HB_KF_PT_FRICTION, 0);
-      hadd(o + Z_P + 2, o + Z_F + 2, -lc * mass);
-      hadd(o + Z_F, o + Z_F, -2.0 * lf);
-      hadd(o + Z_F + 1, o + Z_F + 1, -2.0 * lf);
-      hadd(o + Z_F + 2, o + Z_F + 2, 2.0 * mu * mu * lf);
+      const int o = 15 * lane;
+      if constexpr (TERRAIN == 0) {
+        const int fb_ = lane * HB_KF_PT_COUNT;
+        const double lc = lamrow(fb_ + HB_KF_PT_DCC, 0), lf = lamrow(fb_ + HB_KF_PT_FRICTION, 0);
+        hadd(o + Z_P + 2, o + Z_F + 2, -lc * mass);
+        hadd(o + Z_F, o + Z_F, -2.0 * lf);
+        hadd(o + Z_F + 1, o + Z_F + 1, -2.0 * lf);
+        hadd(o + Z_F + 2, o + Z_F + 2, 2.0 * mu * mu * lf);
+      }
       double La[3];
       for (int c = 0; c < 3; ++c) La[c] = lamrow(HB_KF_H_DYN, 3 + c);
       for (int a = 0; a < 3; ++a)

@@ -372,7 +372,8 @@ def _fill_model_tables(dcfg, model, foot_frames, chest_frame):
 class PoseEvaluator(KinoEvaluator):
     """Evaluator of the static pose finder
     (`/root/reference/src/hippopt/turnkey_planners/humanoid_pose_finder/planner.py:303-413`), the one
-    reference configuration IPOPT solves with the exact Hessian."""
+    reference configuration IPOPT solves with the exact Hessian.  ``PoseSettings(terrain="smooth_steps",
+    n_terrain_params=10)`` poses it on the stairs, with the steps' parameters appended to p."""
 
     def __init__(self, model: RobotModel, settings=None):
         from .pose_layout import PoseLayout, PoseSettings
@@ -385,7 +386,8 @@ class PoseEvaluator(KinoEvaluator):
         icfg = np.zeros(H["HB_KI_COUNT"], dtype=np.int32)
         ints = {
             "HORIZON": 1, "N_X": lay.n_x, "N_P": lay.n_p, "M": lay.m, "NNZ_J": lay.nnz_j, "NNZ_H": lay.nnz_h,
-            "N_JC": lay.n_jc, "N_JK": lay.n_jk, "N_HC": lay.n_hc, "TERRAIN": 0, "HAS_FINAL": 0, "HAS_PERIODICITY": 0,
+            "N_JC": lay.n_jc, "N_JK": lay.n_jk, "N_HC": lay.n_hc, "TERRAIN": 0 if s.terrain == "planar" else 1,
+            "HAS_FINAL": 0, "HAS_PERIODICITY": 0, "PO_TERRAIN": po.terrain,
             "H_INIT": 0, "PO_DESC0": po.desc0, "PO_MASS": po.mass, "PO_INIT": po.ref, "PO_GRAVITY": po.gravity,
             "PO_EPS": po.eps, "PO_MU": po.mu, "PO_MAX_S": po.max_s, "PO_MIN_S": po.min_s,
             "N_BODIES": model.n_bodies, "FOOT_BODY_L": model.frames[s.foot_frames[0]][0],

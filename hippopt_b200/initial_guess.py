@@ -10,6 +10,10 @@
   (interpolators.py -> csrc/interp.cu),
 * the references of get_references (:330-352) and the initial / final state parameters (:470-478).
 
+`stairs_step_guess` builds the same set-up for BASELINE config 5 (walking on stairs): the keyframe poses are solved on
+the smooth-step terrain (pose-finder evaluator with ``terrain="smooth_steps"``), and the contacts land on the first
+tread.
+
 Everything numeric runs on the GPU; the per-instance Python loop of the reference (one IPOPT solve after the other)
 is gone.  How far the interior-point driver gets on the plans built here (some converge, many do not) is recorded
 in DESIGN.md section 9, row (f), and profiles/r01/solver_v11.txt."""
@@ -34,28 +38,35 @@ def periodic_step_phases(step_length: np.ndarray, horizon_time: float, foot_y: f
     """main_periodic_step.py:365-412 with a step length per instance (the reference uses 0.6 for ergoCub)."""
     L = np.asarray(step_length, dtype=np.float64).reshape(-1)
     B = L.shape[0]
-    ident = np.array([0.0, 0.0, 0.0, 1.0])
 
     def pos(x, y, z):
         return np.stack([x, np.full(B, y), np.full(B, z)], axis=1)
+
+    return _left_then_right(pos(0 * L, foot_y, 0.0), pos(L / 2, foot_y, swing_height), pos(L, foot_y, 0.0),
+                            pos(L / 2, -foot_y, 0.0), pos(L, -foot_y, swing_height), pos(1.5 * L, -foot_y, 0.0),
+                            horizon_time, force_z)
+
+
+def _left_then_right(l0, l_mid, l1, r0, r_mid, r1, T, force_z):
+    """Two contact phases per foot, (B, 3) positions, identity rotations: the left foot swings from l0 over l_mid to
+    l1 in (T/6, T/3), then the right foot from r0 over r_mid to r1 in (2T/3, 5T/6) (main_periodic_step.py:365-412)."""
+    ident = np.array([0.0, 0.0, 0.0, 1.0])
 
     def phase(p, mid, act, dea):
         return FootContactPhaseDescriptor(position=p, quaternion_xyzw=ident, mid_swing_position=mid,
                                           mid_swing_quaternion_xyzw=None if mid is None else ident,
                                           force=np.array([0.0, 0.0, force_z]), activation_time=act, deactivation_time=dea)
 
-    T = horizon_time
     return FeetContactPhasesDescriptor(
-        left=[phase(pos(0 * L, foot_y, 0.0), pos(L / 2, foot_y, swing_height), None, T / 6.0),
-              phase(pos(L, foot_y, 0.0), None, T / 3.0, None)],
-        right=[phase(pos(L / 2, -foot_y, 0.0), pos(L, -foot_y, swing_height), None, T * 2.0 / 3.0),
-               phase(pos(1.5 * L, -foot_y, 0.0), None, T * 5.0 / 6.0, None)])
+        left=[phase(l0, l_mid, None, T / 6.0), phase(l1, None, T / 3.0, None)],
+        right=[phase(r0, r_mid, None, T * 2.0 / 3.0), phase(r1, None, T * 5.0 / 6.0, None)])
 
 
 def pose_problem(lay, model, left_position: np.ndarray, right_position: np.ndarray, com_height: float = 0.7):
-    """Pose-finder references of compute_state (main_periodic_step.py:192-258) for feet flat on the ground at the
-    given positions (identity rotations): contact points from the foot transforms, CoM above the middle of the
-    feet, identity base / frame quaternions, the desired joint configuration.  Returns (x guess, p)."""
+    """Pose-finder references of compute_state (main_periodic_step.py:192-258) for feet flat at the given positions
+    (identity rotations): contact points from the foot transforms, CoM com_height above the middle of the feet,
+    identity base / frame quaternions, the desired joint configuration.  Returns (x guess, p); on the smooth-step
+    terrain the caller fills the terrain parameters."""
     po = lay.po
     B = left_position.shape[0]
     p = np.zeros((B, lay.n_p))
@@ -70,7 +81,7 @@ def pose_problem(lay, model, left_position: np.ndarray, right_position: np.ndarr
         p[:, o + 5] = 9.80665 / 8.0
         p[:, o + 6:o + 9] = FOOT_CORNERS[i % 4]
     com = (left_position + right_position) / 2.0
-    com[:, 2] = com_height
+    com[:, 2] += com_height
     p[:, po.ref + po.ST_PB:po.ref + po.ST_PB + 3] = com + [0.0, 0.0, 0.05]
     p[:, po.ref + po.ST_Q + 3] = 1.0
     p[:, po.ref + po.ST_S:po.ref + po.ST_S + NJ] = np.deg2rad(DESIRED_JOINTS_DEG)
@@ -111,17 +122,31 @@ def periodic_step_guess(model, pose_evaluator, kino_evaluator, step_length: np.n
     from `set_initial_guess`): mass_normalised=True does the same, so that force_z = 100 IS the reference's guess."""
     if mass_normalised:
         force_z = force_z / float(model.total_mass())
+    L = np.asarray(step_length, dtype=np.float64).reshape(-1)
+    phases = periodic_step_phases(L, kino_evaluator.layout.N * STEP_DT, force_z=force_z)
+    centroid = np.stack([L / 2.0, np.zeros_like(L), np.zeros_like(L)], axis=1)  # 0.3 for the reference's 0.6 m step
+    return _keyframe_plan(model, pose_evaluator, kino_evaluator, phases, centroid, None, tol, max_iter)
+
+
+STEP_DT = 0.1
+
+
+def _keyframe_plan(model, pose_evaluator, kino_evaluator, phases, centroid, terrain, tol, max_iter) -> PeriodicStepGuess:
+    """The part periodic_step_guess and stairs_step_guess share: the initial / middle / final keyframe poses at the
+    phases' contact positions as one pose-finder batch, the interpolated guess, and the kinodynamic parameters
+    (initial / final states and the references of get_references with the contact centroid ``centroid`` (B, 3)).
+    ``terrain``: (B, n) terrain parameters of both problems, or None on the planar terrain."""
     lay, pl = kino_evaluator.layout, pose_evaluator.layout
     N, po = lay.N, lay.po
-    L = np.asarray(step_length, dtype=np.float64).reshape(-1)
-    B = L.shape[0]
+    B = centroid.shape[0]
     dev = torch.device("cuda", torch.cuda.current_device())
-    dt = 0.1
-    phases = periodic_step_phases(L, N * dt, force_z=force_z)
+    dt = STEP_DT
     # keyframes: (left phase, right phase) of compute_initial_state / compute_middle_state / compute_final_state
     lp = np.concatenate([phases.left[0].position, phases.left[1].position, phases.left[1].position])
     rp = np.concatenate([phases.right[0].position, phases.right[0].position, phases.right[1].position])
     xq, pq = pose_problem(pl, model, lp, rp)
+    if terrain is not None:
+        pq[:, pl.po.terrain:pl.po.terrain + terrain.shape[1]] = np.tile(terrain, (3, 1))
     lb, ub = pose_evaluator.bounds(pq)
     out = BatchedInteriorPoint(pose_evaluator, tol=tol, max_iter=max_iter).solve(
         torch.tensor(xq, device=dev), torch.tensor(pq, device=dev), lb, ub)  # OptiFailure if no keyframe pose converges at all
@@ -136,6 +161,8 @@ def periodic_step_guess(model, pose_evaluator, kino_evaluator, step_length: np.n
     guess = torch.cat([first, second], dim=1).cpu().numpy()  # (B, N, 105): the joint references below
 
     p = kino_parameters(lay, model, B, np.random.default_rng(0), spread=0.0)
+    if terrain is not None:
+        p[:, po.terrain:po.terrain + terrain.shape[1]] = terrain
     k0, k2 = key[0].cpu().numpy(), key[2].cpu().numpy()
     n_state = po.ST_COM + 3
     p[:, po.init:po.init + n_state] = k0
@@ -143,8 +170,7 @@ def periodic_step_guess(model, pose_evaluator, kino_evaluator, step_length: np.n
     for k in range(N):
         r = po.refs0 + 55 * k  # get_references, main_periodic_step.py:330-352
         p[:, r + po.R_CW:r + po.R_CW + 3] = [100.0, 100.0, 10.0]
-        p[:, r + po.R_CC] = L / 2.0  # 0.3 for the reference's 0.6 m step
-        p[:, r + po.R_CC + 1:r + po.R_CC + 3] = 0.0
+        p[:, r + po.R_CC:r + po.R_CC + 3] = centroid
         p[:, r + po.R_COMV:r + po.R_COMV + 3] = [0.1, 0.0, 0.0]
         p[:, r + po.R_YAW_L] = p[:, r + po.R_YAW_R] = 0.0
         p[:, r + po.R_FQ:r + po.R_FQ + 4] = [0.0, 0.0, 0.0, 1.0]
@@ -152,6 +178,54 @@ def periodic_step_guess(model, pose_evaluator, kino_evaluator, step_length: np.n
         p[:, r + po.R_BQV:r + po.R_BQV + 4] = 0.0
         p[:, r + po.R_JR:r + po.R_JR + NJ] = guess[:, k, 79:79 + NJ]
     return PeriodicStepGuess(parameters=p, x0=x0, ok=ok, keyframes=key, pose_iterations=out.iterations)
+
+
+# the stairs of workloads.kino_parameters (main_walking_on_stairs.py:18-28, 397-403): two smooth steps, the first tread
+# at height h for x in (0.225, 0.6975), the second at 2 h beyond; each edge's transition band is about 2 cm wide
+def stairs_terrain(step_height: np.ndarray) -> np.ndarray:
+    """(B, 10) terrain parameters (l, w, height, ox, oy) x 2 of the stairs with the step height h per instance."""
+    h = np.asarray(step_height, dtype=np.float64).reshape(-1)
+    L = 0.45
+    tp = np.tile([2 * L, 0.8, 0.0, 1.5 * L, 0.0, 0.9 * L, 0.8, 0.0, 2 * L, 0.0], (h.shape[0], 1))
+    tp[:, 2] = tp[:, 7] = h
+    return tp
+
+
+def stairs_step_guess(model, pose_evaluator, kino_evaluator, step_height: np.ndarray, tol: float = 1e-8,
+                      max_iter: int = 300, force_z: float = 100.0, mass_normalised: bool = False,
+                      start_x: float = 0.0, tread_x: float = 0.45, foot_y: float = 0.1,
+                      swing_height: float = 0.05) -> PeriodicStepGuess:
+    """BASELINE config 5 (walking on stairs, N = 50, dt = 0.1): the batched counterpart of periodic_step_guess on the
+    stairs of `stairs_terrain`, with the step height h per instance.  The robot starts with both feet on the ground
+    centred at x = start_x (every foot corner, +-0.116 m, clear of the first edge's transition band), steps with the
+    left foot onto the first tread (centred at x = tread_x, clear of both of its edges), then with the right foot.
+
+    * keyframes: initial (both feet on the ground), middle (left foot on the first tread), final (both feet on the first
+      tread), three pose-finder solves per instance as ONE batch of 3 B on the smooth-terrain pose evaluator;
+    * point references and contact phases: the z of every point is the height of the tread it lands on, the mid-swing
+      height is the higher tread plus swing_height;
+    * guess and references as periodic_step_guess (interpolation over both halves, get_references with the contact
+      centroid halfway between start and tread, at half the step height).
+
+    UNPINNED: the reference's stairs main (main_walking_on_stairs.py) is available here only through the lines SURVEY.md
+    cites (terrain, horizon and solver options); this keyframe placement is this project's own, not a restatement."""
+    if mass_normalised:
+        force_z = force_z / float(model.total_mass())
+    h = np.asarray(step_height, dtype=np.float64).reshape(-1)
+    B = h.shape[0]
+    if pose_evaluator.layout.st.terrain != "smooth_steps" or kino_evaluator.layout.st.terrain != "smooth_steps":
+        raise ValueError("stairs_step_guess: both evaluators must be posed on the smooth steps")
+
+    def pos(x, y, z):
+        return np.stack([np.full(B, x), np.full(B, y), z], axis=1)
+
+    zero = np.zeros(B)
+    mid_x = 0.5 * (start_x + tread_x)
+    phases = _left_then_right(pos(start_x, foot_y, zero), pos(mid_x, foot_y, h + swing_height), pos(tread_x, foot_y, h),
+                              pos(start_x, -foot_y, zero), pos(mid_x, -foot_y, h + swing_height),
+                              pos(tread_x, -foot_y, h), kino_evaluator.layout.N * STEP_DT, force_z)
+    centroid = pos(mid_x, 0.0, 0.5 * h)
+    return _keyframe_plan(model, pose_evaluator, kino_evaluator, phases, centroid, stairs_terrain(h), tol, max_iter)
 
 
 def single_step_problem(model, pose_evaluator, kino_evaluator, step_length: np.ndarray, tol: float = 1e-8,

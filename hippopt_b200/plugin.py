@@ -204,11 +204,13 @@ class TemplateMatch:
 
 def match_template(nx: int, np_: int, ng: int) -> TemplateMatch | None:
     """Dimensions of the baked Opti problem -> the template they belong to (SURVEY.md Appendix B), or None.
-    kinodynamic: n_x = 189 N + 6, n_p = 79 N + 326 (+ terrain parameters), m from the constraint families."""
+    kinodynamic: n_x = 189 N + 6, n_p = 79 N + 326 (+ terrain parameters), m from the constraint families.
+    pose finder: (81, 202, 89), or (81, 212, 89) on the smooth steps, whose ten parameters are appended to p."""
     from .kino_layout import NZ, count_rows
 
-    if nx == 81 and np_ == 202 and ng == 89:   # pose finder, Appendix B.4
-        return TemplateMatch("pose_finder")
+    if nx == 81 and np_ in (202, 212) and ng == 89:   # pose finder, Appendix B.4
+        n_terr = np_ - 202
+        return TemplateMatch("pose_finder", smooth_terrain=n_terr > 0, n_terrain_params=n_terr)
     if nx % 9 == 0 and np_ == 3 and ng in (7 * (nx // 9) + 3, 7 * (nx // 9) + 2):  # toy OCP: 9 N variables
         return TemplateMatch("toy", horizon=nx // 9)
     if nx > 6 and (nx - 6) % NZ == 0:
@@ -603,7 +605,11 @@ def make_opti_solver(cs, hp, evaluator_factory=None):
                                          n_terrain_params=match.n_terrain_params)
                 ev = KinoEvaluator(self.robot_model, st)
             elif match.kind == "pose_finder":
-                ev = PoseEvaluator(self.robot_model)
+                from .pose_layout import PoseSettings
+
+                ev = PoseEvaluator(self.robot_model, PoseSettings(
+                    terrain="smooth_steps" if match.smooth_terrain else "planar",
+                    n_terrain_params=match.n_terrain_params))
             else:
                 raise TemplateMismatch("toy OCP: construct ToyEvaluator with the problem's dt explicitly")
             host = HostEvaluator(ev)

@@ -2,8 +2,10 @@
 
 Static-pose NLP of `/root/reference/src/hippopt/turnkey_planners/humanoid_pose_finder/planner.py:
 303-413, 444-788` with the defaults of `planner.py:79-92` (CoM / point positions as costs, hands
-skipped, PlanarTerrain): x (81), p (202), g (89) orderings of SURVEY.md Appendix B.4 and the CCS
-patterns of jac_g / upper-triangular hess_l.
+skipped): x (81), p (202), g (89) orderings of SURVEY.md Appendix B.4 and the CCS patterns of jac_g /
+upper-triangular hess_l.  PlanarTerrain by default; ``terrain="smooth_steps"`` poses the same problem on
+the two smooth steps of the stairs (BASELINE config 5) with their ten parameters (l, w, height, ox, oy) x 2
+appended to p (p = 212), as the kinodynamic layout does.
 
 The device kernels work on a *virtual knot* in the kinodynamic 189-variable layout
 (`kino_layout`): ``zmap[i]`` is the x offset of virtual variable i or -1.  The kinematics kernel keeps
@@ -26,6 +28,8 @@ XPB, XQ, XS, XCOM, NX = 48, 51, 55, 78, 81
 class PoseSettings:
     """`humanoid_pose_finder/main.py:75-98`."""
 
+    terrain: str = "planar"  # "planar" | "smooth_steps"
+    n_terrain_params: int = 0
     foot_frames: tuple = ("l_sole", "r_sole")
     frame_quaternion_cost_frame: str = "chest"
     joint_regularization_cost_weights: np.ndarray = dataclasses.field(
@@ -41,7 +45,7 @@ class PoseSettings:
 
 
 class PoseParamOffsets:
-    def __init__(self):
+    def __init__(self, n_terrain: int = 0):
         o = 0
         self.desc0 = o
         o += 24
@@ -61,6 +65,8 @@ class PoseParamOffsets:
         o += 2 * NJ
         self.lhand_in_frame, self.rhand_in_frame = o, o + 3
         o += 6
+        self.terrain = o
+        o += n_terrain
         self.n_p = o
 
     ST_PB, ST_Q, ST_S, ST_COM = 72, 75, 79, 102
@@ -72,7 +78,12 @@ class PoseLayout:
         self.st = settings or PoseSettings()
         self.N = 1
         self.n_x = NX
-        self.po = PoseParamOffsets()
+        if self.st.terrain not in ("planar", "smooth_steps"):
+            raise ValueError(f"terrain must be 'planar' or 'smooth_steps', not {self.st.terrain!r}")
+        self.smooth = self.st.terrain != "planar"
+        if self.st.n_terrain_params != (10 if self.smooth else 0):
+            raise ValueError("the smooth steps take 10 terrain parameters, the planar terrain none")
+        self.po = PoseParamOffsets(self.st.n_terrain_params)
         self.n_p = self.po.n_p
         zmap = -np.ones(NZ, dtype=np.int32)
         for i in range(NPT):
@@ -119,17 +130,30 @@ class PoseLayout:
 
     # ------------------------------------------------------------------ local orders
     def _enumerate_jp(self):
-        """Pose contact kernel: (row, x column) per local Jacobian entry."""
+        """Pose contact kernel: (row, x column) per local Jacobian entry.  Per point 13 entries on the planar
+        terrain, 25 on the smooth steps, where h = z - T(x, y) and n, R_t depend on (x, y) only."""
         e = []
         z = self.zmap
         for i in range(NPT):
             o = 15 * i
-            e.append((self.row(f"pt{i}.complementarity"), z[o + P + 2]))
-            e.append((self.row(f"pt{i}.complementarity"), z[o + F + 2]))
-            e.append((self.row(f"pt{i}.height"), z[o + P + 2]))
-            e.append((self.row(f"pt{i}.normal"), z[o + F + 2]))
-            for c in range(3):
-                e.append((self.row(f"pt{i}.friction"), z[o + F + c]))
+            if not self.smooth:
+                e.append((self.row(f"pt{i}.complementarity"), z[o + P + 2]))
+                e.append((self.row(f"pt{i}.complementarity"), z[o + F + 2]))
+                e.append((self.row(f"pt{i}.height"), z[o + P + 2]))
+                e.append((self.row(f"pt{i}.normal"), z[o + F + 2]))
+                for c in range(3):
+                    e.append((self.row(f"pt{i}.friction"), z[o + F + c]))
+            else:
+                for blk in (P, F):
+                    for d in range(3):
+                        e.append((self.row(f"pt{i}.complementarity"), z[o + blk + d]))
+                for d in range(3):
+                    e.append((self.row(f"pt{i}.height"), z[o + P + d]))
+                for name in ("normal", "friction"):
+                    for d in range(2):
+                        e.append((self.row(f"pt{i}.{name}"), z[o + P + d]))
+                    for d in range(3):
+                        e.append((self.row(f"pt{i}.{name}"), z[o + F + d]))
             for c in range(3):
                 e.append((self.row(f"pt{i}.fk", c), z[o + P + c]))
             for c in range(3):
@@ -184,6 +208,13 @@ class PoseLayout:
         for i in range(NPT):
             o = 15 * i
             add(o + P + 2, o + F + 2)  # relaxed complementarity
+            if self.smooth:
+                # h(p) n(p).f, n.f and (R_t(p)^T f)^2: every (p, p), (p, f) and (f, f) pair of the point
+                for a in range(3):
+                    for b in range(3):
+                        add(o + P + a, o + P + b)
+                        add(o + P + a, o + F + b)
+                        add(o + F + a, o + F + b)
             for c in range(3):
                 add(o + P + c, o + P + c)  # point position regularisation
                 add(o + F + c, o + F + c)  # friction, force regularisation, average force

@@ -56,7 +56,8 @@ enum {
   HB_KI_N_JC,
   HB_KI_N_JK,
   HB_KI_N_HC,
-  HB_KI_TERRAIN,          /* 0 planar (planar_terrain.py), 1 sum of two smooth steps */
+  HB_KI_TERRAIN,          /* 0 planar (planar_terrain.py), 1 sum of two smooth steps (the stairs); both for either
+                             kind, the steps' ten parameters (l, w, height, ox, oy) x 2 at HB_KI_PO_TERRAIN in p */
   HB_KI_HAS_FINAL,
   HB_KI_HAS_PERIODICITY,
   HB_KI_H_INIT,           /* x offset of initial_state.centroidal_momentum */
