@@ -126,12 +126,9 @@ static cudaError_t ensure_kernel_attributes(int dev) {
   if ((e = cudaFuncSetAttribute(hb::lu_factor_kernel<3, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, lu_big)) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(hb::lu_factor_kernel<1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, lu_big)) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(hb::lu_factor_kernel<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, lu_big)) != cudaSuccess) return e;
-  if ((e = cudaFuncSetAttribute(hb::lu_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, lu_big)) != cudaSuccess) return e;
   const int lu_staged = 232448 - 1024 - 2560;
   if ((e = cudaFuncSetAttribute(hb::lu_solve_staged_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, lu_staged)) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(hb::lu_solve_staged_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, lu_staged)) != cudaSuccess) return e;
-  if ((e = cudaFuncSetAttribute(hb::lu_solve_staged_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, lu_staged)) != cudaSuccess) return e;
-  if ((e = cudaFuncSetAttribute(hb::lu_solve_staged_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, lu_staged)) != cudaSuccess) return e;
   if ((e = cudaDeviceGetAttribute(&device_sms[dev], cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
   done[dev] = true;
   return cudaSuccess;
@@ -761,8 +758,7 @@ extern "C" int hb_eval(hb_handle h, uint32_t mask, const double* x, const double
   int dev_now = 0;
   CUDA_TRY(cudaGetDevice(&dev_now));
   CUDA_TRY(ensure_kernel_attributes(dev_now));
-  static const bool no_overlap_env = getenv("HB_NO_SMALL_BATCH_OVERLAP") != nullptr;
-  const bool overlap = !h->prof && !no_overlap_env && C.kind == 0 && total_warps <= 8L * device_sms[dev_now];
+  const bool overlap = !h->prof && C.kind == 0 && total_warps <= 8L * device_sms[dev_now];
   cudaStream_t st_contact = st;
   if (overlap) {
     if (!h->aux) {
@@ -775,11 +771,6 @@ extern "C" int hb_eval(hb_handle h, uint32_t mask, const double* x, const double
     st_contact = h->aux;
   }
   {
-    {
-      int dev = 0;
-      CUDA_TRY(cudaGetDevice(&dev));
-      CUDA_TRY(ensure_kernel_attributes(dev));
-    }
     const size_t smem = (size_t)(C.kind == 1 ? hb::pose_contact_smem_layout(C.n_hc) : hb::kino_contact_smem_layout(C.n_hc)).total *
                         sizeof(double) * warps_per_block;
     // the shared block holds the kernel's n_hc Hessian accumulators (191 planar, 255 on the smooth steps)
@@ -959,9 +950,8 @@ extern "C" int hb_eval_host(hb_handle h, uint32_t mask, const double* x, const d
     return HB_OK;
   };
   // ---- graph replay of repeating single-chunk calls
-  static const bool no_graph = getenv("HB_NO_HOST_GRAPH") != nullptr;  // A/B timing
   hb_problem_s::HostGraph* hg = nullptr;
-  if (!no_graph && n_chunks == 1 && !h->prof) {
+  if (n_chunks == 1 && !h->prof) {
     const void* key[8] = {x, lam_g, sigma, f, grad_f, g, jac_vals, hess_vals};
     for (auto& e : h->hgraphs)
       if (e.mask == mask && e.batch == batch && std::equal(key, key + 8, e.ptr)) hg = &e;
@@ -1049,42 +1039,32 @@ extern "C" int hb_host_free(void* ptr) {
 //   rpt, mb   lu_factor_kernel<RPT, MB>: panel rows per thread (n <= RPT * LU_THREADS) and CTAs per SM the register
 //             allocation is tuned for -- the 128-register MB = 2 build when the batch exceeds one CTA per SM and two
 //             CTAs fit an SM's shared memory
-//   ct        lu_solve_staged_kernel<CT> (8-column tiles of right-hand sides per CTA), 0 = the unstaged lu_solve_kernel
+//   ct        lu_solve_staged_kernel<CT>: 8-column tiles of right-hand sides per CTA, 4 or 3
 //   chunks    column chunks (CTAs) per matrix of the solve
 struct LuPlan {
   int rpt, mb, ct, chunks;
 };
-static LuPlan lu_plan(int64_t n, int64_t batch, int64_t nrhs, int sms, bool unstaged) {
+static LuPlan lu_plan(int64_t n, int64_t batch, int64_t nrhs, int sms) {
   LuPlan p{};
   const size_t smem = hb::lu_factor_smem((int)n);
   const bool two = batch > sms && 2 * (smem + 2048) <= 227 * 1024;
   p.rpt = n <= hb::LU_THREADS ? 1 : n <= 2 * hb::LU_THREADS ? 2 : 3;
   p.mb = two && p.rpt < 3 ? 2 : 1;
-  // staged substitution (lu.cu): 32 or 24 right-hand sides per CTA while two CTAs fit an SM, else 32 / 24 / 16 / 8 on
-  // one CTA per SM
+  // staged substitution (lu.cu): 32 or 24 right-hand sides per CTA while two CTAs fit an SM, else on one CTA per SM
+  // (lu_staged_smem(768, 3) = 196 112 B fits one)
   const size_t two_per_sm = (233472 / 2) - 1024 - 2560, one_per_sm = 232448 - 1024 - 2560;  // minus the static arrays
-  p.ct = 0;  // 8-column tiles per CTA
-  if (!unstaged) {
-    if (hb::lu_staged_smem((int)n, 4) <= two_per_sm) p.ct = 4;
-    else if (hb::lu_staged_smem((int)n, 3) <= two_per_sm) p.ct = 3;
-    else if (hb::lu_staged_smem((int)n, 4) <= one_per_sm) p.ct = 4;
-    else if (hb::lu_staged_smem((int)n, 3) <= one_per_sm) p.ct = 3;
-    else if (hb::lu_staged_smem((int)n, 2) <= one_per_sm) p.ct = 2;
-    else if (hb::lu_staged_smem((int)n, 1) <= one_per_sm) p.ct = 1;
-  }
-  const int64_t rc = p.ct > 0 ? 8 * p.ct : hb::LU_RC;
-  p.chunks = (int)((nrhs + rc - 1) / rc);
+  if (hb::lu_staged_smem((int)n, 4) <= two_per_sm) p.ct = 4;
+  else if (hb::lu_staged_smem((int)n, 3) <= two_per_sm) p.ct = 3;
+  else if (hb::lu_staged_smem((int)n, 4) <= one_per_sm) p.ct = 4;
+  else p.ct = 3;
+  p.chunks = (int)((nrhs + 8 * p.ct - 1) / (8 * p.ct));
   return p;
-}
-static bool lu_solve_unstaged() {
-  static const bool unstaged = getenv("HB_LU_SOLVE_UNSTAGED") != nullptr;  // A/B timing against the round-1 kernel
-  return unstaged;
 }
 
 extern "C" int hb_debug_lu_plan(int64_t n, int64_t batch, int64_t nrhs, int32_t sms, int32_t* out) {
   if (!out || n <= 0 || n > 768 || batch <= 0 || nrhs <= 0 || sms <= 0)
     return fail(HB_ERR_INVALID, "hb_debug_lu_plan: need 0 < n <= 768, batch > 0, nrhs > 0, sms > 0, out");
-  const LuPlan p = lu_plan(n, batch, nrhs, sms, lu_solve_unstaged());
+  const LuPlan p = lu_plan(n, batch, nrhs, sms);
   out[0] = p.rpt;
   out[1] = p.mb;
   out[2] = p.ct;
@@ -1128,7 +1108,7 @@ extern "C" int hb_lu_factor_batched(double* A, int32_t* piv, int32_t* info, int6
   int dev = 0;
   CUDA_TRY(cudaGetDevice(&dev));
   CUDA_TRY(ensure_kernel_attributes(dev));
-  const LuPlan p = lu_plan(n, batch, 1, device_sms[dev], lu_solve_unstaged());  // (the solve fields are not used here)
+  const LuPlan p = lu_plan(n, batch, 1, device_sms[dev]);  // (the solve fields are not used here)
   cudaStream_t st = (cudaStream_t)stream;
   const unsigned grid = (unsigned)batch;
   if (p.rpt == 1 && p.mb == 2) hb::lu_factor_kernel<1, 2><<<grid, hb::LU_THREADS, smem, st>>>(A, piv, info, (int)n);
@@ -1148,21 +1128,12 @@ extern "C" int hb_lu_solve_batched(const double* LU, const int32_t* piv, double*
   int dev = 0;
   CUDA_TRY(cudaGetDevice(&dev));
   CUDA_TRY(ensure_kernel_attributes(dev));
-  const LuPlan p = lu_plan(n, batch, nrhs, device_sms[dev], lu_solve_unstaged());
-  if (p.ct > 0) {
-    const size_t smem = hb::lu_staged_smem((int)n, p.ct);
-    const int n_chunks = p.chunks;
-    const unsigned grid = (unsigned)(batch * n_chunks);
-    if (p.ct == 4) hb::lu_solve_staged_kernel<4><<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs, n_chunks);
-    else if (p.ct == 3) hb::lu_solve_staged_kernel<3><<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs, n_chunks);
-    else if (p.ct == 2) hb::lu_solve_staged_kernel<2><<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs, n_chunks);
-    else hb::lu_solve_staged_kernel<1><<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs, n_chunks);
-    CUDA_TRY(cudaGetLastError());
-    return HB_OK;
-  }
-  const size_t smem = (size_t)n * (hb::LU_RC + 1) * sizeof(double);
-  const dim3 grid((unsigned)batch, (unsigned)p.chunks);
-  hb::lu_solve_kernel<<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs);
+  const LuPlan p = lu_plan(n, batch, nrhs, device_sms[dev]);
+  const size_t smem = hb::lu_staged_smem((int)n, p.ct);
+  const int n_chunks = p.chunks;
+  const unsigned grid = (unsigned)(batch * n_chunks);
+  if (p.ct == 4) hb::lu_solve_staged_kernel<4><<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs, n_chunks);
+  else hb::lu_solve_staged_kernel<3><<<grid, hb::LU_THREADS, smem, (cudaStream_t)stream>>>(LU, piv, Bm, (int)n, (int)nrhs, n_chunks);
   CUDA_TRY(cudaGetLastError());
   return HB_OK;
 }

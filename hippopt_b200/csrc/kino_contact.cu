@@ -115,9 +115,7 @@ __device__ __forceinline__ void linear_state(int j, int& so, int& ro, int& fam_d
 // CTAs per SM of the planar kernel, kernel time per bench step (config 3, NVIDIA B200 at 1000 W, 1965 MHz, three
 // alternated runs): 5 (96 registers, no spill) 0.241 ms, 6 (80, 12 B spill) 0.224 ms, 7 (72, 8 B spill) 0.213 ms.
 // Shared memory allows 7: 30 976 B per CTA.
-#ifndef CONTACT_MIN_BLOCKS
-#define CONTACT_MIN_BLOCKS 7
-#endif
+constexpr int CONTACT_MIN_BLOCKS = 7;
 template <int TERRAIN>
 __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) kino_contact_kernel(const __grid_constant__ KinTopo T,
                                                            const KinoConst* __restrict__ Cp, unsigned mask,

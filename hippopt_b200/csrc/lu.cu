@@ -11,8 +11,10 @@
 //     t+512): two barriers per column (pivot search, pivot-row exchange);
 //   * applies the panel's 16 interchanges to a trailing column as ONE gather (the composed permutation
 //     touches <= 32 rows), then U12 = L11^{-1} A12 in registers;
-//   * updates the trailing matrix A22 -= L21 U12 from shared memory with 4x4 register tiles, the A22
-//     tile being requested before the products so that its L2 latency overlaps them.
+//   * updates the trailing matrix A22 -= L21 U12 on the fp64 tensor cores (mma.sync m8n8k4), L21 and U12
+//     from shared memory, the A22 fragments read and written in place in global memory.
+// The substitution (lu_solve_staged_kernel) stages half panels of the factor in shared memory with
+// cp.async beside the triangular solve and updates the other rows with the same MMAs.
 //
 // Storage: column-major n x n, leading dimension n (a symmetric matrix can be passed as is).
 // Pivoting: rows are interchanged inside the panel and in the trailing columns, NOT in the columns to
@@ -25,22 +27,8 @@
 namespace hb {
 
 constexpr int LU_NB = 16;
-// Measured on B200, 148 blocks of 337^2 (one wave): 256 threads + A22 prefetch 0.98 ms; 256 threads without
-// prefetch 1.98 ms; 512 threads (128 registers, spills) 1.22 ms with / 1.58 ms without prefetch.
-#ifndef HB_LU_THREADS
-#define HB_LU_THREADS 256
-#endif
-#ifndef HB_LU_PREFETCH
-#define HB_LU_PREFETCH 1  // request the A22 tile before the products: its L2 latency overlaps them
-#endif
-#ifndef HB_LU_DMMA
-#define HB_LU_DMMA 1  // trailing update with mma.sync.m8n8k4.f64 instead of 4 x 4 register tiles of FMAs
-#endif
-#ifndef HB_LU_TR
-#define HB_LU_TR 4  // rows of the trailing-update register tile when one CTA runs per SM (4 or 8)
-#endif
-constexpr int LU_THREADS = HB_LU_THREADS;
-constexpr int LU_MAXN = 768;
+// B200, 148 blocks of 337^2 (one wave): 256 threads 0.98 ms, 512 threads (128 registers, spills) 1.22 ms
+constexpr int LU_THREADS = 256;
 
 __host__ __device__ inline int lu_ldp(int n) { return (n + 3) & ~3; }
 // dynamic shared memory of the factor kernel: panel + U strip (+ slack: the last vector loads of a tile may
@@ -227,16 +215,13 @@ __global__ void __launch_bounds__(LU_THREADS, MB) lu_factor_kernel(double* __res
         }
     }
     __syncthreads();
-    // ---- trailing update A22 -= L21 U12: CTA tile 128 rows x 32 columns, thread tile 4 x 4 (rows strided
-    // by 32 so that every A22 access is a coalesced 256-byte row segment; contiguous rows per thread were
-    // 20 % slower); per k four shared loads of L21 and two 16-byte broadcast loads of U12 feed 16 FMAs
-#ifndef HB_LU_SKIP_TRAILING  // (timing experiments only: how much of a factorisation is the panel work)
-#if HB_LU_DMMA
+    // ---- trailing update A22 -= L21 U12 on the fp64 tensor cores: warp tile 32 rows x 16 columns = 4 x 2 m8n8k4
+    // accumulators, A fragments from L21 (negated), B fragments from the U strip, C fragments read from / written to
+    // A22 in place (a fragment's 8 rows of one column are 64 contiguous bytes), requested before the products so that
+    // their L2 latency overlaps them (with FMA tiles: 0.98 ms vs 1.98 ms without).  32 MMAs per 24 shared-memory
+    // loads against 16 multiply-adds per 6 loads in 4 x 4 FMA register tiles; same time (1.44 ms per 296 blocks of
+    // 337^2: the update streams A22), fewer issue slots.
     {
-      // Trailing update on the fp64 tensor cores (round 2): warp tile 32 rows x 16 columns = 4 x 2 m8n8k4 accumulators,
-      // A fragments from L21 (negated), B fragments from the U strip, C fragments read from / written to A22 in place
-      // (a fragment's 8 rows of one column are 64 contiguous bytes).  32 MMAs per 24 shared-memory loads, where the
-      // 4 x 4 register tiles issued 16 multiply-adds per 6 loads.
       const int lane = tid & 31, w = tid >> 5, g = lane >> 2, t4 = lane & 3;
       const double* L21 = P + nbw;  // local row i of L21 = panel row nbw + i
       double* A22 = A + (size_t)(j0 + nbw) * n + j0 + nbw;
@@ -280,230 +265,21 @@ __global__ void __launch_bounds__(LU_THREADS, MB) lu_factor_kernel(double* __res
           }
       }
     }
-#else
-    {
-      constexpr int TR = MB == 1 ? HB_LU_TR : 4;  // rows per thread tile: TR x 4, CTA tile 32 TR rows x 32 columns
-      const int tx = tid & 31, ty = tid >> 5;
-      const double* L21 = P + nbw;  // local row i of L21 = panel row nbw + i
-      for (int jt = 0; jt < nrem; jt += (nt / 32) * 4)
-        for (int it = 0; it < nrem; it += 32 * TR) {
-          double acc[TR][4];
-#if HB_LU_PREFETCH
-          double a22[TR][4];
-#endif
-          int ii[TR], jc[4];
-#pragma unroll
-          for (int a = 0; a < TR; ++a) ii[a] = it + tx + 32 * a;  // lane = row: coalesced A22 accesses
-#pragma unroll
-          for (int b = 0; b < 4; ++b) jc[b] = jt + ty * 4 + b;
-#pragma unroll
-          for (int b = 0; b < 4; ++b) {
-            const double* col = A + (size_t)(j0 + nbw + jc[b]) * n + j0 + nbw;
-#pragma unroll
-            for (int a = 0; a < TR; ++a) {
-#if HB_LU_PREFETCH
-              a22[a][b] = (jc[b] < nrem && ii[a] < nrem) ? col[ii[a]] : 0.0;
-#else
-              (void)col;
-#endif
-              acc[a][b] = 0.0;
-            }
-          }
-#pragma unroll 4
-          for (int k = 0; k < nbw; ++k) {
-            // entries past nrem are whatever the panel / strip hold (the reads stay inside the shared-memory
-            // block: 15 ldp + nbw + nrem + 32 TR - 1 < 32 ldp); the products they feed are never stored
-            const double* lp = L21 + k * ldp + it + tx;
-            const double2* up = reinterpret_cast<const double2*>(U + k * ldp + jt + ty * 4);
-            const double2 u01 = up[0], u23 = up[1];
-            const double uu[4] = {u01.x, u01.y, u23.x, u23.y};
-            double l[TR];
-#pragma unroll
-            for (int a = 0; a < TR; ++a) l[a] = lp[32 * a];
-#pragma unroll
-            for (int a = 0; a < TR; ++a)
-#pragma unroll
-              for (int b = 0; b < 4; ++b) acc[a][b] = fma(l[a], uu[b], acc[a][b]);
-          }
-#pragma unroll
-          for (int b = 0; b < 4; ++b)
-            if (jc[b] < nrem) {
-              double* col = A + (size_t)(j0 + nbw + jc[b]) * n + j0 + nbw;
-#pragma unroll
-              for (int a = 0; a < TR; ++a)
-#if HB_LU_PREFETCH
-                if (ii[a] < nrem) col[ii[a]] = a22[a][b] - acc[a][b];
-#else
-                if (ii[a] < nrem) col[ii[a]] -= acc[a][b];
-#endif
-            }
-        }
-    }
-#endif
-#endif
     __syncthreads();
   }
   __syncthreads();
   if (tid == 0) infoall[blockIdx.x] = s_info;
 }
 
-// Solve with the factors: B (n x nrhs, row-major, i.e. right-hand side c of row i at B[i * nrhs + c]) is
-// overwritten by the solution.  grid = (batch, ceil(nrhs / 32)); a CTA owns up to 32 right-hand sides,
-// kept in shared memory for the whole forward and backward substitution.  Rows outside the current
-// panel are updated with 4 x 8 register tiles (lane = row: coalesced reads of the factor).
-constexpr int LU_RC = 32;
-#ifndef HB_LU_KD
-// panel columns whose factor entries are requested together in the substitution sweeps.  Measured on B200,
-// 148 / 296 blocks of 337^2 with 88 right-hand sides: a load per column 1.30 / 1.95 ms; 8 columns together
-// (254 registers, 1 CTA per SM) 0.94 / 1.88 ms; 4 columns and 2 CTAs per SM (128 registers) 0.81 / 1.23 ms
-#define HB_LU_KD 4
-#endif
-constexpr int LU_KD = HB_LU_KD;
-
-__device__ __forceinline__ void lu_rows_update(const double* __restrict__ A, double* b, int n, int ldb, int j0, int nbw,
-                                               int r0, int r1, int tid) {
-  // b[i][:] -= sum_k A[i, j0 + k] * b[j0 + k][:] for rows r0 <= i < r1
-  const int lane = tid & 31, w = tid >> 5;
-  const int cg = (w & 3) * 8;  // 8 right-hand sides per warp
-  for (int ib = r0 + (w >> 2) * 128; ib < r1; ib += LU_THREADS) {  // (warps / 4) row blocks of 128
-    double acc[4][8];
-#pragma unroll
-    for (int a = 0; a < 4; ++a)
-#pragma unroll
-      for (int c = 0; c < 8; ++c) acc[a][c] = 0.0;
-    for (int k0 = 0; k0 < nbw; k0 += LU_KD) {
-      // the factor entries of 8 panel columns are requested together (32 loads in flight per thread):
-      // with a load per k the loop ran at the L2 latency
-      double av[LU_KD][4];
-#pragma unroll
-      for (int kk = 0; kk < LU_KD; ++kk)
-#pragma unroll
-        for (int a = 0; a < 4; ++a) {
-          const int i = ib + lane + 32 * a;
-          av[kk][a] = (k0 + kk < nbw && i < r1) ? A[(size_t)(j0 + k0 + kk) * n + i] : 0.0;
-        }
-#pragma unroll
-      for (int kk = 0; kk < LU_KD; ++kk) {
-        const double* bk = b + (j0 + min(k0 + kk, nbw - 1)) * ldb + cg;  // av is zero past the panel
-#pragma unroll
-        for (int c = 0; c < 8; ++c) {
-          const double bv = bk[c];
-#pragma unroll
-          for (int a = 0; a < 4; ++a) acc[a][c] = fma(av[kk][a], bv, acc[a][c]);
-        }
-      }
-    }
-#pragma unroll
-    for (int a = 0; a < 4; ++a) {
-      const int i = ib + lane + 32 * a;
-      if (i < r1)
-#pragma unroll
-        for (int c = 0; c < 8; ++c) b[i * ldb + cg + c] -= acc[a][c];
-    }
-  }
-}
-
-#ifndef HB_LU_SOLVE_MIN_BLOCKS
-#define HB_LU_SOLVE_MIN_BLOCKS 2
-#endif
-__global__ void __launch_bounds__(LU_THREADS, HB_LU_SOLVE_MIN_BLOCKS) lu_solve_kernel(const double* __restrict__ LUall,
-                                                              const int* __restrict__ pivall, double* __restrict__ Ball,
-                                                              int n, int nrhs) {
-  extern __shared__ __align__(16) double lu_sm[];
-  const double* A = LUall + (size_t)blockIdx.x * n * n;
-  const int* piv = pivall + (size_t)blockIdx.x * n;
-  double* Bg = Ball + (size_t)blockIdx.x * n * nrhs;
-  const int c0 = blockIdx.y * LU_RC;
-  const int nc = min(LU_RC, nrhs - c0);
-  const int tid = threadIdx.x;
-  constexpr int nt = LU_THREADS;
-  const int ldb = LU_RC + 1;
-  double* b = lu_sm;  // b[i * ldb + c]; columns >= nc are zero
-  __shared__ double tri[LU_NB][LU_NB + 1];  // diagonal block of the current panel, tri[k][i] = A[j0 + i, j0 + k]
-  __shared__ int s_piv[LU_NB];
-  for (int e = tid; e < n * LU_RC; e += nt) {
-    const int i = e / LU_RC, c = e - i * LU_RC;
-    b[i * ldb + c] = c < nc ? Bg[(size_t)i * nrhs + c0 + c] : 0.0;
-  }
-  // ---- forward: panel by panel -- interchanges of the panel, L11, then the rows below
-  for (int j0 = 0; j0 < n; j0 += LU_NB) {
-    const int nbw = min(LU_NB, n - j0);
-    if (tid < LU_NB * LU_NB) {
-      const int k = tid >> 4, i = tid & 15;
-      tri[k][i] = (k < nbw && i < nbw) ? A[(size_t)(j0 + k) * n + j0 + i] : 0.0;
-      if (tid < nbw) s_piv[tid] = piv[j0 + tid];
-    }
-    __syncthreads();
-    if (tid < LU_RC) {
-      for (int c = 0; c < nbw; ++c) {
-        const int r = s_piv[c];
-        if (r != j0 + c) {
-          const double t = b[(j0 + c) * ldb + tid];
-          b[(j0 + c) * ldb + tid] = b[r * ldb + tid];
-          b[r * ldb + tid] = t;
-        }
-      }
-      double y[LU_NB];
-#pragma unroll
-      for (int k = 0; k < LU_NB; ++k) y[k] = k < nbw ? b[(j0 + k) * ldb + tid] : 0.0;
-#pragma unroll
-      for (int k = 0; k < LU_NB; ++k)
-#pragma unroll
-        for (int i = k + 1; i < LU_NB; ++i) y[i] -= tri[k][i] * y[k];  // entries outside the block are zero
-#pragma unroll
-      for (int k = 0; k < LU_NB; ++k)
-        if (k < nbw) b[(j0 + k) * ldb + tid] = y[k];
-    }
-    __syncthreads();
-    lu_rows_update(A, b, n, ldb, j0, nbw, j0 + nbw, n, tid);
-    __syncthreads();
-  }
-  // ---- backward with U (panels aligned from the end; U is just upper triangular)
-  for (int j1 = n; j1 > 0; j1 -= LU_NB) {
-    const int j0 = max(0, j1 - LU_NB);
-    const int nbw = j1 - j0;
-    if (tid < LU_NB * LU_NB) {
-      const int k = tid >> 4, i = tid & 15;
-      tri[k][i] = (k < nbw && i < nbw) ? A[(size_t)(j0 + k) * n + j0 + i] : 0.0;
-    }
-    __syncthreads();
-    if (tid < LU_RC) {
-      double xv[LU_NB];
-#pragma unroll
-      for (int k = 0; k < LU_NB; ++k) xv[k] = k < nbw ? b[(j0 + k) * ldb + tid] : 0.0;
-#pragma unroll
-      for (int k = LU_NB - 1; k >= 0; --k)
-        if (k < nbw) {
-          xv[k] = xv[k] / tri[k][k];
-#pragma unroll
-          for (int i = 0; i < k; ++i) xv[i] -= tri[k][i] * xv[k];
-        }
-#pragma unroll
-      for (int k = 0; k < LU_NB; ++k)
-        if (k < nbw) b[(j0 + k) * ldb + tid] = xv[k];
-    }
-    __syncthreads();
-    lu_rows_update(A, b, n, ldb, j0, nbw, 0, j0, tid);
-    __syncthreads();
-  }
-  for (int e = tid; e < n * nc; e += nt) {
-    const int i = e / nc, c = e - i * nc;
-    Bg[(size_t)i * nrhs + c0 + c] = b[i * ldb + c];
-  }
-}
-
-}  // namespace hb
-
-namespace hb {
-
 // ---------------------------------------------------------------------------------------------------------------
-// Substitution with the panel STAGED in shared memory (round 2).  In lu_solve_kernel every row update waits for L2
-// four times per panel (the factor entries of 4 panel columns are requested, used, then the next 4), and the
-// triangular solve of a panel runs on one warp while the other seven wait: 17 800 cycles per panel step on B200,
-// 15 % of them arithmetic.  Here the 16 factor columns of the step (rows below the panel going forward, above it going
-// back) are copied to shared memory with cp.async WHILE warp 0 applies the interchanges and solves the 16 x 16
-// triangle -- neither depends on the other -- and the diagonal block and pivots of the NEXT step travel with them.
-// The update then reads only shared memory.
+// Solve with the factors: B (n x nrhs, row-major, i.e. right-hand side c of row i at B[i * nrhs + c]) is overwritten
+// by the solution, the right-hand sides of a CTA kept in shared memory for the whole forward and backward substitution.
+// The factor columns of a step (rows below the panel going forward, above it going back) are STAGED in shared memory
+// with cp.async WHILE warp 0 applies the interchanges and solves the triangle -- neither depends on the other -- and the
+// diagonal block and pivots of the NEXT step travel with them; the update then reads only shared memory.  The round-1
+// substitution read the factor from L2 in its row updates (4 panel columns at a time, FMA register tiles, the triangle
+// on one warp while seven waited): 17 800 cycles per panel step on B200, 15 % of them arithmetic, and 1.18 ms against
+// this kernel's 0.93 ms per stage of 296 blocks of 337^2 with 88 right-hand sides.
 __device__ __forceinline__ void cp_async8(void* smem_dst, const void* gsrc) {
   const unsigned sdst = (unsigned)__cvta_generic_to_shared(smem_dst);
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(sdst), "l"(gsrc));
@@ -526,7 +302,8 @@ __host__ __device__ inline size_t lu_staged_smem(int n, int ct) {
   return ((size_t)n * (8 * ct) + (size_t)8 * lu_staged_ps(n) + 2) * sizeof(double);
 }
 
-// CT = 8-column tiles of right-hand sides per CTA (4: 32 columns, two CTAs per SM for the 337-blocks).
+// CT = 8-column tiles of right-hand sides per CTA: 4 (32 columns, two CTAs per SM for the 337-blocks) or 3 where 32
+// columns no longer fit (api.cu::lu_plan).
 // * The rows outside the panel are updated on the TENSOR CORES: b[rows][:] += (-P) Y with m8n8k4 fp64 MMAs, 8 x fewer
 //   instructions than 4 x 6 register tiles of fused multiply-adds and a third of their shared-memory reads.
 // * With the update that cheap, the triangle of the panel -- one warp, one right-hand side per lane, the other seven

@@ -12,13 +12,12 @@ is block tridiagonal once unknowns are ordered by stage, u_k = (dx_k, dlam_E,k):
 stage k-1 and stage k are the defect rows of stage k acting on dx_{k-1}.  The solve is a block LU sweep
 over the stages (Riccati-like), batched over instances: per stage one dense LU of an
 (n_k + m_E,k)-square block and one solve with the ~87 coupling columns -- O(N) blocks instead of one
-(n_x + m_E)-square factorisation.  The stage blocks are factored and solved by this library's batched LU
-kernels (csrc/lu.cu through `lu_factor` / `lu_solve`, linalg="hb", CUDA only, no fallback) or, as the
-comparison baseline and for the CPU-side structural tests, by torch.linalg (linalg="torch"); the small
-products around them are torch calls.  What this module owns is the structure: the assignment of rows to
-stages and the gather maps from the CCS value arrays the kernels write to the dense stage blocks.  An
-opt-in two-sided variant of the sweep (`_sweep_two_sided`) halves the chain of stage steps at a loss of
-accuracy on ill-conditioned systems.
+(n_x + m_E)-square factorisation.  With linalg="hb" (CUDA only, no fallback) every stage is assembled by
+one kernel (csrc/kkt_assemble.cu) and factored and solved by this library's batched LU kernels (csrc/lu.cu
+through `lu_factor` / `lu_solve`); linalg="torch", the comparison baseline and what the CPU-side structural
+tests use, assembles the stages with torch indexing and solves them with torch.linalg.  What this module
+owns is the structure: the assignment of rows to
+stages and the gather maps from the CCS value arrays the kernels write to the dense stage blocks.
 
 Checked against a dense solve of the same system (tests/test_kkt_cpu.py on random values in the real
 pattern, tests/test_gpu_kkt.py on evaluated values).  Periodicity rows (knot 0 with knot N-1) make
@@ -192,24 +191,10 @@ class StageKKT:
         loc_B[border] = np.arange(self.n_border)
         jb = np.nonzero(far[jac_row] & is_eq[jac_row])[0]
         self.border = {"idx": t(jb), "row": t(loc_B[jac_row[jb]]), "col": t(jcol[jb]), "eq": t(pos_E[border])}
-        # two-sided elimination (_sweep_two_sided): halves the chain of stage steps; pays while twice the batch still
-        # fits a wave of the factor kernel.  Needs every stage after the first to couple through the same number of rows.
-        ncs = [mp["n_cpl"] for mp in self.maps]
-        self._two_sided_ok = N >= 4 and ncs[0] == 0 and ncs[1] > 0 and all(c == ncs[1] for c in ncs[1:])
-        # OFF by default: the bottom-up half eliminates through G = (S'^-1)[cp, cp], the multiplier block of the inverse,
-        # whose entries grow like 1 / delta_c -- on evaluated values (cond 1e11, delta_c = 1e-9) the relative residual
-        # is 2e-8 against 2e-15 for the one-sided sweep (tests/test_gpu_kkt.py).  Good enough for loose tolerances (the
-        # periodic-step plans with the reference's IPOPT options: 40 -> 34.5 s for 64 plans), not for 1e-6 and below;
-        # a stable version needs the coupling rows of the lower half assigned to the upper stage of each pair.
-        self.two_sided = False
-        # 2 B <= 148 (one CTA per SM on a B200) is free; measured: sweeps of 32 / 64 instances 29 / 37 ms against ~50 ms
-        # one-sided, but 148 instances 58 ms against 55 ms -- no gain once the pair no longer fits one wave
-        self.two_sided_max_batch = 74 if linalg == "hb" else 0
         # ---- tables of the fused assembly kernel (hb_kkt_assemble_stage), in the order include/hippopt_b200.h lists.
         # The fused sweep sizes every stage block by ITS variables and equality rows (nb_k = n_var_k + n_eq_k) instead
         # of the padded maximum: with a final-state constraint the last stage has 81 more rows than the others
         # (config 4: 418 against 331), and a padded block costs (418 / 331)^3 = 2 x the factorisation on 29 of 30 stages.
-        self.fused = linalg == "hb"  # one launch per stage instead of ~25 torch calls; CUDA tensors only
         self._stage_np = []
         self.stage_nx = [len(mp_["var"]) for mp_ in self.maps]
         self.stage_nb = [self.stage_nx[k] + len(self.eq_stage_rows[k]) for k in range(N)]
@@ -275,19 +260,6 @@ class StageKKT:
             raise ValueError(f"{type(ev).__name__} has no multiple-shooting stage structure (layout.knot_size)")
         return cls(ev.n_x, ev.m, lay.N, lay.knot_size, jc, jr, hc, hr, eq, ine, device=device, linalg=linalg), eq, ine
 
-    # ------------------------------------------------------------------ dense block algebra
-    def _lu_factor(self, D):
-        if self.linalg == "hb":
-            F, piv, _ = lu_factor(D, symmetric=True)
-            return F, piv
-        lu, piv, _ = torch.linalg.lu_factor_ex(D)
-        return lu, piv
-
-    def _lu_solve(self, fac, rhs):
-        if self.linalg == "hb":
-            return lu_solve(fac[0], fac[1], rhs)
-        return torch.linalg.lu_solve(fac[0], fac[1], rhs)
-
     # ------------------------------------------------------------------ solve
     def solve(self, hess_vals, jac_vals, sigma_I, delta, delta_c, rhs_x, rhs_E, chunk: int | None = None):
         """Solve K [dx; dlam_E] = [rhs_x; rhs_E] for every instance.
@@ -345,9 +317,9 @@ class StageKKT:
 
     def _sweep(self, hess_vals, jac_vals, sigma_I, delta, delta_c, RX, RE):
         """Block-tridiagonal part: K_bt [DX; DL] = [RX; RE] for R right-hand sides (B, n_x | m_E, R)."""
-        if self.two_sided and self._two_sided_ok and hess_vals.shape[0] <= self.two_sided_max_batch:
-            return self._sweep_two_sided(hess_vals, jac_vals, sigma_I, delta, delta_c, RX, RE)
-        if self.fused and self.linalg == "hb" and hess_vals.is_cuda:
+        if self.linalg == "hb":
+            if not hess_vals.is_cuda:
+                raise ValueError("linalg='hb' runs on CUDA tensors only")
             return self._sweep_fused(hess_vals, jac_vals, sigma_I, delta, delta_c, RX, RE)
         B, R = hess_vals.shape[0], RX.shape[2]
         dev, dt = hess_vals.device, hess_vals.dtype
@@ -356,57 +328,27 @@ class StageKKT:
         DL = torch.zeros((B, self.mE, R), dtype=dt, device=dev)
         Wv, Zs = [], []
         w_prev = None
-
-        def coupling(kk):  # defect rows of stage kk with respect to the variables of stage kk - 1
-            mq = self.maps[kk]
-            Ak = torch.zeros((B, self.mCk * nx), dtype=dt, device=dev)
-            Ak[:, mq["a_pos"]] = jac_vals[:, mq["a_idx"]]
-            return Ak.view(B, self.mCk, nx)[:, :mq["n_cpl"], :]
-
         A = Z = None
         for k in range(N):
             mp = self.maps[k]
-            D = torch.zeros((B, nb * nb), dtype=dt, device=dev)
-            D[:, mp["w_pos"]] = hess_vals[:, mp["w_idx"]]
-            D[:, mp["w_pos_t"]] = hess_vals[:, mp["w_idx"]]
-            D[:, mp["c_pos"]] = jac_vals[:, mp["c_idx"]]
-            D[:, mp["c_pos_t"]] = jac_vals[:, mp["c_idx"]]
-            D = D.view(B, nb, nb)
-            nv, ne = mp["n_var"], mp["n_eq"]
-            if mp["n_ine"]:
-                JI = torch.zeros((B, self.mIk * nx), dtype=dt, device=dev)
-                JI[:, mp["i_pos"]] = jac_vals[:, mp["i_idx"]]
-                JI = JI.view(B, self.mIk, nx)
-                sg = torch.zeros((B, self.mIk), dtype=dt, device=dev)
-                sg[:, :mp["n_ine"]] = sigma_I[:, mp["ine"]]
-                D[:, :nx, :nx] += torch.einsum("bin,bi,bik->bnk", JI, sg, JI)
-            idx = torch.arange(nb, device=dev)
-            diag = torch.zeros((B, nb), dtype=dt, device=dev)
-            diag[:, :nv] = delta[:, None]
-            diag[:, nv:nx] = 1.0             # padding variable slots
-            diag[:, nx:nx + ne] = -delta_c
-            diag[:, nx + ne:] = 1.0          # padding multiplier slots
-            D[:, idx, idx] += diag
-            b = torch.zeros((B, nb, R), dtype=dt, device=dev)
-            b[:, :nv, :] = RX[:, mp["var"], :]
-            b[:, nx:nx + ne, :] = RE[:, mp["eq"], :]
+            D, b = self._assemble(k, hess_vals, jac_vals, sigma_I, delta, delta_c, RX, RE)
             Zs.append(Z)
             if Z is not None:  # Z = S_{k-1}^{-1} [A_k^T; 0] came out of the previous stage's solve
                 cp = mp["cpl"]
                 D[:, cp[:, None], cp[None, :]] -= torch.bmm(A, Z[:, :nx, :])
                 b[:, cp, :] -= torch.bmm(A, w_prev[:, :nx, :])
-            fac = self._lu_factor(D)  # the stage block is symmetric
+            fac = torch.linalg.lu_factor_ex(D)[:2]
             # one solve per stage: the stage's right-hand sides and the coupling columns of the next stage
             if k + 1 < N and self.maps[k + 1]["n_cpl"]:
-                A = coupling(k + 1)
+                A = self._coupling(k + 1, jac_vals)
                 rhs = torch.zeros((B, nb, R + A.shape[1]), dtype=dt, device=dev)
                 rhs[:, :, :R] = b
                 rhs[:, :nx, R:] = A.transpose(1, 2)
-                sol = self._lu_solve(fac, rhs)
+                sol = torch.linalg.lu_solve(*fac, rhs)
                 w_prev, Z = sol[:, :, :R], sol[:, :, R:]
             else:
                 A = Z = None
-                w_prev = self._lu_solve(fac, b)
+                w_prev = torch.linalg.lu_solve(*fac, b)
             Wv.append(w_prev)
         u_next = None
         for k in range(N - 1, -1, -1):
@@ -471,7 +413,7 @@ class StageKKT:
             cache[key] = torch.as_tensor(np.ascontiguousarray(self.cpl_local[k]), dtype=torch.long, device=dev)
         return cache[key]
 
-    # ------------------------------------------------------------------ two-sided sweep
+    # ------------------------------------------------------------------ torch assembly of a stage
     def _assemble(self, k, hess_vals, jac_vals, sigma_I, delta, delta_c, RX, RE):
         """Stage block D_k (B, nb, nb) and right-hand sides b_k (B, nb, R) without the coupling terms."""
         B, R = hess_vals.shape[0], RX.shape[2]
@@ -495,9 +437,9 @@ class StageKKT:
         idx = torch.arange(nb, device=dev)
         diag = torch.zeros((B, nb), dtype=dt, device=dev)
         diag[:, :nv] = delta[:, None]
-        diag[:, nv:nx] = 1.0
+        diag[:, nv:nx] = 1.0             # padding variable slots
         diag[:, nx:nx + ne] = -delta_c
-        diag[:, nx + ne:] = 1.0
+        diag[:, nx + ne:] = 1.0          # padding multiplier slots
         D[:, idx, idx] += diag
         b = torch.zeros((B, nb, R), dtype=dt, device=dev)
         b[:, :nv, :] = RX[:, mp["var"], :]
@@ -511,80 +453,6 @@ class StageKKT:
         Ak = torch.zeros((B, self.mCk * self.nx), dtype=jac_vals.dtype, device=jac_vals.device)
         Ak[:, mq["a_pos"]] = jac_vals[:, mq["a_idx"]]
         return Ak.view(B, self.mCk, self.nx)[:, :mq["n_cpl"], :]
-
-    def _sweep_two_sided(self, hess_vals, jac_vals, sigma_I, delta, delta_c, RX, RE):
-        """The same block-tridiagonal solve with the elimination running from both ends towards stage m = N // 2:
-        stages 0 .. m-1 top-down (Schur complement S_k = D_k - [A_k] S_{k-1}^{-1} [A_k]^T on the coupling rows, as in
-        `_sweep`), stages N-1 .. m+1 bottom-up (S'_k = D_k - A_{k+1}^T G_{k+1} A_{k+1} on the variable slots, with
-        G_{k+1} = (S'_{k+1}^{-1})[cp, cp] from a solve against the unit columns of the coupling rows).  Step j factors
-        stage j and stage N-1-j in ONE batched call, so the chain of latency-bound LU steps is N/2 + 1 long instead
-        of N -- worth it while 2 B matrices still fit a wave of the factor kernel."""
-        B, R = hess_vals.shape[0], RX.shape[2]
-        dev, dt = hess_vals.device, hess_vals.dtype
-        nx, nb, N = self.nx, self.nb, self.N
-        m = N // 2
-        nc = self.maps[1]["n_cpl"]
-        args = (hess_vals, jac_vals, sigma_I, delta, delta_c, RX, RE)
-        Wt, Zt = [None] * N, [None] * N      # top-down: w_k = S_k^{-1} b_k, Z_k = S_k^{-1} [A_{k+1}^T; 0]
-        Wb, Yb = [None] * N, [None] * N      # bottom-up: w'_k, Y_k = S'_k^{-1} P_cp
-        Acp = {k: self._coupling(k, jac_vals) for k in range(1, N)}
-
-        def unit_columns(k):
-            P = torch.zeros((B, nb, nc), dtype=dt, device=dev)
-            P[:, self.maps[k]["cpl"], torch.arange(nc, device=dev)] = 1.0
-            return P
-
-        for j in range(max(m, N - 1 - m)):
-            kt = j if j < m else None
-            kb = N - 1 - j if N - 1 - j > m else None
-            Ds, rhss = [], []
-            if kt is not None:
-                D, b = self._assemble(kt, *args)
-                if kt > 0:
-                    cp = self.maps[kt]["cpl"]
-                    D[:, cp[:, None], cp[None, :]] -= torch.bmm(Acp[kt], Zt[kt - 1][:, :nx, :])
-                    b[:, cp, :] -= torch.bmm(Acp[kt], Wt[kt - 1][:, :nx, :])
-                E = torch.zeros((B, nb, nc), dtype=dt, device=dev)
-                E[:, :nx, :] = Acp[kt + 1].transpose(1, 2)
-                Ds.append(D)
-                rhss.append(torch.cat([b, E], dim=2))
-            if kb is not None:
-                D, b = self._assemble(kb, *args)
-                if kb < N - 1:
-                    cpn = self.maps[kb + 1]["cpl"]
-                    An = Acp[kb + 1]
-                    G = Yb[kb + 1][:, cpn, :]
-                    D[:, :nx, :nx] -= torch.bmm(An.transpose(1, 2), torch.bmm(G, An))
-                    b[:, :nx, :] -= torch.bmm(An.transpose(1, 2), Wb[kb + 1][:, cpn, :])
-                Ds.append(D)
-                rhss.append(torch.cat([b, unit_columns(kb)], dim=2))
-            sol = self._lu_solve(self._lu_factor(torch.cat(Ds)), torch.cat(rhss))
-            if kt is not None:
-                Wt[kt], Zt[kt] = sol[:B, :, :R], sol[:B, :, R:]
-            if kb is not None:
-                Wb[kb], Yb[kb] = sol[-B:, :, :R], sol[-B:, :, R:]
-        # middle stage: both contributions
-        D, b = self._assemble(m, *args)
-        cp = self.maps[m]["cpl"]
-        D[:, cp[:, None], cp[None, :]] -= torch.bmm(Acp[m], Zt[m - 1][:, :nx, :])
-        b[:, cp, :] -= torch.bmm(Acp[m], Wt[m - 1][:, :nx, :])
-        if m < N - 1:
-            cpn, An = self.maps[m + 1]["cpl"], Acp[m + 1]
-            D[:, :nx, :nx] -= torch.bmm(An.transpose(1, 2), torch.bmm(Yb[m + 1][:, cpn, :], An))
-            b[:, :nx, :] -= torch.bmm(An.transpose(1, 2), Wb[m + 1][:, cpn, :])
-        U = [None] * N
-        U[m] = self._lu_solve(self._lu_factor(D), b)
-        for k in range(m - 1, -1, -1):
-            U[k] = Wt[k] - torch.bmm(Zt[k], U[k + 1][:, self.maps[k + 1]["cpl"], :])
-        for k in range(m + 1, N):
-            U[k] = Wb[k] - torch.bmm(Yb[k], torch.bmm(Acp[k], U[k - 1][:, :nx, :]))
-        DX = torch.zeros((B, self.n_x, R), dtype=dt, device=dev)
-        DL = torch.zeros((B, self.mE, R), dtype=dt, device=dev)
-        for k in range(N):
-            mp = self.maps[k]
-            DX[:, mp["var"], :] = U[k][:, :mp["n_var"], :]
-            DL[:, mp["eq"], :] = U[k][:, nx:nx + mp["n_eq"], :]
-        return DX, DL
 
     # ------------------------------------------------------------------ reference: the same matrix, dense
     def dense_matrix(self, hess_vals, jac_vals, sigma_I, delta, delta_c, eq_rows, ine_rows, jac_colind, jac_row,

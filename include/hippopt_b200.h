@@ -269,8 +269,8 @@ int hb_eval_cost_terms(hb_handle h, const double* x, const double* p, int64_t p_
  * A call that fits one chunk (batch <= 128) and repeats with the same mask and the same PINNED host pointers -- one
  * instance per call, every iterate, is what a CPU-side IPOPT does -- is captured as a CUDA graph on its second
  * occurrence and replayed from then on (copies, kernels and their events as one launch; up to 8 such call shapes per
- * handle; HB_NO_HOST_GRAPH=1 in the environment turns it off).  The host buffers of such a call must stay allocated
- * (and pinned) for as long as they are passed with that handle; new parameters of another size drop the graphs. */
+ * handle).  The host buffers of such a call must stay allocated (and pinned) for as long as they are passed with that
+ * handle; new parameters of another size drop the graphs. */
 int hb_host_set_parameters(hb_handle h, const double* p, int64_t p_stride, int64_t batch);
 int hb_eval_host(hb_handle h, uint32_t mask, const double* x, const double* lam_g, const double* sigma,
                  double* f, double* grad_f, double* g, double* jac_vals, double* hess_vals, int64_t batch);
@@ -307,7 +307,7 @@ int hb_profile_read(hb_handle h, double* ms3, int64_t* n_evals);
  *                               meant for hb_lu_solve_batched, not for LAPACK's getrs
  *   info  device [batch]        0, or 1 + index of the first exactly-zero / NaN pivot column
  *   Bm    device [batch][n*nrhs] row-major right-hand sides (entry (i, c) at i*nrhs + c), overwritten by X
- * n <= 768 (panel and right-hand sides live in shared memory).  One CTA per matrix (and per 32
+ * n <= 768 (panel and right-hand sides live in shared memory).  One CTA per matrix (and per 24 or 32
  * right-hand sides). */
 int hb_lu_factor_batched(double* A, int32_t* piv, int32_t* info, int64_t n, int64_t batch, void* stream);
 int hb_lu_solve_batched(const double* LU, const int32_t* piv, double* Bm, int64_t n, int64_t nrhs, int64_t batch,
@@ -315,7 +315,7 @@ int hb_lu_solve_batched(const double* LU, const int32_t* piv, double* Bm, int64_
 /* Host-only: the kernel variants hb_lu_factor_batched / hb_lu_solve_batched launch for (n, batch, nrhs) on a device
  * with `sms` SMs (the same function picks them), for tests that must know which variant a case runs.
  *   out[4]  RPT (panel rows per thread), MB (CTAs per SM of the factor kernel's register budget), ct (8-column tiles of
- *           right-hand sides per CTA of the staged solve; 0 = the unstaged kernel), column chunks per matrix */
+ *           right-hand sides per CTA of the solve: 3 or 4), column chunks per matrix */
 int hb_debug_lu_plan(int64_t n, int64_t batch, int64_t nrhs, int32_t sms, int32_t* out);
 
 /* One stage of the block-tridiagonal KKT sweep (hippopt_b200/kkt.py::StageKKT) assembled in one launch from the CCS

@@ -70,18 +70,16 @@ def test_stage_sweep_on_evaluated_values(model, built_library, periodic):
     g = torch.Generator().manual_seed(1)
     hv, jv = out["hess"].clone(), out["jac"].clone()
     sols = {}
-    for linalg in ("hb", "hb-unfused", "torch"):  # hb: one assembly kernel per stage; hb-unfused: the torch assembly
-        kkt, eq, ine = StageKKT.for_evaluator(ev, lb[0], ub[0], device=d, linalg=linalg.split("-")[0])
-        if linalg == "hb-unfused":
-            kkt.fused = False
+    for linalg in ("hb", "torch"):  # hb: one assembly kernel per stage; torch: the torch assembly and torch.linalg
+        kkt, eq, ine = StageKKT.for_evaluator(ev, lb[0], ub[0], device=d, linalg=linalg)
         if linalg == "hb":
-            assert kkt.fused
             sig = (torch.rand((B, len(ine)), generator=g, dtype=torch.float64) * 10.0).to(d)
             delta = torch.full((B,), 1e-2, dtype=torch.float64, device=d)
             rx = torch.randn((B, ev.n_x), generator=g, dtype=torch.float64).to(d)
             rE = torch.randn((B, len(eq)), generator=g, dtype=torch.float64).to(d)
             rE[:, torch.as_tensor(kkt.dead_eq, device=d)] = 0.0
         sols[linalg] = torch.cat(kkt.solve(hv, jv, sig, delta, 1e-9, rx, rE, chunk=2), dim=1)  # 3 chunks
+        assert (kkt._stage_dev is not None) == (linalg == "hb")  # hb ran the fused sweep: its stage tables are uploaded
     jc, jr = ev.jac_sparsity()
     hc, hr = ev.hess_sparsity()
     K = kkt.dense_matrix(hv, jv, sig, delta, 1e-9, eq, ine, jc, jr, hc, hr)
@@ -128,7 +126,6 @@ def test_stage_sweep_at_the_production_chunk(model, built_library, periodic):
     out = ev.eval(ALL, *(torch.tensor(a, device=d) for a in (x, p, lam, np.ones(B))))
     hv, jv = out["hess"].clone(), out["jac"].clone()
     kkt, eq, ine = StageKKT.for_evaluator(ev, lb[0], ub[0], device=d, linalg="hb")
-    assert kkt.fused
     plan = (ctypes.c_int32 * 4)()
     for batch, mb in ((chunk, 2), (3, 1)):
         assert built_library.hb_debug_lu_plan(kkt.nb, batch, 1, sms, plan) == 0 and plan[1] == mb, (kkt.nb, batch)
@@ -139,6 +136,7 @@ def test_stage_sweep_at_the_production_chunk(model, built_library, periodic):
     rE = torch.randn((B, len(eq)), generator=g, dtype=torch.float64).to(d)
     rE[:, torch.as_tensor(kkt.dead_eq, device=d)] = 0.0
     u = torch.cat(kkt.solve(hv, jv, sig, delta, 1e-9, rx, rE), dim=1)  # default chunk
+    assert kkt._stage_dev is not None  # the fused sweep ran (its stage tables are on the device)
     rhs = torch.cat([rx, rE], dim=1)
     jc, jr = ev.jac_sparsity()
     hc, hr = ev.hess_sparsity()

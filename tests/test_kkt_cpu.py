@@ -103,36 +103,6 @@ def test_sparse_operators_match_dense(model):
     assert torch.equal(W, W.transpose(1, 2))
 
 
-@pytest.mark.parametrize("N,final,periodic", [(4, False, False), (5, False, False), (7, True, False), (6, True, True),
-                                              (5, False, True)])
-def test_two_sided_sweep_matches_dense_and_one_sided(model, N, final, periodic):
-    """`_sweep_two_sided` (elimination from both ends towards the middle stage, two stages per batched LU call):
-    same solution as the dense solve and as the one-sided sweep, with and without the periodicity border."""
-    lay, kkt, eq, ine = _setup(model, N, final, periodic)
-    assert kkt._two_sided_ok
-    B = 2
-    g = torch.Generator().manual_seed(100 + N)
-    hv = torch.randn((B, lay.nnz_h), generator=g, dtype=torch.float64)
-    jv = torch.randn((B, lay.nnz_j), generator=g, dtype=torch.float64)
-    sig = torch.rand((B, len(ine)), generator=g, dtype=torch.float64) * 3.0
-    delta = torch.tensor([45.0, 60.0], dtype=torch.float64)
-    rx = torch.randn((B, lay.n_x), generator=g, dtype=torch.float64)
-    rE = torch.randn((B, len(eq)), generator=g, dtype=torch.float64)
-    rE[:, kkt.dead_eq] = 0.0
-    assert not kkt.two_sided  # opt-in: less accurate than the one-sided sweep on ill-conditioned systems (kkt.py)
-    one = torch.cat(kkt.solve(hv, jv, sig, delta, 1e-6, rx, rE), dim=1)
-    kkt.two_sided, kkt.two_sided_max_batch = True, 10 ** 9
-    two = torch.cat(kkt.solve(hv, jv, sig, delta, 1e-6, rx, rE), dim=1)
-    K = kkt.dense_matrix(hv, jv, sig, delta, 1e-6, eq, ine, lay.jac_colind, lay.jac_row, lay.hess_colind, lay.hess_row)
-    ref = torch.linalg.solve(K, torch.cat([rx, rE], dim=1))
-    scale = ref.abs().amax(dim=1, keepdim=True)
-    assert ((two - ref).abs() / scale).max().item() < 1e-9
-    assert ((two - one).abs() / scale).max().item() < 1e-9
-    # N < 4 (or irregular coupling) falls back to the one-sided sweep
-    _, small, _, _ = _setup(model, 3, False)
-    assert not small._two_sided_ok
-
-
 def _emulate_assemble(hdr, tab, hv, jv, sig, delta, delta_c, RX, RE, prev):
     """numpy restatement of csrc/kkt_assemble.cu for ONE instance: what hb_kkt_assemble_stage builds from a stage table."""
     nb, nx, nv, ne, R, n_cpl, n_cpl_next, n_direct, n_targets, n_contrib, n_a, n_an, nb_prev = hdr
@@ -168,7 +138,7 @@ def _emulate_assemble(hdr, tab, hv, jv, sig, delta, delta_c, RX, RE, prev):
 @pytest.mark.parametrize("N,final", [(3, False), (3, True)])
 def test_fused_stage_tables_match_the_torch_assembly(model, N, final):
     """The tables hb_kkt_assemble_stage consumes (per-stage block sizes, value entries, J_I^T Sigma J_I contribution lists,
-    coupling rows) against the torch assembly of the unfused sweep, through a numpy restatement of the kernel."""
+    coupling rows) against the torch assembly of the linalg="torch" sweep, through a numpy restatement of the kernel."""
     lay, kkt, eq, ine = _setup(model, N, final)
     g = torch.Generator().manual_seed(7)
     hv = torch.randn((1, lay.nnz_h), generator=g, dtype=torch.float64)
