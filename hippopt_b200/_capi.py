@@ -127,6 +127,8 @@ def lib() -> ctypes.CDLL:
     L.hb_debug_lu_plan.argtypes = [ctypes.c_int64, ctypes.c_int64, ctypes.c_int64, ctypes.c_int32, i32p]
     L.hb_debug_smooth_terrain.restype = ctypes.c_int
     L.hb_debug_smooth_terrain.argtypes = [vp, vp, ctypes.c_int64, vp, vp]
+    L.hb_debug_tilted_terrain.restype = ctypes.c_int
+    L.hb_debug_tilted_terrain.argtypes = [vp, ctypes.c_int32, vp, ctypes.c_int64, vp, vp]
     i64 = ctypes.c_int64
     L.hb_interpolate_humanoid_states.restype = ctypes.c_int
     L.hb_interpolate_humanoid_states.argtypes = [i64, i64, i64, vp, vp, vp, vp, i64, i64, vp, i64, i64, vp, vp, i64, i64, vp]
@@ -150,7 +152,8 @@ EXPORTED_SYMBOLS = [
     "hb_kino_create", "hb_toy_create", "hb_destroy", "hb_dims", "hb_pattern_jac", "hb_pattern_hess", "hb_eval",
     "hb_last_launch_count", "hb_last_error", "hb_probe_fp64_tflops", "hb_profile_enable", "hb_profile_read",
     "hb_host_set_parameters", "hb_eval_host", "hb_host_last_traffic", "hb_host_alloc", "hb_host_free",
-    "hb_lu_factor_batched", "hb_lu_solve_batched", "hb_debug_lu_plan", "hb_debug_smooth_terrain", "hb_set_option", "hb_interpolate_humanoid_states",
+    "hb_lu_factor_batched", "hb_lu_solve_batched", "hb_debug_lu_plan", "hb_debug_smooth_terrain", "hb_debug_tilted_terrain",
+    "hb_set_option", "hb_interpolate_humanoid_states",
     "hb_eval_cost_terms", "hb_debug_sweep_schedule", "hb_debug_sweep_schedule_n_base", "hb_kino_attach_tables",
     "hb_bounds", "hb_save", "hb_load",
     "hb_ccs_group_mul", "hb_external_bind", "hb_external_stats", "hb_kkt_assemble_stage",

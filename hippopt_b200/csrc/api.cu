@@ -116,10 +116,12 @@ static cudaError_t ensure_kernel_attributes(int dev) {
   cudaError_t e;
   if ((e = cudaFuncSetAttribute(hb::kino_contact_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, big)) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(hb::kino_contact_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, big)) != cudaSuccess) return e;
+  if ((e = cudaFuncSetAttribute(hb::kino_contact_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, big)) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(hb::kino_kin_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, big)) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(hb::kino_kin_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, big)) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(hb::pose_contact_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, big)) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(hb::pose_contact_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, big)) != cudaSuccess) return e;
+  if ((e = cudaFuncSetAttribute(hb::pose_contact_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, big)) != cudaSuccess) return e;
   const int lu_big = 210 * 1024;
   if ((e = cudaFuncSetAttribute(hb::lu_factor_kernel<1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, lu_big)) != cudaSuccess) return e;
   if ((e = cudaFuncSetAttribute(hb::lu_factor_kernel<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, lu_big)) != cudaSuccess) return e;
@@ -271,9 +273,15 @@ extern "C" int hb_kino_create(const int32_t* icfg, const double* dcfg, const int
     delete h;
     return fail(HB_ERR_UNSUPPORTED, "hb_kino_create: the pose finder is a single-knot problem");
   }
-  if (C.terrain != 0 && C.terrain != 1) {
+  if (C.terrain != 0 && C.terrain != 1 && C.terrain != 2) {
     delete h;
-    return fail(HB_ERR_UNSUPPORTED, "hb_kino_create: terrain must be 0 (planar) or 1 (two smooth steps)");
+    return fail(HB_ERR_UNSUPPORTED,
+                "hb_kino_create: terrain must be 0 (planar), 1 (two smooth steps) or 2 (general smooth steps)");
+  }
+  if (C.terrain == 2 && (C.n_p - C.po_terrain < 10 || (C.n_p - C.po_terrain) % 10 != 0)) {
+    delete h;
+    return fail(HB_ERR_INVALID, "hb_kino_create: terrain 2 needs n_p - po_terrain to be a positive multiple of 10 "
+                                "(one (l, w, height, ox, oy, oz, yaw, n_x, n_y, n_z) record per step)");
   }
   if (C.nb < 2 || C.nb > HB_MAX_BODIES || C.nb - 1 != HB_N_JOINTS) {
     delete h;
@@ -778,12 +786,20 @@ extern "C" int hb_eval(hb_handle h, uint32_t mask, const double* x, const double
       hb::pose_contact_kernel<0><<<grid, 32 * warps_per_block, smem, st>>>(h->dev, mask, x, p, (long)p_stride, lam_g, sigma,
                                                                           d_fpart, grad_f, g, jac_vals, hess_vals,
                                                                           (long)batch);
-    } else if (C.kind == 1) {
+    } else if (C.kind == 1 && C.terrain == 1) {
       hb::pose_contact_kernel<1><<<grid, 32 * warps_per_block, smem, st>>>(h->dev, mask, x, p, (long)p_stride, lam_g, sigma,
+                                                                          d_fpart, grad_f, g, jac_vals, hess_vals,
+                                                                          (long)batch);
+    } else if (C.kind == 1) {
+      hb::pose_contact_kernel<2><<<grid, 32 * warps_per_block, smem, st>>>(h->dev, mask, x, p, (long)p_stride, lam_g, sigma,
                                                                           d_fpart, grad_f, g, jac_vals, hess_vals,
                                                                           (long)batch);
     } else if (C.terrain == 0)
       hb::kino_contact_kernel<0><<<grid, 32 * warps_per_block, smem, st_contact>>>(h->topo, h->dev, mask, x, p, (long)p_stride,
+                                                                                  lam_g, sigma, d_fpart, grad_f, g, jac_vals,
+                                                                                  hess_vals, (long)batch);
+    else if (C.terrain == 2)
+      hb::kino_contact_kernel<2><<<grid, 32 * warps_per_block, smem, st_contact>>>(h->topo, h->dev, mask, x, p, (long)p_stride,
                                                                                   lam_g, sigma, d_fpart, grad_f, g, jac_vals,
                                                                                   hess_vals, (long)batch);
     else
@@ -1074,17 +1090,18 @@ extern "C" int hb_debug_lu_plan(int64_t n, int64_t batch, int64_t nrhs, int32_t 
 
 namespace hb {
 // one thread per point: the production surface and frame jets, unchanged, written out for the tests
-__global__ void debug_smooth_terrain_kernel(const double* __restrict__ tp, const double* __restrict__ pts, long n,
-                                            double* __restrict__ out) {
+template <int TERRAIN>
+__global__ void debug_terrain_kernel(const double* __restrict__ tp, int n_steps, const double* __restrict__ pts, long n,
+                                     double* __restrict__ out) {
   const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const double* t = tp + 10 * i;
+  const double* t = tp + 10 * (TERRAIN == 1 ? 1 : n_steps) * i;
   const double x = pts[3 * i], y = pts[3 * i + 1], z = pts[3 * i + 2];
   double* o = out + HB_SMOOTH_TERRAIN_OUT * i;
-  const BJ<4> T = smooth_steps_surface(t, x, y);
+  const BJ<4> T = terrain_surface<TERRAIN>(t, n_steps, x, y);
   for (int k = 0; k < BJ<4>::SIZE; ++k) o[k] = T.c[k];
   TFrame F;
-  smooth_terrain_frame(t, x, y, z, F);
+  terrain_frame<TERRAIN>(t, n_steps, x, y, z, F);
   const TJ* f[18] = {&F.h, &F.gx, &F.gy, &F.n[0], &F.n[1], &F.n[2], &F.xh[0], &F.xh[1], &F.xh[2],
                      &F.yh[0], &F.yh[1], &F.yh[2], &F.Dn[0][0], &F.Dn[0][1], &F.Dn[1][0], &F.Dn[1][1],
                      &F.Dn[2][0], &F.Dn[2][1]};
@@ -1096,7 +1113,17 @@ static_assert(BJ<4>::SIZE + 18 * 10 == HB_SMOOTH_TERRAIN_OUT, "hb_debug_smooth_t
 
 extern "C" int hb_debug_smooth_terrain(const double* tp, const double* pts, int64_t n, double* out, void* stream) {
   if (!tp || !pts || !out || n <= 0) return fail(HB_ERR_INVALID, "hb_debug_smooth_terrain: null argument or n <= 0");
-  hb::debug_smooth_terrain_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(tp, pts, (long)n, out);
+  hb::debug_terrain_kernel<1><<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(tp, 0, pts, (long)n, out);
+  CUDA_TRY(cudaGetLastError());
+  return HB_OK;
+}
+
+extern "C" int hb_debug_tilted_terrain(const double* tp, int32_t n_steps, const double* pts, int64_t n, double* out,
+                                       void* stream) {
+  if (!tp || !pts || !out || n <= 0 || n_steps <= 0)
+    return fail(HB_ERR_INVALID, "hb_debug_tilted_terrain: null argument, n <= 0 or n_steps <= 0");
+  hb::debug_terrain_kernel<2><<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(tp, n_steps, pts, (long)n,
+                                                                                            out);
   CUDA_TRY(cudaGetLastError());
   return HB_OK;
 }
@@ -1432,6 +1459,9 @@ extern "C" int hb_eval_cost_terms(hb_handle h, const double* x, const double* p,
   const size_t smem_c = (size_t)hb::kino_contact_smem_layout(C.n_hc).total * sizeof(double) * wpb;
   if (C.terrain == 0)
     hb::kino_contact_kernel<0><<<grid, 32 * wpb, smem_c, st>>>(h->topo, h->dev, mask, x, p, (long)p_stride, nullptr, nullptr,
+                                                              terms, nullptr, nullptr, nullptr, nullptr, (long)batch);
+  else if (C.terrain == 2)
+    hb::kino_contact_kernel<2><<<grid, 32 * wpb, smem_c, st>>>(h->topo, h->dev, mask, x, p, (long)p_stride, nullptr, nullptr,
                                                               terms, nullptr, nullptr, nullptr, nullptr, (long)batch);
   else
     hb::kino_contact_kernel<1><<<grid, 32 * wpb, smem_c, st>>>(h->topo, h->dev, mask, x, p, (long)p_stride, nullptr, nullptr,

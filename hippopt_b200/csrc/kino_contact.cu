@@ -111,7 +111,8 @@ __device__ __forceinline__ void linear_state(int j, int& so, int& ro, int& fam_d
   }
 }
 
-// TERRAIN: 0 = PlanarTerrain, 1 = sum of two smooth steps (kino_smooth.cuh)
+// TERRAIN: 0 = PlanarTerrain, 1 = sum of two smooth steps, 2 = sum of K general (rotated, raised, tilted) smooth steps
+// (kino_smooth.cuh)
 // CTAs per SM of the planar kernel, kernel time per bench step (config 3, NVIDIA B200 at 1000 W, 1965 MHz, three
 // alternated runs): 5 (96 registers, no spill) 0.241 ms, 6 (80, 12 B spill) 0.224 ms, 7 (72, 8 B spill) 0.213 ms.
 // Shared memory allows 7: 30 976 B per CTA.
@@ -207,7 +208,7 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
     }
     if (rd >= 0) lam_dcc = lb[rd];
     if (rf >= 0) lam_fr = lb[rf];
-    if constexpr (TERRAIN == 1) {
+    if constexpr (TERRAIN != 0) {
       lam_h = lamrow(fb_ + HB_KF_PT_HEIGHT, k, 0);
       lam_n = lamrow(fb_ + HB_KF_PT_NORMAL, k, 0);
     }
@@ -302,14 +303,15 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
   const D3 pv = ld3(zpt + Z_V), pfd = ld3(zpt + Z_FD), ppos = ld3(zpt + Z_P), pf = ld3(zpt + Z_F), pu = ld3(zpt + Z_U);
   const double tau = tanh(kt * ppos.z);
 
-  if constexpr (TERRAIN == 1) {
-    // ---------------------------------------------------------------- smooth-step terrain (config 5)
+  if constexpr (TERRAIN != 0) {
+    // ---------------------------------------------------------------- smooth-step terrains (config 5, the ramp)
     const double* tp = pp + C.po_terrain;
+    const int n_steps = TERRAIN == 2 ? (G.n_p - C.po_terrain) / 10 : 0;  // the step records close p
     if (lane < 8) {
       const int fb_ = lane * HB_KF_PT_COUNT;
       const int o = 15 * lane;
       TFrame F;
-      smooth_terrain_frame(tp, ppos.x, ppos.y, ppos.z, F);
+      terrain_frame<TERRAIN>(tp, n_steps, ppos.x, ppos.y, ppos.z, F);
       const double t0 = tanh(kt * F.h.c[0]);
       const double t1 = kt * (1.0 - t0 * t0);
       const TJ tauj = tj_compose(F.h, t0, t1, -kt * t0 * t1);
@@ -468,7 +470,7 @@ __global__ void __launch_bounds__(128, TERRAIN == 0 ? CONTACT_MIN_BLOCKS : 1) ki
     }
     if (lane == 8) {
       // minimum CoM height: h(com) = com_z - T(com_x, com_y)
-      const BJ<2> T2 = bj_trunc<4, 2>(smooth_steps_surface(tp, comv.x, comv.y));
+      const BJ<2> T2 = bj_trunc<4, 2>(terrain_surface<TERRAIN>(tp, n_steps, comv.x, comv.y));
       if (want_g) {
         const int r = grow(C, HB_KF_COM_HEIGHT, k, 0);
         if (r >= 0) gb[r] = comv.z - T2.c[0];

@@ -1,20 +1,48 @@
-// kino_smooth.cuh -- smooth-step terrain (BASELINE config 5) for the contact kernel.
+// kino_smooth.cuh -- smooth-step terrains for the contact kernels.
 //
 // Restates, with runtime parameters instead of baked constants,
 //   SmoothTerrain.create_height_function   utilities/smooth_terrain.py:201-227
-//   SmoothTerrain.step                     utilities/smooth_terrain.py:266-336   (edge 5, side 10, yaw 0)
+//   SmoothTerrain.step                     utilities/smooth_terrain.py:235-336
 //   TerrainSum.create_height_function      utilities/terrain_sum.py:19-38
 //   TerrainDescriptor normal / orientation utilities/terrain_descriptor.py:45-80
 // and the terrain-dependent rows/costs of the contact block (complementarity.py:24-32, 68-89;
 // contacts.py:24, 54-66, 158-166) including their first and second derivatives, obtained from
 // truncated Taylor series of the surface (hb_jet.cuh) instead of CasADi's graph AD.
 //
+// Kernel terrain 1, the stairs (BASELINE config 5): two axis-aligned flat steps with origins at z = 0,
 //   h(p) = z - sum_i exp(-g_i^20) height_i,   g_i = (2 (x - ox_i) / l_i)^10 + (2 (y - oy_i) / w_i)^10
 // terrain parameters tp[10] = (l, w, height, ox, oy) x 2.
+//
+// Kernel terrain 2, K general steps (the ramp's terrain): yaw theta, origin o and a top tilted to the normal n,
+//   (x_t, y_t) = R_z(theta)^T (p - o),   g = (2 x_t / l)^10 + (2 y_t / w)^10,
+//   h(p) = z - sum_i [exp(-g_i^20) pi_i(x_t, y_t) + oz_i],   pi = height - n_x / n_z x_t - n_y / n_z y_t
+// terrain parameters tp[10 K] = (l, w, height, ox, oy, oz, yaw, n_x, n_y, n_z) x K.
 #pragma once
 #include "hb_jet.cuh"
 
 namespace hb {
+
+// exp(-g^20) of one step as a series, from the series of g.  Far outside the step exp(-g^20) underflows to exactly 0
+// while the powers of g overflow; the reference's graph then evaluates 0 * inf = NaN in the high derivatives.  The limit
+// is 0, so callers skip the step where g0 > STEP_CUTOFF (identical wherever the reference is finite, finite where it is
+// not): g^20 > 1100 > -log(DBL_TRUE_MIN), so exp(-G) == 0 in fp64.
+constexpr double STEP_CUTOFF = 1.42;
+__device__ __forceinline__ BJ<4> step_bump(const BJ<4>& g) {
+  // G = g^20: C(20,k) g0^(20-k)
+  const double g0 = g.c[0];
+  const double g2 = g0 * g0, g4 = g2 * g2, g8 = g4 * g4, g16 = g8 * g8;
+  double fp[5];
+  fp[4] = 4845.0 * g16;
+  fp[3] = 1140.0 * g16 * g0;
+  fp[2] = 190.0 * g16 * g2;
+  fp[1] = 20.0 * g16 * g2 * g0;
+  fp[0] = g16 * g4;
+  const BJ<4> G = bj_compose<4>(g, fp);
+  // E = exp(-G)
+  const double e0 = exp(-G.c[0]);
+  const double fe[5] = {e0, e0, e0 / 2.0, e0 / 6.0, e0 / 24.0};
+  return bj_compose<4>(-G, fe);
+}
 
 __device__ __forceinline__ BJ<4> smooth_steps_surface(const double* __restrict__ tp, double x, double y) {
   BJ<4> T = bj_const<4>(0.0);
@@ -34,27 +62,59 @@ __device__ __forceinline__ BJ<4> smooth_steps_surface(const double* __restrict__
     g.c[bidx(0, 2)] = 45.0 * Y6 * Y2 * dY * dY;
     g.c[bidx(0, 3)] = 120.0 * Y6 * Y0 * dY * dY * dY;
     g.c[bidx(0, 4)] = 210.0 * Y6 * dY * dY * dY * dY;
-    // G = g^20: C(20,k) g0^(20-k)
     const double g0 = g.c[0];
-    // Far outside the step exp(-g^20) underflows to exactly 0 while the powers of g overflow; the
-    // reference's graph then evaluates 0 * inf = NaN in the high derivatives.  The limit is 0, so the
-    // step is skipped there (identical wherever the reference is finite, finite where it is not).
-    if (g0 > 1.42) continue;  // g^20 > 1100 > -log(DBL_TRUE_MIN): exp(-G) == 0 in fp64
-    const double g2 = g0 * g0, g4 = g2 * g2, g8 = g4 * g4, g16 = g8 * g8;
-    double fp[5];
-    fp[4] = 4845.0 * g16;
-    fp[3] = 1140.0 * g16 * g0;
-    fp[2] = 190.0 * g16 * g2;
-    fp[1] = 20.0 * g16 * g2 * g0;
-    fp[0] = g16 * g4;
-    const BJ<4> G = bj_compose<4>(g, fp);
-    // E = exp(-G)
-    const double e0 = exp(-G.c[0]);
-    const double fe[5] = {e0, e0, e0 / 2.0, e0 / 6.0, e0 / 24.0};
-    const BJ<4> E = bj_compose<4>(-G, fe);
+    if (g0 > STEP_CUTOFF) continue;
+    const BJ<4> E = step_bump(g);
     T = T + height * E;
   }
   return T;
+}
+
+// t^10 of a linear series t: C(10,k) t0^(10-k) composed with t - t0
+__device__ __forceinline__ BJ<4> bj_pow10(const BJ<4>& t) {
+  const double t0 = t.c[0], t2 = t0 * t0, t4 = t2 * t2, t6 = t4 * t2;
+  const double f[5] = {t6 * t4, 10.0 * t6 * t2 * t0, 45.0 * t6 * t2, 120.0 * t6 * t0, 210.0 * t6};
+  return bj_compose<4>(t, f);
+}
+// a + bx (x - x0) + by (y - y0) as a series at (x0, y0)
+__device__ __forceinline__ BJ<4> bj_linear(double a, double bx, double by) {
+  BJ<4> r = bj_const<4>(a);
+  r.c[bidx(1, 0)] = bx;
+  r.c[bidx(0, 1)] = by;
+  return r;
+}
+
+__device__ __forceinline__ BJ<4> tilted_steps_surface(const double* __restrict__ tp, int n_steps, double x, double y) {
+  BJ<4> T = bj_const<4>(0.0);
+#pragma unroll 1
+  for (int s = 0; s < n_steps; ++s) {
+    const double* q = tp + 10 * s;
+    const double l = q[0], w = q[1], height = q[2], ox = q[3], oy = q[4], oz = q[5], yaw = q[6];
+    const double nx = q[7], ny = q[8], nz = q[9];
+    T.c[0] += oz;  // the origin height counts everywhere, also past the cut-off
+    double sn, cs;
+    sincos(yaw, &sn, &cs);
+    const double dx = x - ox, dy = y - oy;
+    const double xt = cs * dx + sn * dy, yt = cs * dy - sn * dx;
+    // X = 2 x_t / l, Y = 2 y_t / w: linear in (x, y)
+    const BJ<4> X = bj_linear(2.0 * xt / l, 2.0 * cs / l, 2.0 * sn / l);
+    const BJ<4> Y = bj_linear(2.0 * yt / w, -2.0 * sn / w, 2.0 * cs / w);
+    const BJ<4> g = bj_pow10(X) + bj_pow10(Y);
+    if (g.c[0] > STEP_CUTOFF) continue;
+    const BJ<4> E = step_bump(g);
+    // tilted top pi = height + a x_t + b y_t
+    const double a = -nx / nz, b = -ny / nz;
+    T = T + E * bj_linear(height + a * xt + b * yt, a * cs - b * sn, a * sn + b * cs);
+  }
+  return T;
+}
+
+// the surface of kernel terrain 1 or 2; n_steps is read by terrain 2 only
+template <int TERRAIN>
+__device__ __forceinline__ BJ<4> terrain_surface(const double* __restrict__ tp, int n_steps, double x, double y) {
+  static_assert(TERRAIN == 1 || TERRAIN == 2, "smooth terrains are 1 and 2");
+  if constexpr (TERRAIN == 1) return smooth_steps_surface(tp, x, y);
+  else return tilted_steps_surface(tp, n_steps, x, y);
 }
 
 struct TFrame {
@@ -63,9 +123,10 @@ struct TFrame {
   TJ Dn[3][2];       // d n_a / d x, d n_a / d y  (d / d z = 0)
 };
 
-__device__ __forceinline__ void smooth_terrain_frame(const double* __restrict__ tp, double x, double y, double z,
-                                                     TFrame& F) {
-  const BJ<4> T = smooth_steps_surface(tp, x, y);
+template <int TERRAIN>
+__device__ __forceinline__ void terrain_frame(const double* __restrict__ tp, int n_steps, double x, double y, double z,
+                                              TFrame& F) {
+  const BJ<4> T = terrain_surface<TERRAIN>(tp, n_steps, x, y);
   const BJ<3> gx3 = -bj_ddx<4>(T), gy3 = -bj_ddy<4>(T);
   const BJ<3> inv3 = bj_invsqrt<3>(gx3 * gx3 + gy3 * gy3 + 1.0);
   BJ<3> n3[3];

@@ -15,7 +15,8 @@
 // slots: w_centroid = com, w_ratio = average force, w_swing = point position, w_fd = force.
 //
 // TERRAIN: 0 = PlanarTerrain (h = p_z, n = e_z, R_t = I), 1 = the two smooth steps of the stairs (BASELINE config 5,
-// kino_smooth.cuh) with their ten parameters at p + po_terrain.  On the steps h depends on the whole point position and
+// kino_smooth.cuh) with their ten parameters at p + po_terrain, 2 = K general smooth steps (kino_smooth.cuh) with their
+// 10 K parameters closing p.  On the steps h depends on the whole point position and
 // n, R_t on (x, y): lane i < 8 evaluates the terrain frame of point i as order-2 series in its position and forms the
 // four terrain rows, their 25 Jacobian entries and the multiplier-weighted second derivatives from them.
 #include "kino_const.cuh"
@@ -26,14 +27,15 @@ namespace hb {
 // Terrain rows of contact point i on the smooth steps: relaxed complementarity eps - h n.(f mass), height h, normal
 // force n.f and friction-cone margin mu^2 (n.f)^2 - (x.f)^2 - (y.f)^2 (g rows, local Jacobian entries 25 i .. 25 i + 18
 // in pose_layout.py::_enumerate_jp order, and the multiplier-weighted (p, p), (p, f), (f, f) second derivatives).
-template <class JPut, class HAdd, class LamRow>
-__device__ __forceinline__ void smooth_point_rows(const KinoConst& C, const double* __restrict__ tp, int i, D3 ppos, D3 pf,
+template <int TERRAIN, class JPut, class HAdd, class LamRow>
+__device__ __forceinline__ void smooth_point_rows(const KinoConst& C, const double* __restrict__ tp, int n_steps, int i,
+                                                  D3 ppos, D3 pf,
                                                   double mass, double eps, double mu, bool want_g, bool want_jac,
                                                   bool want_hess, double* __restrict__ gb, JPut& jput, HAdd& hadd,
                                                   LamRow& lamrow) {
   const int fb_ = i * HB_KF_PT_COUNT, o = 15 * i;
   TFrame F;
-  smooth_terrain_frame(tp, ppos.x, ppos.y, ppos.z, F);
+  terrain_frame<TERRAIN>(tp, n_steps, ppos.x, ppos.y, ppos.z, F);
   const FrameForce ff = frame_force(F, pf, mu);
   const TJ hN = F.h * ff.N;  // h n.f: the complementarity row is eps - mass h n.f
   if (want_g) {
@@ -154,9 +156,10 @@ __global__ void __launch_bounds__(128) pose_contact_kernel(const KinoConst* __re
                              __shfl_sync(0xffffffffu, lin.z, 0));
   const D3 asum = v3<double>(__shfl_sync(0xffffffffu, ang.x, 0), __shfl_sync(0xffffffffu, ang.y, 0),
                              __shfl_sync(0xffffffffu, ang.z, 0));
-  if constexpr (TERRAIN == 1) {
+  if constexpr (TERRAIN != 0) {
+    const int n_steps = TERRAIN == 2 ? (C.n_p - C.po_terrain) / 10 : 0;  // the step records close p
     if (lane < 8 && (want_g || want_jac || want_hess))
-      smooth_point_rows(C, pp + C.po_terrain, lane, ppos, pf, mass, eps, mu, want_g, want_jac, want_hess,
+      smooth_point_rows<TERRAIN>(C, pp + C.po_terrain, n_steps, lane, ppos, pf, mass, eps, mu, want_g, want_jac, want_hess,
                         gb, jput, hadd, lamrow);
   }
   if (want_g) {
@@ -262,7 +265,7 @@ __global__ void __launch_bounds__(128) pose_contact_kernel(const KinoConst* __re
         jput(b0 + 10 + c, -1.0);
       }
     }
-    if (TERRAIN == 1 && lane < 8) {
+    if (TERRAIN != 0 && lane < 8) {
       const int b0 = JC_PT * lane + 19;  // the FK entries follow the point's 19 terrain-row entries
       for (int c = 0; c < 3; ++c) {
         jput(b0 + c, 1.0);

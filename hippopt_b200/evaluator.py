@@ -241,7 +241,7 @@ class KinoEvaluator(_Evaluator):
         po = lay.po
         ints = {
             "HORIZON": lay.N, "N_X": lay.n_x, "N_P": lay.n_p, "M": lay.m, "NNZ_J": lay.nnz_j, "NNZ_H": lay.nnz_h,
-            "N_JC": lay.n_jc, "N_JK": lay.n_jk, "N_HC": lay.n_hc, "TERRAIN": 0 if settings.terrain == "planar" else 1,
+            "N_JC": lay.n_jc, "N_JK": lay.n_jk, "N_HC": lay.n_hc, "TERRAIN": lay.kernel_terrain,
             "HAS_FINAL": int(settings.final_state_constraint), "HAS_PERIODICITY": int(settings.periodicity_constraint),
             "H_INIT": lay.h_init, "PO_DESC0": po.desc0, "PO_MASS": po.mass, "PO_INIT": po.init, "PO_FINAL": po.final,
             "PO_DT": po.dt, "PO_GRAVITY": po.gravity, "PO_KT": po.kt, "PO_KBS": po.k_bs, "PO_EPS": po.eps,
@@ -373,7 +373,8 @@ class PoseEvaluator(KinoEvaluator):
     """Evaluator of the static pose finder
     (`/root/reference/src/hippopt/turnkey_planners/humanoid_pose_finder/planner.py:303-413`), the one
     reference configuration IPOPT solves with the exact Hessian.  ``PoseSettings(terrain="smooth_steps",
-    n_terrain_params=10)`` poses it on the stairs, with the steps' parameters appended to p."""
+    n_terrain_params=10)`` poses it on the stairs, ``PoseSettings(terrain="tilted_steps", n_terrain_params=10 K)`` on K
+    general smooth steps (the ramp), with the steps' parameters appended to p."""
 
     def __init__(self, model: RobotModel, settings=None):
         from .pose_layout import PoseLayout, PoseSettings
@@ -386,7 +387,7 @@ class PoseEvaluator(KinoEvaluator):
         icfg = np.zeros(H["HB_KI_COUNT"], dtype=np.int32)
         ints = {
             "HORIZON": 1, "N_X": lay.n_x, "N_P": lay.n_p, "M": lay.m, "NNZ_J": lay.nnz_j, "NNZ_H": lay.nnz_h,
-            "N_JC": lay.n_jc, "N_JK": lay.n_jk, "N_HC": lay.n_hc, "TERRAIN": 0 if s.terrain == "planar" else 1,
+            "N_JC": lay.n_jc, "N_JK": lay.n_jk, "N_HC": lay.n_hc, "TERRAIN": lay.kernel_terrain,
             "HAS_FINAL": 0, "HAS_PERIODICITY": 0, "PO_TERRAIN": po.terrain,
             "H_INIT": 0, "PO_DESC0": po.desc0, "PO_MASS": po.mass, "PO_INIT": po.ref, "PO_GRAVITY": po.gravity,
             "PO_EPS": po.eps, "PO_MU": po.mu, "PO_MAX_S": po.max_s, "PO_MIN_S": po.min_s,

@@ -12,7 +12,7 @@
 
 `stairs_step_guess` builds the same set-up for BASELINE config 5 (walking on stairs): the keyframe poses are solved on
 the smooth-step terrain (pose-finder evaluator with ``terrain="smooth_steps"``), and the contacts land on the first
-tread.
+tread.  `ramp_step_guess` does the same for a step onto a ramp (``terrain="tilted_steps"``, one tilted step).
 
 Everything numeric runs on the GPU; the per-instance Python loop of the reference (one IPOPT solve after the other)
 is gone.  How far the interior-point driver gets on the plans built here (some converge, many do not) is recorded
@@ -47,28 +47,32 @@ def periodic_step_phases(step_length: np.ndarray, horizon_time: float, foot_y: f
                             horizon_time, force_z)
 
 
-def _left_then_right(l0, l_mid, l1, r0, r_mid, r1, T, force_z):
-    """Two contact phases per foot, (B, 3) positions, identity rotations: the left foot swings from l0 over l_mid to
-    l1 in (T/6, T/3), then the right foot from r0 over r_mid to r1 in (2T/3, 5T/6) (main_periodic_step.py:365-412)."""
+def _left_then_right(l0, l_mid, l1, r0, r_mid, r1, T, force_z, q1=None):
+    """Two contact phases per foot, (B, 3) positions: the left foot swings from l0 over l_mid to l1 in (T/6, T/3), then
+    the right foot from r0 over r_mid to r1 in (2T/3, 5T/6) (main_periodic_step.py:365-412).  Identity rotations, except
+    that q1 (xyzw, (4,) or (B, 4)), if given, is the rotation of both feet at their landing (and mid-swing) poses."""
     ident = np.array([0.0, 0.0, 0.0, 1.0])
+    q1 = ident if q1 is None else q1
 
-    def phase(p, mid, act, dea):
-        return FootContactPhaseDescriptor(position=p, quaternion_xyzw=ident, mid_swing_position=mid,
-                                          mid_swing_quaternion_xyzw=None if mid is None else ident,
+    def phase(p, mid, act, dea, q):
+        return FootContactPhaseDescriptor(position=p, quaternion_xyzw=q, mid_swing_position=mid,
+                                          mid_swing_quaternion_xyzw=None if mid is None else q1,
                                           force=np.array([0.0, 0.0, force_z]), activation_time=act, deactivation_time=dea)
 
     return FeetContactPhasesDescriptor(
-        left=[phase(l0, l_mid, None, T / 6.0), phase(l1, None, T / 3.0, None)],
-        right=[phase(r0, r_mid, None, T * 2.0 / 3.0), phase(r1, None, T * 5.0 / 6.0, None)])
+        left=[phase(l0, l_mid, None, T / 6.0, ident), phase(l1, None, T / 3.0, None, q1)],
+        right=[phase(r0, r_mid, None, T * 2.0 / 3.0, ident), phase(r1, None, T * 5.0 / 6.0, None, q1)])
 
 
-def pose_problem(lay, model, left_position: np.ndarray, right_position: np.ndarray, com_height: float = 0.7):
-    """Pose-finder references of compute_state (main_periodic_step.py:192-258) for feet flat at the given positions
-    (identity rotations): contact points from the foot transforms, CoM com_height above the middle of the feet,
-    identity base / frame quaternions, the desired joint configuration.  Returns (x guess, p); on the smooth-step
-    terrain the caller fills the terrain parameters."""
+def pose_problem(lay, model, left_position: np.ndarray, right_position: np.ndarray, com_height: float = 0.7,
+                 left_rotation: np.ndarray | None = None, right_rotation: np.ndarray | None = None):
+    """Pose-finder references of compute_state (main_periodic_step.py:192-258) for feet at the given positions
+    (identity rotations, or the (B, 3, 3) rotations given): contact points from the foot transforms, CoM com_height
+    above the middle of the feet, identity base / frame quaternions, the desired joint configuration.  Returns
+    (x guess, p); on a smooth-step terrain the caller fills the terrain parameters."""
     po = lay.po
     B = left_position.shape[0]
+    rot = [left_rotation, right_rotation]
     p = np.zeros((B, lay.n_p))
     for i in range(NPT):
         p[:, po.desc0 + 3 * i:po.desc0 + 3 * i + 3] = FOOT_CORNERS[i % 4]
@@ -77,7 +81,8 @@ def pose_problem(lay, model, left_position: np.ndarray, right_position: np.ndarr
     feet = (left_position, right_position)
     for i in range(NPT):
         o = po.ref + 9 * i
-        p[:, o:o + 3] = feet[i // 4] + FOOT_CORNERS[i % 4]
+        R = rot[i // 4]
+        p[:, o:o + 3] = feet[i // 4] + (FOOT_CORNERS[i % 4] if R is None else R @ FOOT_CORNERS[i % 4])
         p[:, o + 5] = 9.80665 / 8.0
         p[:, o + 6:o + 9] = FOOT_CORNERS[i % 4]
     com = (left_position + right_position) / 2.0
@@ -144,7 +149,19 @@ def _keyframe_plan(model, pose_evaluator, kino_evaluator, phases, centroid, terr
     # keyframes: (left phase, right phase) of compute_initial_state / compute_middle_state / compute_final_state
     lp = np.concatenate([phases.left[0].position, phases.left[1].position, phases.left[1].position])
     rp = np.concatenate([phases.right[0].position, phases.right[0].position, phases.right[1].position])
-    xq, pq = pose_problem(pl, model, lp, rp)
+
+    def rotations(ph):  # (B, 3, 3) foot rotation of a phase, or None when it is the identity
+        q = np.broadcast_to(np.asarray(ph.quaternion_xyzw, dtype=np.float64), (B, 4))
+        if np.all(q == [0.0, 0.0, 0.0, 1.0]):
+            return None
+        return _rotation_xyzw(q)
+
+    lr = [rotations(phases.left[0]), rotations(phases.left[1]), rotations(phases.left[1])]
+    rr = [rotations(phases.right[0]), rotations(phases.right[0]), rotations(phases.right[1])]
+    ident = np.broadcast_to(np.eye(3), (B, 3, 3))
+    lrot = None if all(r is None for r in lr) else np.concatenate([ident if r is None else r for r in lr])
+    rrot = None if all(r is None for r in rr) else np.concatenate([ident if r is None else r for r in rr])
+    xq, pq = pose_problem(pl, model, lp, rp, left_rotation=lrot, right_rotation=rrot)
     if terrain is not None:
         pq[:, pl.po.terrain:pl.po.terrain + terrain.shape[1]] = np.tile(terrain, (3, 1))
     lb, ub = pose_evaluator.bounds(pq)
@@ -226,6 +243,101 @@ def stairs_step_guess(model, pose_evaluator, kino_evaluator, step_height: np.nda
                               pos(tread_x, -foot_y, h), kino_evaluator.layout.N * STEP_DT, force_z)
     centroid = pos(mid_x, 0.0, 0.5 * h)
     return _keyframe_plan(model, pose_evaluator, kino_evaluator, phases, centroid, stairs_terrain(h), tol, max_iter)
+
+
+def _rotation_xyzw(q: np.ndarray) -> np.ndarray:
+    """(B, 4) unit quaternions (x, y, z, w) -> (B, 3, 3) rotation matrices."""
+    x, y, z, w = q[:, 0], q[:, 1], q[:, 2], q[:, 3]
+    return np.stack([
+        np.stack([1 - 2 * (y * y + z * z), 2 * (x * y - z * w), 2 * (x * z + y * w)], axis=1),
+        np.stack([2 * (x * y + z * w), 1 - 2 * (x * x + z * z), 2 * (y * z - x * w)], axis=1),
+        np.stack([2 * (x * z - y * w), 2 * (y * z + x * w), 1 - 2 * (x * x + y * y)], axis=1)], axis=1)
+
+
+def tilted_steps_terrain(length, width, height, origin, yaw=0.0, normal=(0.0, 0.0, 1.0)) -> np.ndarray:
+    """(B, 10 K) parameters of K general smooth steps (``terrain="tilted_steps"``), the arguments of
+    `SmoothTerrain.step` (smooth_terrain.py:235-336) per step: length l, width w, height, origin (ox, oy, oz), yaw and
+    the normal (n_x, n_y, n_z) of the tilted top.  Each argument is a scalar, a (K,) or (B, K) array (origin and normal:
+    (3,), (K, 3) or (B, K, 3)); a leading batch dimension B broadcasts.  The normal is taken as given (the reference does
+    not normalise it either); l, w > 0 and n_z > 0 are required."""
+    lw = np.asarray(length, dtype=np.float64)
+    K = 1 if lw.ndim == 0 else lw.shape[-1]
+
+    def scalars(a):
+        a = np.asarray(a, dtype=np.float64)
+        return np.atleast_2d(a.reshape(-1, K) if a.ndim else np.full((1, K), float(a)))
+
+    def vectors(a):
+        a = np.asarray(a, dtype=np.float64)
+        return a.reshape(1, 1, 3) if a.ndim == 1 else (a.reshape(1, K, 3) if a.ndim == 2 else a)
+
+    cols = [scalars(length), scalars(width), scalars(height), vectors(origin), scalars(yaw), vectors(normal)]
+    B = max(c.shape[0] for c in cols)
+    tp = np.zeros((B, K, 10))
+    tp[:, :, 0], tp[:, :, 1], tp[:, :, 2] = (np.broadcast_to(c, (B, K)) for c in cols[:3])
+    tp[:, :, 3:6] = np.broadcast_to(cols[3], (B, K, 3))
+    tp[:, :, 6] = np.broadcast_to(cols[4], (B, K))
+    tp[:, :, 7:10] = np.broadcast_to(cols[5], (B, K, 3))
+    if not np.all(np.isfinite(tp)):
+        raise ValueError("tilted_steps_terrain: non-finite parameter")
+    if np.any(tp[:, :, 0] <= 0.0) or np.any(tp[:, :, 1] <= 0.0):
+        raise ValueError("tilted_steps_terrain: length and width must be positive")
+    if np.any(tp[:, :, 9] <= 0.0):
+        raise ValueError("tilted_steps_terrain: the normal's z component must be positive")
+    return tp.reshape(B, 10 * K)
+
+
+# the ramp of ramp_step_guess: one smooth step of length RAMP_LENGTH whose top rises along +x with the slope s (rise
+# over run), its low edge (at height 0) at x = RAMP_START, its high edge at height s RAMP_LENGTH
+RAMP_START, RAMP_LENGTH, RAMP_WIDTH = 0.225, 2.0, 0.8
+
+
+def ramp_terrain(slope: np.ndarray) -> np.ndarray:
+    """(B, 10) tilted_steps parameters of the ramp with the slope s (rise over run) per instance."""
+    s = np.asarray(slope, dtype=np.float64).reshape(-1)
+    n = np.stack([-s, np.zeros_like(s), np.ones_like(s)], axis=1) / np.sqrt(1.0 + s * s)[:, None]
+    return tilted_steps_terrain(RAMP_LENGTH, RAMP_WIDTH, s[:, None] * (0.5 * RAMP_LENGTH),
+                                [RAMP_START + 0.5 * RAMP_LENGTH, 0.0, 0.0], 0.0, n[:, None, :])
+
+
+def ramp_step_guess(model, pose_evaluator, kino_evaluator, slope: np.ndarray, tol: float = 1e-8, max_iter: int = 300,
+                    force_z: float = 100.0, mass_normalised: bool = False, start_x: float = 0.0,
+                    tread_x: float = 0.5, foot_y: float = 0.1, swing_height: float = 0.05) -> PeriodicStepGuess:
+    """The ramp counterpart of stairs_step_guess (N = 50, dt = 0.1): a step onto the ramp of `ramp_terrain` with the
+    slope s per instance, on evaluators posed on ``terrain="tilted_steps"`` with one step.  The robot starts with both
+    feet flat on the ground centred at x = start_x (every foot corner clear of the ramp's low edge at RAMP_START), steps
+    with the left foot onto the slope (centred at x = tread_x), then with the right foot.
+
+    * keyframes: initial (both feet on the ground), middle (left foot on the slope), final (both feet on the slope),
+      three pose-finder solves per instance as ONE batch of 3 B; the feet on the slope are pitched to it (rotation
+      about y by -atan s) and their centres lie on the slope's surface;
+    * guess and references as stairs_step_guess (contact centroid halfway between start and tread, at half the tread
+      height).
+
+    UNPINNED: the reference's ramp main is available here only through the terrain SURVEY.md A.10 cites; this keyframe
+    placement is this project's own, not a restatement."""
+    if mass_normalised:
+        force_z = force_z / float(model.total_mass())
+    s = np.asarray(slope, dtype=np.float64).reshape(-1)
+    B = s.shape[0]
+    for ev in (pose_evaluator, kino_evaluator):
+        if ev.layout.st.terrain != "tilted_steps" or ev.layout.st.n_terrain_params != 10:
+            raise ValueError("ramp_step_guess: both evaluators must be posed on tilted_steps with one step")
+
+    def pos(x, y, z):
+        return np.stack([np.full(B, x), np.full(B, y), z], axis=1)
+
+    zero = np.zeros(B)
+    top = s * (tread_x - RAMP_START)  # surface height under the tread's centre
+    mid_x = 0.5 * (start_x + tread_x)
+    half = -0.5 * np.arctan(s)  # pitch about y that lifts the toe onto the slope
+    q1 = np.stack([zero, np.sin(half), zero, np.cos(half)], axis=1)
+    phases = _left_then_right(pos(start_x, foot_y, zero), pos(mid_x, foot_y, top + swing_height),
+                              pos(tread_x, foot_y, top), pos(start_x, -foot_y, zero),
+                              pos(mid_x, -foot_y, top + swing_height), pos(tread_x, -foot_y, top),
+                              kino_evaluator.layout.N * STEP_DT, force_z, q1=q1)
+    centroid = pos(mid_x, 0.0, 0.5 * top)
+    return _keyframe_plan(model, pose_evaluator, kino_evaluator, phases, centroid, ramp_terrain(s), tol, max_iter)
 
 
 def single_step_problem(model, pose_evaluator, kino_evaluator, step_length: np.ndarray, tol: float = 1e-8,

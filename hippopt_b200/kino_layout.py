@@ -41,12 +41,32 @@ NCV = 129
 SKEW_PAIRS = [(0, 1), (0, 2), (1, 0), (1, 2), (2, 0), (2, 1)]
 
 
+# terrain name -> kernel terrain (HB_KI_TERRAIN).  "smooth_steps": the two axis-aligned flat steps of the stairs, ten
+# parameters (l, w, height, ox, oy) x 2; "tilted_steps": K >= 1 general steps (yaw, origin height, tilted top), 10 K
+# parameters (l, w, height, ox, oy, oz, yaw, n_x, n_y, n_z) per step.  The terrain parameters close p.
+TERRAINS = {"planar": 0, "smooth_steps": 1, "tilted_steps": 2}
+
+
+def kernel_terrain(terrain: str, n_terrain_params: int) -> int:
+    """The kernel terrain of a terrain name, after checking that the parameter count fits it."""
+    if terrain not in TERRAINS:
+        raise ValueError(f"terrain must be one of {sorted(TERRAINS)}, not {terrain!r}")
+    n = n_terrain_params
+    if terrain == "planar" and n != 0:
+        raise ValueError("the planar terrain takes no terrain parameters")
+    if terrain == "smooth_steps" and n != 10:
+        raise ValueError("the smooth steps take 10 terrain parameters")
+    if terrain == "tilted_steps" and (n < 10 or n % 10 != 0):
+        raise ValueError(f"tilted_steps takes 10 parameters per step (a positive multiple of 10), not {n}")
+    return TERRAINS[terrain]
+
+
 @dataclasses.dataclass
 class KinoSettings:
     """Numeric settings; defaults = `main_single_step_flat_ground.py:54-104` (BASELINE config 3)."""
 
     horizon: int = 30
-    terrain: str = "planar"  # "planar" | "smooth_steps"
+    terrain: str = "planar"  # one of TERRAINS
     n_terrain_params: int = 0
     final_state_constraint: bool = False
     periodicity_constraint: bool = False
@@ -137,6 +157,7 @@ class KinoLayout:
     def __init__(self, model: RobotModel, settings: KinoSettings):
         self.model = model
         self.st = settings
+        self.kernel_terrain = kernel_terrain(settings.terrain, settings.n_terrain_params)
         N = self.N = settings.horizon
         self.knot_size = NZ  # variables per knot (stage size of the KKT sweep)
         self.n_x = NZ * N + 6

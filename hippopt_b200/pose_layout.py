@@ -18,7 +18,7 @@ import dataclasses
 
 import numpy as np
 
-from .kino_layout import COM, F, H, NCV, NJ, NPT, NZ, P, PB, Q, QD, S, SD, SKEW_PAIRS, VB
+from .kino_layout import COM, F, H, NCV, NJ, NPT, NZ, P, PB, Q, QD, S, SD, SKEW_PAIRS, VB, kernel_terrain
 from .robot_model import RobotModel
 
 XPB, XQ, XS, XCOM, NX = 48, 51, 55, 78, 81
@@ -28,7 +28,7 @@ XPB, XQ, XS, XCOM, NX = 48, 51, 55, 78, 81
 class PoseSettings:
     """`humanoid_pose_finder/main.py:75-98`."""
 
-    terrain: str = "planar"  # "planar" | "smooth_steps"
+    terrain: str = "planar"  # one of kino_layout.TERRAINS
     n_terrain_params: int = 0
     foot_frames: tuple = ("l_sole", "r_sole")
     frame_quaternion_cost_frame: str = "chest"
@@ -78,11 +78,8 @@ class PoseLayout:
         self.st = settings or PoseSettings()
         self.N = 1
         self.n_x = NX
-        if self.st.terrain not in ("planar", "smooth_steps"):
-            raise ValueError(f"terrain must be 'planar' or 'smooth_steps', not {self.st.terrain!r}")
+        self.kernel_terrain = kernel_terrain(self.st.terrain, self.st.n_terrain_params)
         self.smooth = self.st.terrain != "planar"
-        if self.st.n_terrain_params != (10 if self.smooth else 0):
-            raise ValueError("the smooth steps take 10 terrain parameters, the planar terrain none")
         self.po = PoseParamOffsets(self.st.n_terrain_params)
         self.n_p = self.po.n_p
         zmap = -np.ones(NZ, dtype=np.int32)

@@ -27,7 +27,7 @@ def kino_parameters(lay: KinoLayout, model: RobotModel, B: int, rng: np.random.G
     p[:, po.mass] = M
     # initial / final state: feet flat at y = +-0.1, base above, forces = weight / 8 (mass-normalised)
     # on the stairs the robot starts in front of the first step edge (x = 0.225) and ends on it
-    x_start = 0.15 if lay.st.n_terrain_params == 10 else 0.0
+    x_start = 0.15 if lay.st.terrain == "smooth_steps" else 0.0
     for base, dx in ((po.init, 0.0), (po.final, 0.3)):
         step = x_start + dx * rng.uniform(0.8, 1.2, B) * spread
         for i in range(NPT):
@@ -72,7 +72,7 @@ def kino_parameters(lay: KinoLayout, model: RobotModel, B: int, rng: np.random.G
             p[:, r + o:r + o + 4] = qq / np.linalg.norm(qq, axis=1, keepdims=True)
         p[:, r + po.R_BQV:r + po.R_BQV + 4] = 0.01 * spread * rng.normal(size=(B, 4))
         p[:, r + po.R_JR:r + po.R_JR + NJ] = 0.05 * spread * rng.normal(size=(B, NJ))
-    if lay.st.n_terrain_params == 10:
+    if lay.st.terrain == "smooth_steps":
         # two smooth steps of `main_walking_on_stairs.py:18-28,397-403` (step_length 0.9, width 0.8), with
         # the step height randomised per instance in U(0.05, 0.15) (BASELINE config 5)
         L = 0.45
@@ -81,7 +81,26 @@ def kino_parameters(lay: KinoLayout, model: RobotModel, B: int, rng: np.random.G
         p[:, po.terrain:po.terrain + 10] = tp
         p[:, po.terrain + 2] = height
         p[:, po.terrain + 7] = height
+    elif lay.st.terrain == "tilted_steps":
+        p[:, po.terrain:] = tilted_steps_sample(lay.st.n_terrain_params // 10, B, rng)
     return p
+
+
+def tilted_steps_sample(K: int, B: int, rng: np.random.Generator) -> np.ndarray:
+    """(B, 10 K) parameters of K rotated, raised and tilted steps that overlap around the origin, where the contact
+    points of kino_points lie: per step (l, w, height, ox, oy, oz, yaw, n_x, n_y, n_z), a unit normal tilted by up to
+    about 20 degrees."""
+    tp = np.zeros((B, K, 10))
+    tp[:, :, 0] = rng.uniform(0.6, 1.4, (B, K))
+    tp[:, :, 1] = rng.uniform(0.5, 1.0, (B, K))
+    tp[:, :, 2] = rng.uniform(0.02, 0.12, (B, K))
+    tp[:, :, 3] = rng.uniform(-0.3, 0.3, (B, K))
+    tp[:, :, 4] = rng.uniform(-0.2, 0.2, (B, K))
+    tp[:, :, 5] = rng.uniform(-0.03, 0.03, (B, K))
+    tp[:, :, 6] = rng.uniform(-0.6, 0.6, (B, K))
+    n = np.concatenate([rng.uniform(-0.25, 0.25, (B, K, 2)), np.ones((B, K, 1))], axis=2)
+    tp[:, :, 7:10] = n / np.linalg.norm(n, axis=2, keepdims=True)
+    return tp.reshape(B, 10 * K)
 
 
 def kino_points(lay: KinoLayout, p: np.ndarray, rng: np.random.Generator, noise: float = 1e-2):

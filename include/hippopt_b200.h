@@ -56,8 +56,11 @@ enum {
   HB_KI_N_JC,
   HB_KI_N_JK,
   HB_KI_N_HC,
-  HB_KI_TERRAIN,          /* 0 planar (planar_terrain.py), 1 sum of two smooth steps (the stairs); both for either
-                             kind, the steps' ten parameters (l, w, height, ox, oy) x 2 at HB_KI_PO_TERRAIN in p */
+  HB_KI_TERRAIN,          /* 0 planar (planar_terrain.py), 1 sum of two smooth steps (the stairs), 2 sum of K general
+                             smooth steps (the ramp); all for either kind.  1: the steps' ten parameters
+                             (l, w, height, ox, oy) x 2 at HB_KI_PO_TERRAIN in p.  2: K records
+                             (l, w, height, ox, oy, oz, yaw, n_x, n_y, n_z) from HB_KI_PO_TERRAIN to the end of p;
+                             K = (n_p - HB_KI_PO_TERRAIN) / 10, which must be a whole number >= 1 (else HB_ERR_INVALID) */
   HB_KI_HAS_FINAL,
   HB_KI_HAS_PERIODICITY,
   HB_KI_H_INIT,           /* x offset of initial_state.centroidal_momentum */
@@ -473,13 +476,17 @@ int hb_debug_sweep_schedule_n_base(int32_t nb, const int32_t* parent, int32_t fo
                                    int32_t typed, int32_t n_base, int32_t* tasks, int32_t* info);
 
 /* The smooth-step terrain jets of the contact kernel (hippopt_b200/csrc/kino_smooth.cuh), evaluated by the production
- * smooth_steps_surface and smooth_terrain_frame at n points, for tests that compare them with a symbolic reference.
+ * smooth_steps_surface and terrain_frame<1> at n points, for tests that compare them with a symbolic reference.
  *   tp   device [n][10]   terrain parameters of each point, (l, w, height, ox, oy) x 2
  *   pts  device [n][3]    (x, y, z)
  *   out  device [n][HB_SMOOTH_TERRAIN_OUT]  the 15 normalised coefficients of the order-4 surface jet T(x, y), then the
  *        TFrame fields in declaration order, 10 trivariate coefficients each: h, gx, gy, n[3], xh[3], yh[3], Dn[3][2] */
 #define HB_SMOOTH_TERRAIN_OUT 195
 int hb_debug_smooth_terrain(const double* tp, const double* pts, int64_t n, double* out, void* stream);
+
+/* The same for kernel terrain 2 (tilted_steps_surface, K = n_steps general steps) with the same output layout.
+ *   tp   device [n][10 n_steps]  terrain parameters of each point, (l, w, height, ox, oy, oz, yaw, n_x, n_y, n_z) per step */
+int hb_debug_tilted_terrain(const double* tp, int32_t n_steps, const double* pts, int64_t n, double* out, void* stream);
 
 const char* hb_last_error(void);
 
