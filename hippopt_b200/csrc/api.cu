@@ -145,6 +145,14 @@ __global__ void reduce_f_kernel(const double* __restrict__ fpart, double* __rest
   f[b] = acc;
 }
 
+// contact kernel of a terrain (hb_kino_create accepts 0, 1 and 2)
+static decltype(&hb::kino_contact_kernel<0>) kino_contact_kernel_for(int terrain) {
+  return terrain == 0 ? hb::kino_contact_kernel<0> : terrain == 2 ? hb::kino_contact_kernel<2> : hb::kino_contact_kernel<1>;
+}
+static decltype(&hb::pose_contact_kernel<0>) pose_contact_kernel_for(int terrain) {
+  return terrain == 0 ? hb::pose_contact_kernel<0> : terrain == 2 ? hb::pose_contact_kernel<2> : hb::pose_contact_kernel<1>;
+}
+
 // ---------------------------------------------------------------------------------------------
 // Schedule of the packed tangent sweep: sweep_schedule.h (host-only, also reachable through
 // hb_debug_sweep_schedule for the CPU tests)
@@ -369,10 +377,10 @@ extern "C" int hb_kino_create(const int32_t* icfg, const double* dcfg, const int
   }
   {
     hb::KinTopo& T = h->topo;
+    static_cast<hb::KinScalars&>(T) = C;
     for (int l = 0; l < HB_MAX_BODIES; ++l) {
       const bool in = l < C.nb;
       T.mass[l] = in ? C.body[l].mass : 0.0;
-      T.sub_mask[l] = C.sub_mask[l];
       T.parent[l] = (signed char)(in ? C.body[l].parent : -1);
       T.slot[l] = (signed char)(in ? C.body[l].slot : -1);
       T.carry[l] = (signed char)(in ? C.body[l].carry : 0);
@@ -388,60 +396,8 @@ extern "C" int hb_kino_create(const int32_t* icfg, const double* dcfg, const int
           T.n_steps++;
         }
       }
-    std::memcpy(T.fam, C.fam, sizeof(T.fam));
-    T.nb = C.nb;
-    T.foot_body[0] = C.foot_body[0];
-    T.foot_body[1] = C.foot_body[1];
-    T.chest_body = C.chest_body;
-    T.max_depth = C.max_depth;
-    T.n_slots = C.n_slots;
-    T.max_sib = C.max_sib;
-    T.N = C.N;
-    T.n_x = C.n_x;
-    T.m = C.m;
-    T.nnz_j = C.nnz_j;
-    T.nnz_h = C.nnz_h;
-    T.n_jk = C.n_jk;
-    T.x_stride = C.x_stride;
-    T.cost_k0 = C.cost_k0;
-    T.joint_cost_kind = C.joint_cost_kind;
     T.zmap_identity = 1;
     for (int i = 0; i < 189; ++i) T.zmap_identity = T.zmap_identity && C.zmap[i] == i;
-    T.po_desc0 = C.po_desc0;
-    T.po_mass = C.po_mass;
-    T.po_fq = C.po_fq;
-    T.po_bq = C.po_bq;
-    T.po_bqv = C.po_bqv;
-    T.po_jr = C.po_jr;
-    T.ref_stride = C.ref_stride;
-    T.w_frame = C.w_frame;
-    T.w_bq = C.w_bq;
-    T.w_bqv = C.w_bqv;
-    T.w_joint = C.w_joint;
-    T.total_mass = C.total_mass;
-    T.n_jc = C.n_jc;
-    T.n_hc = C.n_hc;
-    T.has_final = C.has_final;
-    T.has_per = C.has_per;
-    T.h_init = C.h_init;
-    T.po_dt = C.po_dt;
-    T.po_gravity = C.po_gravity;
-    T.po_kt = C.po_kt;
-    T.po_kbs = C.po_kbs;
-    T.po_eps = C.po_eps;
-    T.po_mu = C.po_mu;
-    T.po_refs0 = C.po_refs0;
-    T.po_terrain = C.po_terrain;
-    for (int i = 0; i < 3; ++i) {
-      T.yaw[i] = C.yaw[i];
-      T.w_comvel[i] = C.w_comvel[i];
-    }
-    T.w_swing = C.w_swing;
-    T.w_u = C.w_u;
-    T.w_fd = C.w_fd;
-    T.w_centroid = C.w_centroid;
-    T.w_ratio = C.w_ratio;
-    T.w_yaw = C.w_yaw;
   }
   const size_t N = C.N;
   h->c_icfg.assign(icfg, icfg + HB_KI_COUNT);
@@ -782,30 +738,15 @@ extern "C" int hb_eval(hb_handle h, uint32_t mask, const double* x, const double
     const size_t smem = (size_t)(C.kind == 1 ? hb::pose_contact_smem_layout(C.n_hc) : hb::kino_contact_smem_layout(C.n_hc)).total *
                         sizeof(double) * warps_per_block;
     // the shared block holds the kernel's n_hc Hessian accumulators (191 planar, 255 on the smooth steps)
-    if (C.kind == 1 && C.terrain == 0) {
-      hb::pose_contact_kernel<0><<<grid, 32 * warps_per_block, smem, st>>>(h->dev, mask, x, p, (long)p_stride, lam_g, sigma,
-                                                                          d_fpart, grad_f, g, jac_vals, hess_vals,
-                                                                          (long)batch);
-    } else if (C.kind == 1 && C.terrain == 1) {
-      hb::pose_contact_kernel<1><<<grid, 32 * warps_per_block, smem, st>>>(h->dev, mask, x, p, (long)p_stride, lam_g, sigma,
-                                                                          d_fpart, grad_f, g, jac_vals, hess_vals,
-                                                                          (long)batch);
-    } else if (C.kind == 1) {
-      hb::pose_contact_kernel<2><<<grid, 32 * warps_per_block, smem, st>>>(h->dev, mask, x, p, (long)p_stride, lam_g, sigma,
-                                                                          d_fpart, grad_f, g, jac_vals, hess_vals,
-                                                                          (long)batch);
-    } else if (C.terrain == 0)
-      hb::kino_contact_kernel<0><<<grid, 32 * warps_per_block, smem, st_contact>>>(h->topo, h->dev, mask, x, p, (long)p_stride,
-                                                                                  lam_g, sigma, d_fpart, grad_f, g, jac_vals,
-                                                                                  hess_vals, (long)batch);
-    else if (C.terrain == 2)
-      hb::kino_contact_kernel<2><<<grid, 32 * warps_per_block, smem, st_contact>>>(h->topo, h->dev, mask, x, p, (long)p_stride,
-                                                                                  lam_g, sigma, d_fpart, grad_f, g, jac_vals,
-                                                                                  hess_vals, (long)batch);
-    else
-      hb::kino_contact_kernel<1><<<grid, 32 * warps_per_block, smem, st_contact>>>(h->topo, h->dev, mask, x, p, (long)p_stride,
-                                                                                  lam_g, sigma, d_fpart, grad_f, g, jac_vals,
-                                                                                  hess_vals, (long)batch);
+    if (C.kind == 1) {
+      const auto kernel = pose_contact_kernel_for(C.terrain);
+      kernel<<<grid, 32 * warps_per_block, smem, st>>>(h->dev, mask, x, p, (long)p_stride, lam_g, sigma, d_fpart, grad_f, g,
+                                                       jac_vals, hess_vals, (long)batch);
+    } else {
+      const auto kernel = kino_contact_kernel_for(C.terrain);
+      kernel<<<grid, 32 * warps_per_block, smem, st_contact>>>(h->topo, h->dev, mask, x, p, (long)p_stride, lam_g, sigma,
+                                                               d_fpart, grad_f, g, jac_vals, hess_vals, (long)batch);
+    }
     CUDA_TRY(cudaGetLastError());
     h->launches++;
     if (overlap) CUDA_TRY(cudaEventRecord(h->ev_join, h->aux));
@@ -1457,15 +1398,9 @@ extern "C" int hb_eval_cost_terms(hb_handle h, const double* x, const double* p,
   CUDA_TRY(cudaGetDevice(&dev));
   CUDA_TRY(ensure_kernel_attributes(dev));
   const size_t smem_c = (size_t)hb::kino_contact_smem_layout(C.n_hc).total * sizeof(double) * wpb;
-  if (C.terrain == 0)
-    hb::kino_contact_kernel<0><<<grid, 32 * wpb, smem_c, st>>>(h->topo, h->dev, mask, x, p, (long)p_stride, nullptr, nullptr,
-                                                              terms, nullptr, nullptr, nullptr, nullptr, (long)batch);
-  else if (C.terrain == 2)
-    hb::kino_contact_kernel<2><<<grid, 32 * wpb, smem_c, st>>>(h->topo, h->dev, mask, x, p, (long)p_stride, nullptr, nullptr,
-                                                              terms, nullptr, nullptr, nullptr, nullptr, (long)batch);
-  else
-    hb::kino_contact_kernel<1><<<grid, 32 * wpb, smem_c, st>>>(h->topo, h->dev, mask, x, p, (long)p_stride, nullptr, nullptr,
-                                                              terms, nullptr, nullptr, nullptr, nullptr, (long)batch);
+  const auto contact_kernel = kino_contact_kernel_for(C.terrain);
+  contact_kernel<<<grid, 32 * wpb, smem_c, st>>>(h->topo, h->dev, mask, x, p, (long)p_stride, nullptr, nullptr, terms, nullptr,
+                                                 nullptr, nullptr, nullptr, (long)batch);
   CUDA_TRY(cudaGetLastError());
   const size_t smem_k = (size_t)hb::kin_smem_layout(C.nb, C.n_slots, false).total * sizeof(double) * wpb;
   hb::kino_kin_kernel<false><<<grid, 32 * wpb, smem_k, st>>>(h->topo, h->dev, mask, x, p, (long)p_stride, nullptr, nullptr,

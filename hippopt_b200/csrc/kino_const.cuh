@@ -59,7 +59,10 @@ struct alignas(16) KnotMaps {
   int jk_base, jk_off, jk_cnt, hk_base, hk_off, hk_cnt, hk2_base, hk2_off;
 };
 
-struct KinoConst {
+// Scalars of one problem: sizes, offsets into x / p / g, weights, frames and the tree.  Both constant blocks below
+// (KinoConst in global memory, KinTopo as a kernel parameter) derive from it: hb_kino_create fills the scalars once
+// and copies them into KinTopo in one assignment.
+struct KinScalars {
   int N, n_x, n_p, m, nnz_j, nnz_h, n_jc, n_jk, n_hc, terrain, has_final, has_per, h_init;
   int po_desc0, po_mass, po_init, po_final, po_dt, po_gravity, po_kt, po_kbs, po_eps, po_mu, po_max_u, po_max_fd,
       po_max_L, po_min_com_h, po_min_feet_d, po_max_feet_h, po_max_s, po_min_s, po_max_sd, po_min_sd, po_refs0,
@@ -78,6 +81,9 @@ struct KinoConst {
   double wj[HB_N_JOINTS];
   double total_mass;
   double foot_R[2][9], foot_t[2][3], chest_R[9];
+};
+
+struct KinoConst : KinScalars {
   BodyC body[HB_MAX_BODIES];
   const int* jc_map;
   const int* jk_map;
@@ -91,31 +97,23 @@ struct KinoConst {
   const unsigned* hc_list;
 };
 
+static_assert(sizeof(KinoConst) == 15024, "KinoConst layout: body[] and the tables follow the scalars unchanged");
+
 // Warp-uniform part of KinoConst.  It is passed BY VALUE as a __grid_constant__ kernel parameter:
 // reads whose index is the same for every lane (tree topology inside the sweeps, row families with a
 // compile-time id) become constant-bank operands instead of global loads -- in the ncu capture of the
 // previous version those loads were ~40 % of the long-scoreboard stalls of the kinematics kernel.
+// The scalars (KinScalars, shared with KinoConst) are read from the constant bank too, so that the first
+// global load of a warp is its data, not the address of its data.
 // Lane-indexed data (joint frames, inertias, per-point families) stays in KinoConst / global memory,
 // where a divergent index costs one coalesced load rather than a serialised constant fetch.
-struct KinTopo {
+struct KinTopo : KinScalars {
   double mass[HB_MAX_BODIES];
-  unsigned sub_mask[HB_MAX_BODIES];
   signed char parent[HB_MAX_BODIES], slot[HB_MAX_BODIES], carry[HB_MAX_BODIES];
   // (depth, sibling rank) pairs that hold at least one body, deepest first (level-wise adjoint pass)
   signed char step_depth[2 * HB_MAX_BODIES], step_rank[2 * HB_MAX_BODIES];
   int n_steps;
-  int fam[HB_KF_COUNT][4];
-  int nb, foot_body[2], chest_body, max_depth, n_slots, max_sib;
-  // scalars of the kinematics kernel (offsets into x / p / g and weights): read from the constant bank, so
-  // that the first global load of a warp is its data, not the address of its data
-  int N, n_x, m, nnz_j, nnz_h, n_jk, x_stride, cost_k0, joint_cost_kind, zmap_identity;
-  int po_desc0, po_mass, po_fq, po_bq, po_bqv, po_jr, ref_stride;
-  double w_frame, w_bq, w_bqv, w_joint, total_mass;
-  // ... and of the contact kernel
-  int n_jc, n_hc, has_final, has_per, h_init;
-  int po_dt, po_gravity, po_kt, po_kbs, po_eps, po_mu, po_refs0, po_terrain;
-  int yaw[3];
-  double w_swing, w_u, w_fd, w_centroid, w_comvel[3], w_ratio, w_yaw;
+  int zmap_identity;  // zmap[i] == i for every virtual variable: the knot block of x is read without the map
   const int* jc_map;
   const short* hc_index;
   const int* hc_map;
@@ -133,6 +131,7 @@ struct KinTopo {
   unsigned round_seed_mask;  // bit r: some task of round r sits on a foot / chest body (seed tangents needed)
   unsigned round_heavy_mask;  // bit r: round r holds "in" tasks (sub-tree of the direction); else pure propagation
 };
+static_assert(sizeof(KinTopo) <= 4096, "KinTopo is passed as a kernel parameter");
 
 // global g index of local row r of family `fam` at knot k, or -1 when the row does not exist
 template <class Tab>
